@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- audio-seconds per second of the stage-1 STFT + FDAF echo canceller on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 2|3|4]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 2|3|4] [--dump-outputs DIR]
     (N > 1: launched by torchrun, one rank per GPU)
 
 One "step" = one pass of the hot path over one batch of synthetic utterances:
@@ -19,6 +19,9 @@ One "step" = one pass of the hot path over one batch of synthetic utterances:
             roofline, SURVEY.md 8d) with the HBM fraction (MEASURED_PEAKS.json) beside it.
   cpu_baseline  the C oracle (builder-authored port; the reference has no stage-1 filter) on the
             box's host cores over a bounded sample of the same workload.
+  dump      --dump-outputs DIR writes what the headline's last timed step returned (rank 0's utterances): DIR/erle_db.npy,
+            the per-utterance ERLE [B], and DIR/error_signal.npy, the error signal of a fixed seeded sample of utterances
+            (dump_rows), both float32.  The inputs are seeded, so two builds can be compared output for output.
 `--impl reference` times that CPU port alone (there is no reference implementation of this path).
 """
 import argparse
@@ -173,6 +176,17 @@ def workload_config(wl, world):
             "generator": "bench.make_inputs (SURVEY 8d recipe, CPU-seeded draws, seed 1000 + rank)",
             "l2": "inputs %.1f GB/GPU per step >> 126 MB L2 (no flush needed)" % (2 * B * L * 4 / 1e9),
             "parallelism": f"utterance-sharded x{world}, metrics-only all_gather"}
+
+
+DUMP_BYTES = 48 << 20       # error-signal rows of --dump-outputs: with the ERLE, well under 64 MB per dump
+
+
+def dump_rows(B, L):
+    """the utterances whose error signal --dump-outputs writes: a fixed seeded sample, sorted"""
+    import numpy as np
+
+    k = max(1, min(B, DUMP_BYTES // (4 * L)))
+    return np.sort(np.random.default_rng(0).choice(B, size=k, replace=False))
 
 
 def cpu_sample_size(cores, B):
@@ -471,7 +485,13 @@ def main():
     ap.add_argument("--no-numa-bind", action="store_true")
     ap.add_argument("--e2e-slots", type=int, default=0)
     ap.add_argument("--e2e-slice", type=int, default=128)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned to DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     wl = WORKLOADS[args.config]
     if args.algo is not None and args.algo != wl["algo"]:
         wl = dict(wl, algo=args.algo, name=wl["name"] + " -- run through aec_cfg.algo = %d (%s)" % (
@@ -535,6 +555,9 @@ def main():
         A.stage1_aec(far, mic, cfg, out=err, return_erle=True)
     total_ms, kern_ms, launches, erle, (wall0, wall1) = device_timed(A, torch, dist, sharding, far, mic, err, cfg,
                                                                     args.steps, world, n_total)
+    dump = None
+    if args.dump_outputs and rank == 0:      # device copies now (untimed), written to DIR at the end
+        dump = {"error_signal": err[torch.from_numpy(dump_rows(B, L)).cuda()], "erle_db": erle}
     wall = wall1 - wall0
     clocks = None
     if rank == 0:
@@ -697,6 +720,10 @@ def main():
         "wall_s_timed_region": wall, "erle_db_mean": erle_mean, "outputs_finite": finite,
         "parity": "FDAF recurrence: parity UNPINNED (no reference implementation); STFT/iSTFT pinned by golden vectors",
     }
+    if dump is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, t in dump.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), t.cpu().numpy())
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()

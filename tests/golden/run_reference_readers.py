@@ -1,11 +1,11 @@
 """Runs the REFERENCE's own dataset readers on files written by this repository's generators, with
-``acoustic_echo_cancellation_b200.h5lite`` standing in for ``h5py`` (absent from the image) -- TEST INFRASTRUCTURE, executed
-in a subprocess by tests/test_h5lite.py and only where /root/reference exists (this container; not the GPU box).
+``acoustic_echo_cancellation_b200.h5lite`` standing in for ``h5py`` -- TEST INFRASTRUCTURE, executed in a subprocess by
+tests/test_h5lite.py and only where AEC_REFERENCE_DIR names a checkout of the reference.
 
-    python run_reference_readers.py <repo root> <tr_list.txt> <tt/test.ex> <out.npz>
+    python run_reference_readers.py <repo root> <reference Stage2_lhm/scripts> <tr_list.txt> <tt/test.ex> <out.npz>
 
 Imports Stage2_lhm/scripts/test.py:19-33 (``ValidateDataset``) and scripts/train1.py:29-42 (``TrainDataset``) unmodified
-from /root/reference; ``soundfile`` (absent, used only by the tester's wav writer) is stubbed with an empty module.
+from the reference; ``soundfile`` (used only by the tester's wav writer) is stubbed with an empty module.
 Every array the readers return is saved to <out.npz> for the caller to compare with what went in.
 """
 import sys
@@ -13,13 +13,13 @@ import types
 
 import numpy as np
 
-repo, tr_list, test_ex, out = sys.argv[1:5]
+repo, ref_scripts, tr_list, test_ex, out = sys.argv[1:6]
 sys.path.insert(0, repo)
 from acoustic_echo_cancellation_b200 import h5lite  # noqa: E402
 
 sys.modules["h5py"] = h5lite
 sys.modules.setdefault("soundfile", types.ModuleType("soundfile"))
-sys.path.insert(0, "/root/reference/Stage2_lhm/scripts")
+sys.path.insert(0, ref_scripts)
 saved_argv, sys.argv = sys.argv, [sys.argv[0]]
 from test import ValidateDataset  # noqa: E402  (Stage2_lhm/scripts/test.py)
 from train1 import TrainDataset  # noqa: E402   (Stage2_lhm/scripts/train1.py)

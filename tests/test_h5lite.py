@@ -1,8 +1,8 @@
 """h5lite: the package's own writer / reader of the HDF5 subset the reference's ``.ex`` files need (h5py and libhdf5 are
 not in the image).  The reader is pinned on a file libhdf5 itself produced; the writer is checked by that reader, by an
 independent structural walk of the bytes (B-tree key invariants, sorted symbol tables, sibling links, alignment, end-of-
-file address), through the three ``create_h5`` generators, and -- where /root/reference exists -- by the reference's own
-``TrainDataset`` / ``ValidateDataset`` with h5lite standing in for h5py."""
+file address), through the three ``create_h5`` generators, and -- where AEC_REFERENCE_DIR names a checkout of the
+reference -- by the reference's own ``TrainDataset`` / ``ValidateDataset`` with h5lite standing in for h5py."""
 import os
 import struct
 import subprocess
@@ -19,12 +19,8 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def _libhdf5_sample():
-    import scipy.io
-
-    p = os.path.join(os.path.dirname(scipy.io.__file__), "matlab", "tests", "data", "testhdf5_7.4_GLNX86.mat")
-    if not os.path.exists(p):
-        pytest.skip("scipy's test data (a libhdf5-written file) is not installed")
-    return p
+    # a copy of scipy's test file scipy/io/matlab/tests/data/testhdf5_7.4_GLNX86.mat (BSD-3-Clause), written by libhdf5
+    return os.path.join(ROOT, "tests", "golden", "testhdf5_7.4_GLNX86.mat")
 
 
 def test_reader_on_a_file_written_by_libhdf5():
@@ -265,7 +261,12 @@ def test_create_h5_writes_real_hdf5_without_h5py(tmp_path):
     assert sorted(z) == sorted(f"{g}/{k}" for g in range(3) for k in list(wav2h5.VAL_KEYS) + ["stage1_error", "stage1_echo"])
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/Stage2_lhm/scripts"), reason="the reference tree is not on this box")
+# a checkout of SZU-Speech/Acoustic-Echo-Cancellation; its sources are not part of this repository
+REFERENCE_SCRIPTS = os.path.join(os.environ.get("AEC_REFERENCE_DIR", ""), "Stage2_lhm", "scripts")
+
+
+@pytest.mark.skipif(not os.environ.get("AEC_REFERENCE_DIR") or not os.path.isdir(REFERENCE_SCRIPTS),
+                    reason="needs the reference's sources: set AEC_REFERENCE_DIR to a checkout of it")
 def test_reference_readers_open_the_generated_files(tmp_path):
     """a7 with the reference's OWN code: TrainDataset (train1.py:29-42) and ValidateDataset (test.py:19-33), imported
     unmodified in a subprocess with h5lite standing in for the absent h5py, read the files create_h5 wrote"""
@@ -276,7 +277,8 @@ def test_reference_readers_open_the_generated_files(tmp_path):
     tpath = wav2h5.create_h5(targs, runner=_fake_runner, batch=4, h5=h5lite)
     out = str(tmp_path / "read.npz")
     r = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "golden", "run_reference_readers.py"), ROOT,
-                        str(list_dir / "tr_list.txt"), tpath, out], capture_output=True, text=True, timeout=600)
+                        REFERENCE_SCRIPTS, str(list_dir / "tr_list.txt"), tpath, out],
+                       capture_output=True, text=True, timeout=600)
     assert r.returncode == 0, r.stderr[-2000:]
     z = np.load(out)
     f32 = lambda x: x.astype(np.float32) / np.float32(32768)            # noqa: E731
