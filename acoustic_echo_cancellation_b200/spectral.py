@@ -18,7 +18,7 @@ import numpy as np
 import torch
 
 from . import _lib
-from .stage1 import _require_cuda_f32, _stream_ptr, num_frames
+from .stage1 import _disjoint_rows, _require_cuda_f32, _stream_ptr, num_frames
 
 
 def _check_ctor(win_len, win_inc, fft_len, win_type, feature_type):
@@ -51,14 +51,15 @@ class ConvSTFT(torch.nn.Module):
                 raise ValueError("expected [B, 1, L]")
             inputs = inputs[:, 0]
         _require_cuda_f32("inputs", inputs)
-        x = inputs if inputs.stride(-1) == 1 else inputs.contiguous()
+        if inputs.dim() != 2:
+            raise ValueError("expected [B, L] or [B, 1, L]")
+        x, stride = _disjoint_rows(inputs)
         B, L = x.shape
         T = num_frames(L, self.win_len)
         K = self.win_len // 2 + 1
         with torch.cuda.device(x.device):
             spec = torch.empty((B, 2 * K, T), dtype=torch.float32, device=x.device)
-            rc = _lib.load().aec_stft(x.data_ptr(), spec.data_ptr(), B, L, max(x.stride(0), L) if B > 1 else L,
-                                      self.win_len, _stream_ptr(x))
+            rc = _lib.load().aec_stft(x.data_ptr(), spec.data_ptr(), B, L, stride, self.win_len, _stream_ptr(x))
         _lib.check(rc, "aec_stft")
         return spec
 
@@ -117,6 +118,7 @@ def batch_shift(x: torch.Tensor, out: torch.Tensor = None) -> torch.Tensor:
     _require_cuda_f32("x", x)
     if x.dim() != 2 or x.stride(1) != 1:
         raise ValueError("x must be [B, L] with unit inner stride")
+    x, stride = _disjoint_rows(x)
     lib = _lib.load()
     with torch.cuda.device(x.device):
         if out is None:
@@ -124,8 +126,7 @@ def batch_shift(x: torch.Tensor, out: torch.Tensor = None) -> torch.Tensor:
         nbytes = int(lib.aec_batch_shift_workspace_bytes())
         ws = torch.empty(nbytes // 8, dtype=torch.float64, device=x.device)
         B, L = x.shape
-        rc = lib.aec_batch_shift(x.data_ptr(), B, L, max(x.stride(0), L) if B > 1 else L, out.data_ptr(), ws.data_ptr(),
-                                 nbytes, _stream_ptr(x))
+        rc = lib.aec_batch_shift(x.data_ptr(), B, L, stride, out.data_ptr(), ws.data_ptr(), nbytes, _stream_ptr(x))
     _lib.check(rc, "aec_batch_shift")
     return out
 

@@ -76,6 +76,27 @@ def _require_cuda_f32(name: str, t: torch.Tensor) -> None:
         raise TypeError(f"{name} must be float32 (the reference stores float32 wav data)")
 
 
+def _disjoint_rows(x: torch.Tensor):
+    """``(x', row_stride)`` for a [B, L] tensor: ``x`` itself when its rows are unit-stride and do not overlap (a column
+    slice of a wider tensor keeps its stride, no copy), else ``x.contiguous()``.  Overlapping or broadcast rows
+    (``unfold`` / ``expand`` views: row stride < L) would otherwise be read as if they were ``max(stride, L)`` apart."""
+    B, L = x.shape
+    if x.stride(1) != 1 or (B > 1 and x.stride(0) < L):
+        x = x.contiguous()
+    return x, (x.stride(0) if B > 1 else L)
+
+
+def _shared_rows(far: torch.Tensor, mic: torch.Tensor):
+    """``(far', mic', row_stride)``: ``_disjoint_rows`` of both signals, which the stage-1 entries read with ONE row
+    stride; contiguous copies of both when their strides differ."""
+    far, fs = _disjoint_rows(far)
+    mic, ms = _disjoint_rows(mic)
+    if fs != ms:
+        far, mic = far.contiguous(), mic.contiguous()
+        fs = far.shape[1]
+    return far, mic, fs
+
+
 def stage1_aec(far: torch.Tensor, mic: torch.Tensor, cfg: Optional[Stage1Config] = None,
                n_samples: Optional[torch.Tensor] = None, return_echo: bool = False,
                return_erle: bool = False, out: Optional[torch.Tensor] = None):
@@ -95,10 +116,8 @@ def stage1_aec(far: torch.Tensor, mic: torch.Tensor, cfg: Optional[Stage1Config]
         far, mic = far[None], mic[None]
     if far.shape != mic.shape or far.dim() != 2 or far.device != mic.device:
         raise ValueError("far and mic must be [B, L] tensors of equal shape on one device")
-    if far.stride(1) != 1 or mic.stride(1) != 1 or far.stride(0) != mic.stride(0):
-        far, mic = far.contiguous(), mic.contiguous()
+    far, mic, in_stride = _shared_rows(far, mic)
     B, L = far.shape
-    in_stride = far.stride(0) if B > 1 else max(far.stride(0), L)
     lib = _lib.load()
     with torch.cuda.device(far.device):
         if out is None:
@@ -157,11 +176,9 @@ def stage1_aec_features(far: torch.Tensor, mic: torch.Tensor, erb: torch.Tensor,
         if int(span.clamp(min=0).sum()) > 512:
             raise ValueError("the ERB bank has more than 512 coefficients inside its bands' non-zero ranges")
         _checked_banks.add(key)
-    if far.stride(1) != 1 or mic.stride(1) != 1 or far.stride(0) != mic.stride(0):
-        far, mic = far.contiguous(), mic.contiguous()
+    far, mic, in_stride = _shared_rows(far, mic)
     erb = erb.contiguous()
     B, L = far.shape
-    in_stride = far.stride(0) if B > 1 else max(far.stride(0), L)
     lib = _lib.load()
     with torch.cuda.device(far.device):
         if out is None:

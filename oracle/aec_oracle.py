@@ -448,19 +448,22 @@ def stage2_features(mic: np.ndarray, ref: np.ndarray, erb: np.ndarray,
 
 
 def stage2_little_net(mic: np.ndarray, ref: np.ndarray, erb: np.ndarray, w: dict,
-                      frame: int = WIN_SIZE, hop: int = HOP_SIZE, dtype=np.float64) -> np.ndarray:
+                      frame: int = WIN_SIZE, hop: int = HOP_SIZE, dtype=np.float64,
+                      in_norm: bool = True) -> np.ndarray:
     """Inference path of the reference's live Stage-2 model ``Little_net.forward``
     (network/ERB.py:252-316; pinned by tests/golden/reference_stage2.npz, produced by running the
     reference module itself).  ``w`` holds the state_dict arrays ``gru1_weight_ih_l0`` [96,64],
     ``gru1_weight_hh_l0`` [96,32], ``gru1_bias_ih_l0``, ``gru1_bias_hh_l0`` (PyTorch gate order r, z, n),
     ``linear1_weight`` [32,64], ``linear1_bias``, ``linear2_weight`` [32,32], ``linear2_bias``.
-    Returns ``out_wav`` [B, (T-1)*hop]."""
+    ``in_norm=False`` skips the batch-global shift (as ``stage2_features`` does): each row is then independent of the
+    others.  Returns ``out_wav`` [B, (T-1)*hop]."""
     mic = np.atleast_2d(np.asarray(mic, dtype=dtype))
     ref = np.atleast_2d(np.asarray(ref, dtype=dtype))
     erb = np.asarray(erb, dtype=dtype)
     g = {k: np.asarray(v, dtype=dtype) for k, v in w.items()}
-    mic = mic - mic.mean() / mic.std(ddof=1)                               # ERB.py:254
-    ref = ref - ref.mean() / ref.std(ddof=1)                               # ERB.py:255
+    if in_norm:
+        mic = mic - mic.mean() / mic.std(ddof=1)                           # ERB.py:254
+        ref = ref - ref.mean() / ref.std(ddof=1)                           # ERB.py:255
     M = stft_complex(mic, frame, hop, dtype)                               # ERB.py:263
     R = stft_complex(ref, frame, hop, dtype)                               # ERB.py:264
     merb = np.sqrt(M.real ** 2 + M.imag ** 2 + 1e-9) @ erb                 # ERB.py:277, 282

@@ -392,3 +392,38 @@ def test_stage1_batch_sends_exact_pcm16_as_int16_and_everything_else_as_float32(
     assert seen["dtype"] == np.float32
     assert wav2h5.as_pcm16(np.array([1.0], dtype=np.float32)) is None          # +1.0 would be 32768: out of range
     assert wav2h5.as_pcm16(np.array([-1.0, 0.5], dtype=np.float32)).tolist() == [-32768, 16384]
+
+
+def test_row_stride_helper_copies_overlapping_rows_only():
+    """the [B, L] row handling of ConvSTFT, batch_shift and the stage-1 entries: the kernels read row b at
+    b * row_stride, so rows that overlap or are broadcast (row stride < L) must become a copy, while disjoint
+    unit-stride rows (a column slice of a wider tensor) go through as they are, with their own stride"""
+    from acoustic_echo_cancellation_b200.stage1 import _disjoint_rows, _shared_rows
+
+    sig = torch.arange(20000, dtype=torch.float32)
+    chunks = sig.unfold(0, 4096, 1000)                     # chunks of a long recording: rows 1000 apart, 4096 long
+    assert chunks.stride() == (1000, 1)
+    x, s = _disjoint_rows(chunks)
+    assert s == 4096 and x.stride() == (4096, 1) and x.data_ptr() != chunks.data_ptr() and torch.equal(x, chunks)
+    rep = sig[:513].expand(5, 513)                         # one signal broadcast to five rows
+    assert rep.stride() == (0, 1)
+    x, s = _disjoint_rows(rep)
+    assert s == 513 and x.stride() == (513, 1) and torch.equal(x, rep)
+    wide = torch.arange(4 * 700, dtype=torch.float32).reshape(4, 700)
+    cols = wide[:, 3:515]                                  # disjoint rows 700 apart: no copy
+    x, s = _disjoint_rows(cols)
+    assert x is cols and s == 700
+    for one in (wide[1:2, 3:515], chunks[2:3], rep[:1]):  # one row: its stride is never used, no copy
+        x, s = _disjoint_rows(one)
+        assert x is one and s == one.shape[1]
+    for strided in (wide[:, ::2], wide[:1, ::2]):         # non-unit inner stride: copy
+        x, s = _disjoint_rows(strided)
+        assert x.is_contiguous() and s == 350 and torch.equal(x, strided)
+    assert _disjoint_rows(torch.zeros(6, 1))[1] == 1
+    # the stage-1 entries take one stride for both signals: kept when they agree, contiguous copies when not
+    far, mic, s = _shared_rows(cols, wide[:, 100:612])
+    assert far is cols and s == 700 and mic.data_ptr() == wide[:, 100:612].data_ptr()
+    far, mic, s = _shared_rows(cols, torch.zeros(4, 512))
+    assert s == 512 and far.is_contiguous() and torch.equal(far, cols) and mic.is_contiguous()
+    far, mic, s = _shared_rows(chunks[:4, :512], cols)
+    assert s == 512 and far.is_contiguous() and mic.is_contiguous() and torch.equal(far, chunks[:4, :512])
