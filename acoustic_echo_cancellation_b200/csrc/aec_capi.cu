@@ -368,17 +368,22 @@ static int stage1_run_impl(const float* far, const float* mic, float* err, float
         // (defaults: the first instantiation listed for (P, algo, echo) in stage1_inst_nw*.cu --
         //  128 registers for the two-warp kernels so that 7 utterances stay resident per SM)
     }
+    // A variant names one build: a warp count the selected kernel does not have is refused, never silently replaced.
     cudaError_t e;
     if (cfg->algo == AEC_ALGO_PBFDAF || cfg->algo == AEC_ALGO_PBFKF) {
         if (feat) return AEC_EUNSUPPORTED;               // no fused features for the overlap-save filters
         if (wide) {
             if (cfg->variant > 0) return AEC_EUNSUPPORTED;
             e = launch_stage1_ols1024(P, cfg->algo == AEC_ALGO_PBFKF, echo, p, s);
-        } else
-            e = launch_stage1_ols(P, cfg->algo == AEC_ALGO_PBFKF, echo, cfg->variant > 0 ? cfg->variant % 1000 : 0, p, s);
+        } else {
+            if (cfg->variant > 0 && nw != ols_warps(P)) return AEC_EUNSUPPORTED;   // the warp count follows from P
+            e = launch_stage1_ols(P, cfg->algo == AEC_ALGO_PBFKF, echo, minb, p, s);
+        }
     } else if (feat) {
+        if (cfg->variant > 0) return AEC_EUNSUPPORTED;   // the feature build is chosen from the batch size
         e = launch_stage1_feat(P, cfg->algo, p, s);
     } else if (wide) {
+        if (cfg->variant > 0 && nw != 8) return AEC_EUNSUPPORTED;                // eight warps per utterance
         e = launch_stage1_1024(P, cfg->algo, echo, minb, p, s);
     } else
     switch (nw) {

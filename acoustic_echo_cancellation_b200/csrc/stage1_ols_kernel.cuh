@@ -162,9 +162,11 @@ __device__ __forceinline__ void ols_mid_parallel(int p, int t, float2* midW, flo
 // do the split of the pair and keep their own bin, and swap their results by shuffle for the packing).  The transform
 // phase is the same for all of them (one warp carries the chain, one the far-end transforms); the roles rotate over all
 // warps of the CTA.
+__host__ __device__ constexpr int ols_warps(int P) { return P <= 4 ? 2 : P / 2; }
+
 template <int P>
 struct OlsShape {
-    static constexpr int NW = P <= 4 ? 2 : P / 2;
+    static constexpr int NW = ols_warps(P);
     static constexpr int NT = 32 * NW;
     static constexpr bool kSplit = (NW == 8);
     static constexpr int PPT = kSplit ? 1 : 128 / NT;      // pair slots per thread

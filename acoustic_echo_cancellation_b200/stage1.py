@@ -24,7 +24,12 @@ from ._lib import ALGO_KALMAN, ALGO_NLMS, ALGO_PBFDAF, ALGO_PBFKF  # noqa: F401 
 @dataclass
 class Stage1Config:
     """Python mirror of ``aec_cfg``.  ``frame``/``hop`` follow ``speech_conf``
-    (Stage2_lhm/scripts/configs.py:1-8); ``delta=None`` means 1e-6 * frame."""
+    (Stage2_lhm/scripts/configs.py:1-8); ``delta=None`` means 1e-6 * frame.
+
+    ``variant`` picks one compiled kernel build for A/B timing: ``1000 * warps_per_utterance + register cap`` (e.g.
+    2168), 0 = the library default.  A build that was not compiled for (frame, partitions, algo, echo output) raises
+    ``AecError`` with code -2 instead of running another one; ``stage1_aec_features`` and the frame-1024
+    overlap-save filters take only ``variant=0``."""
 
     frame: int = 512
     partitions: int = 4

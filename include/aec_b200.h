@@ -67,7 +67,11 @@ typedef struct aec_cfg {
     float kalman_c0;        /* initial covariance                  (default 1) */
     float kalman_eps;       /* floor added to the innovation power (default 1e-10) */
     int32_t erle_skip_hops; /* hops excluded from the ERLE sums at the start of each utterance */
-    int32_t variant;        /* 0 = library default; otherwise 1000*warps_per_utterance + register cap (DESIGN.md) */
+    int32_t variant;        /* 0 = library default; otherwise 1000*warps_per_utterance + register cap of one built kernel
+                             * (DESIGN.md; e.g. 2168).  A warp count or cap that (frame, partitions, algo, echo) was not
+                             * built with returns AEC_EUNSUPPORTED: the overlap-save kernels take 2 warps up to 4
+                             * partitions and P / 2 above, the frame-1024 STFT-domain kernel 8; the frame-1024 overlap-save
+                             * path and aec_stage1_run_features (build chosen from the batch size) take no variant. */
     int32_t stagger_ns;     /* tuning: start-up skew (ns per resident slot) between co-resident utterances; <= 0 = off (default) */
     float pb_lambda;        /* algo 2: smoothing of the per-bin input power (default 0.5) */
     int32_t reserved[3];

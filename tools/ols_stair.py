@@ -1,4 +1,7 @@
-"""Launch time of the overlap-save kernel against the number of resident utterances per SM (1 .. 9 x 148)."""
+"""Launch time of the overlap-save kernel against the number of resident utterances per SM (1 .. 9 x 148).
+    python tools/ols_stair.py [algo] [P] [variant] [counts]
+variant: 0 (default build) or the full 1000 * warps + register cap, e.g. 2168 at P <= 4 (2 warps), 4128 at P = 8,
+8128 at P = 16; a bare register cap such as 168 is refused."""
 import os
 import sys
 
