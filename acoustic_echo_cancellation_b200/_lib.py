@@ -40,6 +40,12 @@ class AecCfg(C.Structure):
     ]
 
 
+class AecDelayCfg(C.Structure):
+    """Mirror of ``struct aec_delay_cfg`` (include/aec_b200.h)."""
+
+    _fields_ = [("max_delay", C.c_int32), ("margin", C.c_int32), ("min_peak", C.c_float), ("reserved", C.c_int32 * 5)]
+
+
 class AecError(RuntimeError):
     def __init__(self, code: int, what: str):
         self.code = code
@@ -81,6 +87,13 @@ SIGNATURES = {
     "aec_host_ctx_wait": (C.c_int, [_P]),
     "aec_stage1_run_host": (C.c_int, [_P, _P, _P, _P, _P, _P, _P, _I64, _I64, _I64, _I64, C.POINTER(AecCfg)]),
     "aec_stage1_run_host_pcm16": (C.c_int, [_P, _P, _P, _P, _P, _P, _P, _I64, _I64, _I64, _I64, C.POINTER(AecCfg)]),
+    "aec_stage1_run_host_ex": (C.c_int, [_P, _P, _P, _P, _P, _P, _P, _I64, _I64, _I64, _I64, C.POINTER(AecCfg),
+                                         C.POINTER(AecDelayCfg), _P, _P]),
+    "aec_stage1_run_host_pcm16_ex": (C.c_int, [_P, _P, _P, _P, _P, _P, _P, _I64, _I64, _I64, _I64, C.POINTER(AecCfg),
+                                               C.POINTER(AecDelayCfg), _P, _P]),
+    "aec_delay_cfg_default": (C.c_int, [C.POINTER(AecDelayCfg)]),
+    "aec_delay_estimate": (C.c_int, [_P, _P, _P, _I64, _I64, _I64, C.POINTER(AecDelayCfg), _P, _P, _P, _P, _P]),
+    "aec_delay_align": (C.c_int, [_P, _P, _P, _I64, _I64, _I64, _I64, _P]),
     "aec_host_alloc": (C.c_int, [C.POINTER(_P), _I64]),
     "aec_host_alloc_ex": (C.c_int, [C.POINTER(_P), _I64, _I32]),
     "aec_host_free": (C.c_int, [_P]),

@@ -441,13 +441,20 @@ struct aec_host_ctx {
     float* d_erle[kMaxSlots] = {};
     long long* d_n[kMaxSlots] = {};
     int16_t* d_pcm[kMaxSlots] = {};    // [2 signals][slice][stride] int16 staging (allocated on first use)
+    float* d_falign[kMaxSlots] = {};   // aligned far end, allocated on the first call that aligns
+    int32_t* d_shift[kMaxSlots] = {};  // per-utterance shift / peak of the aligned calls (with d_falign)
+    float* d_peak[kMaxSlots] = {};
     // page-locked staging for the small per-utterance arrays: a copy to / from pageable host memory
     // would serialise the multi-stream pipeline
     float* h_erle[kMaxSlots] = {};
     long long* h_n[kMaxSlots] = {};
-    int64_t pending_off[kMaxSlots];    // slice whose ERLE still sits in h_erle[k] (-1: none)
+    int32_t* h_shift[kMaxSlots] = {};  // (with d_falign)
+    float* h_peak[kMaxSlots] = {};
+    int64_t pending_off[kMaxSlots];    // slice whose ERLE / shift / peak still sit in h_erle[k] .. (-1: none)
     int64_t pending_nb[kMaxSlots] = {};
     float* pending_dst[kMaxSlots] = {}; // ... and the caller's erle_db array it belongs to (calls may overlap: deferred mode)
+    int32_t* pending_shift[kMaxSlots] = {};   // ... the caller's shift_out / peak_out arrays
+    float* pending_peak[kMaxSlots] = {};
     int deferred = 0;                  // 1: a run call returns without waiting for its last slices (aec_host_ctx_wait does)
     aec_host_ctx() {
         for (int i = 0; i < kMaxSlots; ++i) pending_off[i] = -1;
@@ -471,10 +478,16 @@ static int64_t host_slice(const aec_host_ctx* ctx, int64_t done, int64_t remaini
 // drain slot k: wait for its stream, hand the staged ERLE values to the caller (of the call that produced them)
 static int host_ctx_drain(aec_host_ctx* ctx, int k) {
     const cudaError_t e = cudaStreamSynchronize(ctx->stream[k]);
-    if (e == cudaSuccess && ctx->pending_dst[k] && ctx->pending_off[k] >= 0)
-        memcpy(ctx->pending_dst[k] + ctx->pending_off[k], ctx->h_erle[k], (size_t)ctx->pending_nb[k] * sizeof(float));
+    if (e == cudaSuccess && ctx->pending_off[k] >= 0) {
+        const int64_t off = ctx->pending_off[k], nb = ctx->pending_nb[k];
+        if (ctx->pending_dst[k]) memcpy(ctx->pending_dst[k] + off, ctx->h_erle[k], (size_t)nb * sizeof(float));
+        if (ctx->pending_shift[k]) memcpy(ctx->pending_shift[k] + off, ctx->h_shift[k], (size_t)nb * sizeof(int32_t));
+        if (ctx->pending_peak[k]) memcpy(ctx->pending_peak[k] + off, ctx->h_peak[k], (size_t)nb * sizeof(float));
+    }
     ctx->pending_off[k] = -1;
     ctx->pending_dst[k] = nullptr;
+    ctx->pending_shift[k] = nullptr;
+    ctx->pending_peak[k] = nullptr;
     if (e != cudaSuccess) {
         set_cuda_error(e, "aec_stage1_run_host: cudaStreamSynchronize");
         return AEC_ECUDA;
@@ -489,6 +502,8 @@ static void host_ctx_quiesce(aec_host_ctx* ctx) {
         if (ctx->stream[i]) (void)cudaStreamSynchronize(ctx->stream[i]);
         ctx->pending_off[i] = -1;
         ctx->pending_dst[i] = nullptr;
+        ctx->pending_shift[i] = nullptr;
+        ctx->pending_peak[i] = nullptr;
     }
     (void)cudaGetLastError();
 }
@@ -507,8 +522,13 @@ extern "C" int aec_host_ctx_destroy(aec_host_ctx* ctx) {
         cudaFree(ctx->d_erle[i]);
         cudaFree(ctx->d_n[i]);
         cudaFree(ctx->d_pcm[i]);
+        cudaFree(ctx->d_falign[i]);
+        cudaFree(ctx->d_shift[i]);
+        cudaFree(ctx->d_peak[i]);
         cudaFreeHost(ctx->h_erle[i]);
         cudaFreeHost(ctx->h_n[i]);
+        cudaFreeHost(ctx->h_shift[i]);
+        cudaFreeHost(ctx->h_peak[i]);
         if (ctx->stream[i]) cudaStreamDestroy(ctx->stream[i]);
     }
     if (prev >= 0) (void)cudaSetDevice(prev);
@@ -575,15 +595,21 @@ extern "C" int aec_host_ctx_create(aec_host_ctx** out, int64_t slice_utterances,
 
 namespace {
 // One body for both host entries: In = float (samples as librosa.load returns them) or int16_t (the PCM the wav
-// files hold; converted on the GPU).
+// files hold; converted on the GPU).  align = NULL: no delay estimate, no copies or launches beyond stage 1's.
 template <typename In>
 int run_host_impl(aec_host_ctx* ctx, const In* far, const In* mic, float* err, float* echo_est, float* erle_db,
                   const int64_t* n_samples, int64_t B, int64_t L, int64_t in_stride, int64_t out_stride,
-                  const aec_cfg* cfg) {
+                  const aec_cfg* cfg, const aec_delay_cfg* align, int32_t* shift_out, float* peak_out) {
     constexpr bool kPcm = std::is_same<In, int16_t>::value;
     if (!ctx) return AEC_EINVAL;
     int rc = validate_cfg(cfg);
     if (rc != AEC_OK) return rc;
+    if (align) {
+        rc = validate_delay_cfg(align);
+        if (rc != AEC_OK) return rc;
+    } else if (shift_out || peak_out) {
+        return AEC_EINVAL;
+    }
     if (B < 0 || L < 0 || L > ctx->max_samples || in_stride < L || out_stride < L) return AEC_EINVAL;
     if (B == 0) return AEC_OK;
     if (!far || !mic || !err) return AEC_EINVAL;
@@ -594,6 +620,13 @@ int run_host_impl(aec_host_ctx* ctx, const In* far, const In* mic, float* err, f
     for (int i = 0; i < ctx->slots; ++i) {
         if (echo_est && !ctx->d_echo[i]) AEC_CUDA_CHECK(cudaMalloc(&ctx->d_echo[i], sig_elems * sizeof(float)));
         if (kPcm && !ctx->d_pcm[i]) AEC_CUDA_CHECK(cudaMalloc(&ctx->d_pcm[i], 2 * sig_elems * sizeof(int16_t)));
+        if (align && !ctx->d_falign[i]) {
+            AEC_CUDA_CHECK(cudaMalloc(&ctx->d_falign[i], sig_elems * sizeof(float)));
+            AEC_CUDA_CHECK(cudaMalloc(&ctx->d_shift[i], (size_t)ctx->slice * sizeof(int32_t)));
+            AEC_CUDA_CHECK(cudaMalloc(&ctx->d_peak[i], (size_t)ctx->slice * sizeof(float)));
+            AEC_CUDA_CHECK(cudaHostAlloc(&ctx->h_shift[i], (size_t)ctx->slice * sizeof(int32_t), cudaHostAllocDefault));
+            AEC_CUDA_CHECK(cudaHostAlloc(&ctx->h_peak[i], (size_t)ctx->slice * sizeof(float), cudaHostAllocDefault));
+        }
     }
     int sms = 148;
     (void)cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, ctx->device);
@@ -639,10 +672,18 @@ int run_host_impl(aec_host_ctx* ctx, const In* far, const In* mic, float* err, f
             if (!ok(cudaMemcpyAsync(ctx->d_n[k], ctx->h_n[k], (size_t)nb * sizeof(int64_t), cudaMemcpyHostToDevice, s)))
                 break;
         }
-        rc = aec_stage1_run(ctx->d_far[k], ctx->d_mic[k], ctx->d_err[k], echo_est ? ctx->d_echo[k] : nullptr,
-                            erle_db ? ctx->d_erle[k] : nullptr,
-                            n_samples ? reinterpret_cast<const int64_t*>(ctx->d_n[k]) : nullptr, nb, L, ctx->stride,
-                            ctx->stride, cfg, s);
+        const int64_t* d_n = n_samples ? reinterpret_cast<const int64_t*>(ctx->d_n[k]) : nullptr;
+        const float* far_s1 = ctx->d_far[k];
+        if (align) {
+            rc = aec_delay_estimate(ctx->d_far[k], ctx->d_mic[k], d_n, nb, L, ctx->stride, align, nullptr,
+                                    ctx->d_shift[k], ctx->d_peak[k], nullptr, s);
+            if (rc == AEC_OK)
+                rc = aec_delay_align(ctx->d_far[k], ctx->d_falign[k], ctx->d_shift[k], nb, L, ctx->stride, ctx->stride, s);
+            if (rc != AEC_OK) break;
+            far_s1 = ctx->d_falign[k];
+        }
+        rc = aec_stage1_run(far_s1, ctx->d_mic[k], ctx->d_err[k], echo_est ? ctx->d_echo[k] : nullptr,
+                            erle_db ? ctx->d_erle[k] : nullptr, d_n, nb, L, ctx->stride, ctx->stride, cfg, s);
         if (rc != AEC_OK) break;
         if (lin_out) {
             ok(cudaMemcpyAsync(err + off * out_stride, ctx->d_err[k], out_row * (size_t)nb, cudaMemcpyDeviceToHost, s));
@@ -658,9 +699,19 @@ int run_host_impl(aec_host_ctx* ctx, const In* far, const In* mic, float* err, f
         }
         if (erle_db) {
             ok(cudaMemcpyAsync(ctx->h_erle[k], ctx->d_erle[k], (size_t)nb * sizeof(float), cudaMemcpyDeviceToHost, s));
+            ctx->pending_dst[k] = erle_db;
+        }
+        if (shift_out) {
+            ok(cudaMemcpyAsync(ctx->h_shift[k], ctx->d_shift[k], (size_t)nb * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+            ctx->pending_shift[k] = shift_out;
+        }
+        if (peak_out) {
+            ok(cudaMemcpyAsync(ctx->h_peak[k], ctx->d_peak[k], (size_t)nb * sizeof(float), cudaMemcpyDeviceToHost, s));
+            ctx->pending_peak[k] = peak_out;
+        }
+        if (erle_db || shift_out || peak_out) {
             ctx->pending_off[k] = off;
             ctx->pending_nb[k] = nb;
-            ctx->pending_dst[k] = erle_db;
         }
     }
     if (e != cudaSuccess) {
@@ -679,13 +730,31 @@ int run_host_impl(aec_host_ctx* ctx, const In* far, const In* mic, float* err, f
 extern "C" int aec_stage1_run_host(aec_host_ctx* ctx, const float* far, const float* mic, float* err, float* echo_est,
                                    float* erle_db, const int64_t* n_samples, int64_t B, int64_t L, int64_t in_stride,
                                    int64_t out_stride, const aec_cfg* cfg) {
-    return run_host_impl<float>(ctx, far, mic, err, echo_est, erle_db, n_samples, B, L, in_stride, out_stride, cfg);
+    return run_host_impl<float>(ctx, far, mic, err, echo_est, erle_db, n_samples, B, L, in_stride, out_stride, cfg,
+                                nullptr, nullptr, nullptr);
+}
+
+extern "C" int aec_stage1_run_host_ex(aec_host_ctx* ctx, const float* far, const float* mic, float* err,
+                                      float* echo_est, float* erle_db, const int64_t* n_samples, int64_t B, int64_t L,
+                                      int64_t in_stride, int64_t out_stride, const aec_cfg* cfg,
+                                      const aec_delay_cfg* align, int32_t* shift_out, float* peak_out) {
+    return run_host_impl<float>(ctx, far, mic, err, echo_est, erle_db, n_samples, B, L, in_stride, out_stride, cfg,
+                                align, shift_out, peak_out);
 }
 
 extern "C" int aec_stage1_run_host_pcm16(aec_host_ctx* ctx, const int16_t* far, const int16_t* mic, float* err,
                                          float* echo_est, float* erle_db, const int64_t* n_samples, int64_t B,
                                          int64_t L, int64_t in_stride, int64_t out_stride, const aec_cfg* cfg) {
-    return run_host_impl<int16_t>(ctx, far, mic, err, echo_est, erle_db, n_samples, B, L, in_stride, out_stride, cfg);
+    return run_host_impl<int16_t>(ctx, far, mic, err, echo_est, erle_db, n_samples, B, L, in_stride, out_stride, cfg,
+                                  nullptr, nullptr, nullptr);
+}
+
+extern "C" int aec_stage1_run_host_pcm16_ex(aec_host_ctx* ctx, const int16_t* far, const int16_t* mic, float* err,
+                                            float* echo_est, float* erle_db, const int64_t* n_samples, int64_t B,
+                                            int64_t L, int64_t in_stride, int64_t out_stride, const aec_cfg* cfg,
+                                            const aec_delay_cfg* align, int32_t* shift_out, float* peak_out) {
+    return run_host_impl<int16_t>(ctx, far, mic, err, echo_est, erle_db, n_samples, B, L, in_stride, out_stride, cfg,
+                                  align, shift_out, peak_out);
 }
 
 extern "C" int aec_host_alloc_ex(void** ptr, int64_t bytes, int32_t flags) {

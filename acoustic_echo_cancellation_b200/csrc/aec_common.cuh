@@ -28,6 +28,8 @@ int get_tables(Tables* out);
 
 void set_cuda_error(cudaError_t e, const char* where);
 void count_launch(int n = 1);
+// AEC_OK or AEC_EINVAL for an aec_delay_cfg (aec_delay.cu)
+int validate_delay_cfg(const aec_delay_cfg* dcfg);
 
 #define AEC_CUDA_CHECK(expr)                          \
     do {                                              \

@@ -59,6 +59,24 @@ class Stage1Config:
             stagger_ns=self.stagger_ns)
 
 
+@dataclass
+class DelayConfig:
+    """Python mirror of ``aec_delay_cfg``: far-end bulk-delay estimation (GCC-PHAT over the whole utterance) and the
+    shift applied to the far end before stage 1.  ``max_delay`` D: largest lag searched, a power of two in [256, 8192]
+    (8192 = 512 ms at 16 kHz); ``margin``: samples of echo path kept in front of the estimated delay; ``min_peak``:
+    normalised correlation peak below which the far end is not shifted (DESIGN.md "Far-end delay estimation")."""
+
+    max_delay: int = 8192
+    margin: int = 128
+    min_peak: float = 0.1
+
+    def to_c(self) -> _lib.AecDelayCfg:
+        c = _lib.AecDelayCfg()
+        _lib.check(_lib.load().aec_delay_cfg_default(C.byref(c)), "aec_delay_cfg_default")
+        c.max_delay, c.margin, c.min_peak = int(self.max_delay), int(self.margin), float(self.min_peak)
+        return c
+
+
 def num_frames(n_samples: int, frame: int = 512) -> int:
     """Frame count of the reference STFT (attention_ccrn.py:48-49)."""
     return int(_lib.load().aec_num_frames(int(n_samples), int(frame)))
@@ -102,25 +120,110 @@ def _shared_rows(far: torch.Tensor, mic: torch.Tensor):
     return far, mic, fs
 
 
-def stage1_aec(far: torch.Tensor, mic: torch.Tensor, cfg: Optional[Stage1Config] = None,
-               n_samples: Optional[torch.Tensor] = None, return_echo: bool = False,
-               return_erle: bool = False, out: Optional[torch.Tensor] = None):
-    """Run the stage-1 canceller on a batch of CUDA tensors.
+def _device_lengths(n_samples: Optional[torch.Tensor], B: int, device):
+    """``(n_samples as a contiguous int64 CUDA tensor, its pointer)``, or ``(None, None)``."""
+    if n_samples is None:
+        return None, None
+    n_samples = n_samples.to(device=device, dtype=torch.int64).contiguous()
+    if n_samples.numel() != B:
+        raise ValueError("n_samples must have B entries")
+    return n_samples, n_samples.data_ptr()
 
-    far, mic : [B, L] float32 CUDA (``farend_speech`` / ``nearend_mic`` rows)
-    n_samples: optional int64 [B] true lengths (ragged batch, zero-padded to L as the
-               reference's ``collate_fn`` does, Stage2_lhm/scripts/train1.py:52-61)
-    Returns ``err`` [B, L] (zero beyond ``out_samples(n_b)``), plus ``echo`` [B, L] and/or
-    ``erle_db`` [B] when requested (in that order).
-    The call is asynchronous on the current stream of ``far.device``.
-    """
-    cfg = cfg or Stage1Config()
+
+def _pair(far: torch.Tensor, mic: torch.Tensor):
     _require_cuda_f32("far", far)
     _require_cuda_f32("mic", mic)
     if far.dim() == 1:
         far, mic = far[None], mic[None]
     if far.shape != mic.shape or far.dim() != 2 or far.device != mic.device:
         raise ValueError("far and mic must be [B, L] tensors of equal shape on one device")
+    return far, mic
+
+
+def estimate_delay(far: torch.Tensor, mic: torch.Tensor, cfg: Optional[DelayConfig] = None,
+                   n_samples: Optional[torch.Tensor] = None, return_corr: bool = False):
+    """Far-end bulk delay of every utterance (``aec_delay_estimate``): GCC-PHAT of ``mic`` against ``far`` at lags
+    0 .. ``cfg.max_delay``.
+
+    far, mic : [B, L] float32 CUDA;  n_samples: optional int64 [B] true lengths.
+    Returns CUDA tensors ``(delay int32 [B], shift int32 [B], peak float32 [B])``, plus ``corr`` [B, D + 1] (the
+    normalised correlation r) with ``return_corr``.  ``shift`` is what ``align_far`` delays the far end by.
+    Asynchronous on the current stream of ``far.device``."""
+    cfg = cfg or DelayConfig()
+    far, mic = _pair(far, mic)
+    far, mic, in_stride = _shared_rows(far, mic)
+    B, L = far.shape
+    c = cfg.to_c()
+    with torch.cuda.device(far.device):
+        delay = torch.empty((B,), dtype=torch.int32, device=far.device)
+        shift = torch.empty_like(delay)
+        peak = torch.empty((B,), dtype=torch.float32, device=far.device)
+        corr = torch.empty((B, int(cfg.max_delay) + 1), dtype=torch.float32, device=far.device) if return_corr else None
+        n_samples, ns_ptr = _device_lengths(n_samples, B, far.device)
+        rc = _lib.load().aec_delay_estimate(far.data_ptr(), mic.data_ptr(), ns_ptr, B, L, in_stride, C.byref(c),
+                                            delay.data_ptr(), shift.data_ptr(), peak.data_ptr(),
+                                            corr.data_ptr() if corr is not None else None, _stream_ptr(far))
+        _lib.check(rc, "aec_delay_estimate")
+    return (delay, shift, peak, corr) if return_corr else (delay, shift, peak)
+
+
+def align_far(far: torch.Tensor, shift: torch.Tensor, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """``out[b, n] = far[b, n - shift[b]]`` for ``n >= shift[b]``, 0 below (``aec_delay_align``); rows keep their
+    length L.  far: [B, L] float32 CUDA; shift: int [B] (``estimate_delay``'s, or any).  ``out`` must not overlap far."""
+    _require_cuda_f32("far", far)
+    squeeze = far.dim() == 1
+    if squeeze:
+        far = far[None]
+    if far.dim() != 2:
+        raise ValueError("far must be a [B, L] tensor")
+    far, in_stride = _disjoint_rows(far)
+    B, L = far.shape
+    shift = shift.to(device=far.device, dtype=torch.int32).reshape(-1).contiguous()
+    if shift.numel() != B:
+        raise ValueError("shift must have B entries")
+    with torch.cuda.device(far.device):
+        if out is None:
+            out = torch.empty((B, L), dtype=torch.float32, device=far.device)
+        else:
+            if squeeze and out.dim() == 1:
+                out = out[None]
+            if out.shape != (B, L) or not out.is_cuda or out.dtype != torch.float32 or out.stride(1) != 1 \
+                    or (B > 1 and out.stride(0) < L):
+                raise ValueError("out must be a [B, L] float32 CUDA tensor with disjoint unit-stride rows")
+        out_stride = out.stride(0) if B > 1 else max(out.stride(0), L)
+        rc = _lib.load().aec_delay_align(far.data_ptr(), out.data_ptr(), shift.data_ptr(), B, L, in_stride, out_stride,
+                                         _stream_ptr(far))
+        _lib.check(rc, "aec_delay_align")
+    return out[0] if squeeze else out
+
+
+def stage1_aec(far: torch.Tensor, mic: torch.Tensor, cfg: Optional[Stage1Config] = None,
+               n_samples: Optional[torch.Tensor] = None, return_echo: bool = False,
+               return_erle: bool = False, out: Optional[torch.Tensor] = None,
+               align: Optional[DelayConfig] = None, return_shift: bool = False):
+    """Run the stage-1 canceller on a batch of CUDA tensors.
+
+    far, mic : [B, L] float32 CUDA (``farend_speech`` / ``nearend_mic`` rows)
+    n_samples: optional int64 [B] true lengths (ragged batch, zero-padded to L as the
+               reference's ``collate_fn`` does, Stage2_lhm/scripts/train1.py:52-61)
+    align    : optional ``DelayConfig``: estimate each utterance's far-end delay and run stage 1 on the far end
+               delayed by the resulting shift (``estimate_delay`` + ``align_far`` into a temporary buffer); off by
+               default.  ``return_shift`` (needs ``align``) also returns that shift, int32 [B].
+    Returns ``err`` [B, L] (zero beyond ``out_samples(n_b)``), plus ``echo`` [B, L], ``erle_db`` [B] and
+    ``shift`` [B] when requested (in that order).
+    The call is asynchronous on the current stream of ``far.device``.
+    """
+    cfg = cfg or Stage1Config()
+    if return_shift and align is None:
+        raise ValueError("return_shift needs align")
+    far, mic = _pair(far, mic)
+    shift = None
+    if align is not None:
+        _, shift, _ = estimate_delay(far, mic, align, n_samples)
+        mic, m_stride = _disjoint_rows(mic)
+        with torch.cuda.device(far.device):
+            buf = torch.empty((far.shape[0], m_stride), dtype=torch.float32, device=far.device)
+        far = align_far(far, shift, out=buf[:, :far.shape[1]])      # rows spaced like mic's: no copy of mic below
     far, mic, in_stride = _shared_rows(far, mic)
     B, L = far.shape
     lib = _lib.load()
@@ -131,12 +234,7 @@ def stage1_aec(far: torch.Tensor, mic: torch.Tensor, cfg: Optional[Stage1Config]
             raise ValueError("out must be a [B, L] float32 CUDA tensor with unit inner stride")
         echo = torch.empty_like(out) if return_echo else None
         erle = torch.empty((B,), dtype=torch.float32, device=far.device) if return_erle else None
-        ns_ptr = None
-        if n_samples is not None:
-            n_samples = n_samples.to(device=far.device, dtype=torch.int64).contiguous()
-            if n_samples.numel() != B:
-                raise ValueError("n_samples must have B entries")
-            ns_ptr = n_samples.data_ptr()
+        n_samples, ns_ptr = _device_lengths(n_samples, B, far.device)
         out_stride = out.stride(0) if B > 1 else max(out.stride(0), L)
         if echo is not None and echo.stride(0) != out.stride(0):
             echo = torch.empty_strided(out.shape, out.stride(), dtype=torch.float32, device=far.device)
@@ -151,6 +249,8 @@ def stage1_aec(far: torch.Tensor, mic: torch.Tensor, cfg: Optional[Stage1Config]
         res.append(echo)
     if return_erle:
         res.append(erle)
+    if return_shift:
+        res.append(shift)
     return res[0] if len(res) == 1 else tuple(res)
 
 
@@ -250,10 +350,14 @@ class HostPipeline:
 
     def run(self, far: np.ndarray, mic: np.ndarray, cfg: Optional[Stage1Config] = None,
             n_samples: Optional[np.ndarray] = None, err: Optional[np.ndarray] = None,
-            echo: Optional[np.ndarray] = None, erle: Optional[np.ndarray] = None, wait: bool = True):
+            echo: Optional[np.ndarray] = None, erle: Optional[np.ndarray] = None, wait: bool = True,
+            align: Optional[DelayConfig] = None, shift: Optional[np.ndarray] = None,
+            peak: Optional[np.ndarray] = None):
         """``wait=False`` (streaming, batch after batch): return once the last slice is enqueued, so that the tail of
         this batch runs under the first uploads of the next; outputs are complete after ``wait()``.  Consecutive
-        deferred calls need different output arrays."""
+        deferred calls need different output arrays.  ``align``: estimate each utterance's far-end delay and run
+        stage 1 on the shifted far end (``aec_stage1_run_host_ex``); ``shift`` (int32 [B]) and ``peak`` (float32 [B])
+        receive the estimator's outputs, like ``erle``."""
         cfg = cfg or Stage1Config()
         pcm16 = far.dtype == np.int16
         item = 2 if pcm16 else 4
@@ -270,21 +374,30 @@ class HostPipeline:
                 raise TypeError(f"{name} must be a [B, L] float32 array with contiguous rows")
         if echo is not None and echo.strides[0] != err.strides[0]:
             raise ValueError("echo and err must share the row stride")
+        for name, a, dt in (("shift", shift, np.int32), ("peak", peak, np.float32)):
+            if a is not None and (a.dtype != dt or a.shape != (B,) or not a.flags.c_contiguous):
+                raise TypeError(f"{name} must be a contiguous {np.dtype(dt).name} array of B entries")
+        if align is None and (shift is not None or peak is not None):
+            raise ValueError("shift / peak need align")
         ns = None
         if n_samples is not None:
             ns = np.ascontiguousarray(n_samples, dtype=np.int64)
         c = cfg.to_c()
-        fn = self._lib.aec_stage1_run_host_pcm16 if pcm16 else self._lib.aec_stage1_run_host
+        dc = align.to_c() if align is not None else None
+        fn = self._lib.aec_stage1_run_host_pcm16_ex if pcm16 else self._lib.aec_stage1_run_host_ex
         if not wait:     # the arrays of a deferred call must outlive it
-            self._keep = getattr(self, "_keep", [])[-8:] + [(far, mic, err, echo, erle, ns)]
+            self._keep = getattr(self, "_keep", [])[-8:] + [(far, mic, err, echo, erle, ns, shift, peak)]
         with torch.cuda.device(self.device):
             _lib.check(self._lib.aec_host_ctx_set_deferred(self._ctx, 0 if wait else 1), "aec_host_ctx_set_deferred")
             rc = fn(self._ctx, far.ctypes.data, mic.ctypes.data, err.ctypes.data,
                     echo.ctypes.data if echo is not None else None,
                     erle.ctypes.data if erle is not None else None,
                     ns.ctypes.data if ns is not None else None,
-                    B, L, far.strides[0] // item, err.strides[0] // 4, C.byref(c))
-        _lib.check(rc, "aec_stage1_run_host_pcm16" if pcm16 else "aec_stage1_run_host")
+                    B, L, far.strides[0] // item, err.strides[0] // 4, C.byref(c),
+                    C.byref(dc) if dc is not None else None,
+                    shift.ctypes.data if shift is not None else None,
+                    peak.ctypes.data if peak is not None else None)
+        _lib.check(rc, "aec_stage1_run_host_pcm16_ex" if pcm16 else "aec_stage1_run_host_ex")
         return err
 
 

@@ -9,7 +9,8 @@ far-end : white Gaussian -> one-pole low-pass y[n] = 0.9 y[n-1] + x[n] -> 4 Hz r
           amplitude modulation -> peak-scaled to 0.5                      (seed 1000 + u)
 RIR     : g[n] exp(-n / tau), g ~ N(0,1), length = P*H, tau = length / 6.9, ||h||_2 = 0.5
                                                                           (seed 2000 + u)
-echo    : far * h truncated to L
+echo    : far * h truncated to L; with bulk_delay = d the response starts after d zeros (the playback and
+          capture latency of a real device), so the echo arrives d samples late
 near-end: zero (single talk) or the far-end generator gated on [0.4 L, 0.7 L], SER = 0 dB
                                                                           (seed 3000 + u)
 mic     : echo + near + white noise at -40 dB re echo                     (seed 4000 + u)
@@ -37,10 +38,12 @@ def make_rir(u: int, length: int) -> np.ndarray:
 
 
 def make_utterance(u: int, n_samples: int, sample_rate: int = 16000, rir_len: int = 1024,
-                   double_talk: bool = False):
+                   double_talk: bool = False, bulk_delay: int = 0):
     """Returns dict of float32 arrays: far, mic, echo, near (all [n_samples])."""
     far = _speechlike(np.random.default_rng(1000 + u), n_samples, sample_rate)
     h = make_rir(u, rir_len)
+    if bulk_delay:
+        h = np.concatenate([np.zeros(int(bulk_delay)), h])
     echo = fftconvolve(far, h)[:n_samples]
     near = np.zeros(n_samples)
     if double_talk:
@@ -65,12 +68,12 @@ def make_utterance(u: int, n_samples: int, sample_rate: int = 16000, rir_len: in
 
 
 def make_batch(first_u: int, batch: int, n_samples: int, sample_rate: int = 16000,
-               rir_len: int = 1024, double_talk: bool = False):
+               rir_len: int = 1024, double_talk: bool = False, bulk_delay: int = 0):
     """Stacked [batch, n_samples] float32 arrays for utterances first_u .. first_u+batch-1."""
     keys = ("far", "mic", "echo", "near")
     out = {k: np.empty((batch, n_samples), dtype=np.float32) for k in keys}
     for i in range(batch):
-        utt = make_utterance(first_u + i, n_samples, sample_rate, rir_len, double_talk)
+        utt = make_utterance(first_u + i, n_samples, sample_rate, rir_len, double_talk, bulk_delay)
         for k in keys:
             out[k][i] = utt[k]
     return out

@@ -12,7 +12,10 @@ names (``tr/tr_<idx>.ex``, ``tt/test.ex``, ``tt/test2.ex``, ``tr_list.txt``, ``t
 ``mic``/``ref``/``near``/``echo`` for the val form), so the reference readers (Stage2_lhm/scripts/train1.py:33-40,
 scripts/test.py:20-33, scripts/utils/data_utils.py:31-34) keep working; two datasets are ADDED beside them:
 ``stage1_error`` and ``stage1_echo``.  In ``test.ex`` / ``test2.ex`` they go INSIDE each numbered group because
-``ValidateDataset`` counts root members (scripts/test.py:23).
+``ValidateDataset`` counts root members (scripts/test.py:23).  With far-end alignment on (``--stage1_align_max_delay``,
+``Stage1Runner(align=...)``) stage 1 runs on the far end delayed by its estimated bulk delay, and a third dataset,
+``stage1_far_shift`` (float32, one element: that delay in samples), goes beside them; ``farend_speech`` stays as
+recorded.
 
 How a run is organised (the reference is one serial loop: decode 4 wavs, write, next utterance):
 
@@ -109,16 +112,20 @@ def _local_device() -> int:
 
 class Stage1Runner:
     """``runner(far, mic, n) -> (err, echo)`` backed by ``aec_stage1_run_host`` / ``_pcm16`` (no CPU fallback).
+    With ``align`` (a ``DelayConfig``) the far end is aligned to the microphone first (``aec_stage1_run_host_ex``) and
+    the runner returns ``(err, echo, shift)``, ``shift`` int32 [B] the samples each far end was delayed by.
 
     Inputs that are not page-locked (arrays a caller got from ``librosa.load`` and stacked with numpy) are staged
     through page-locked buffers first: a ``cudaMemcpyAsync`` from pageable memory is staged by the driver and
     serialises the slices of the pipeline.  Outputs are page-locked buffers owned by the runner, valid until the
     call after next (two sets alternate), which is what lets a writer thread drain batch k while batch k+1 runs."""
 
-    def __init__(self, cfg=None, slice_utterances: int = 128, device: Optional[int] = None, want_echo: bool = True):
+    def __init__(self, cfg=None, slice_utterances: int = 128, device: Optional[int] = None, want_echo: bool = True,
+                 align=None):
         from .stage1 import Stage1Config
 
         self.cfg = cfg or Stage1Config()
+        self.align = align
         self.slice_utterances = int(slice_utterances)
         self.device = _local_device() if device is None else int(device)
         self.want_echo = want_echo
@@ -159,10 +166,11 @@ class Stage1Runner:
         self._flip ^= 1
         err = self._pinned(out, "err", far.shape, np.float32)
         echo = self._pinned(out, "echo", far.shape, np.float32) if self.want_echo else None
+        shift = np.zeros(far.shape[0], dtype=np.int32) if self.align is not None else None
         t0 = time.perf_counter()
-        self.pipe.run(far, mic, self.cfg, n_samples=n, err=err, echo=echo)
+        self.pipe.run(far, mic, self.cfg, n_samples=n, err=err, echo=echo, align=self.align, shift=shift)
         self.seconds += time.perf_counter() - t0
-        return err, echo
+        return (err, echo) if shift is None else (err, echo, shift)
 
     def buffers_pinned(self) -> bool:
         """True when every staging / output buffer this runner has allocated is page-locked (tested on the GPU)."""
@@ -177,9 +185,9 @@ class Stage1Runner:
             self.pipe = None
 
 
-def default_runner(cfg=None, slice_utterances: int = 128, device: Optional[int] = None) -> Callable:
+def default_runner(cfg=None, slice_utterances: int = 128, device: Optional[int] = None, align=None) -> Callable:
     """Runner backed by ``aec_stage1_run_host`` on this rank's GPU (LOCAL_RANK under torchrun)."""
-    return Stage1Runner(cfg, slice_utterances, device)
+    return Stage1Runner(cfg, slice_utterances, device, align=align)
 
 
 def _h5py():
@@ -339,11 +347,14 @@ class _Engine:
 
     def _run(self, b: ingest.DecodedBatch):
         t0 = time.perf_counter()
-        err, echo = self.runner(b.far, b.mic, b.n)
+        res = self.runner(b.far, b.mic, b.n)
+        err, echo = res[0], res[1]
         self.stats["stage1_s"] += time.perf_counter() - t0
         self.stats["pcm16_batches" if b.pcm16 else "float32_batches"] += 1
         nb = len(b.n)
-        return [err[i, :b.n[i]] for i in range(nb)], [echo[i, :b.n[i]] for i in range(nb)]
+        # a runner that aligns the far end returns its per-utterance shift third
+        shifts = [np.array([res[2][i]], dtype=np.float32) for i in range(nb)] if len(res) > 2 else None
+        return [err[i, :b.n[i]] for i in range(nb)], [echo[i, :b.n[i]] for i in range(nb)], shifts
 
     def run(self, ids: Sequence[str], paths_of: Callable[[Sequence[str]], dict], emit: Callable):
         t_start = time.perf_counter()
@@ -368,8 +379,8 @@ class _Engine:
                     writes[k - 2].result()
                 if k + 1 < len(chunks):
                     fut_dec = dec.submit(self._decode, paths_of(chunks[k + 1]))
-                errs, echos = gpu.submit(self._run, b).result()
-                writes.append(wr.submit(timed_emit, k, chunk, b, errs, echos))
+                errs, echos, shifts = gpu.submit(self._run, b).result()
+                writes.append(wr.submit(timed_emit, k, chunk, b, errs, echos, shifts))
                 self.stats["utterances"] += len(chunk)
             for w in writes:
                 w.result()
@@ -437,25 +448,29 @@ def create_h5_train(args, runner: Optional[Callable] = None, batch: int = 256, h
     eng = _Engine(args.sr, runner, batch, decode_threads, pinned=(runner is None) if pinned is None else pinned)
     pool = ThreadPoolExecutor(max(1, write_threads), thread_name_prefix="aec-h5")
 
-    def write_one(name, b, j, err, echo):
+    def write_one(name, b, j, err, echo, shift):
         w = h5.File(name, "w")
         for k in KEYS:                                                   # train_wav2h5.py:39-42
             _create_dataset(w, k, _signal(b, k, j))
         _create_dataset(w, "stage1_error", err)
         _create_dataset(w, "stage1_echo", echo)
+        if shift is not None:
+            _create_dataset(w, "stage1_far_shift", shift)
         w.close()
 
-    def emit(k, chunk, b, errs, echos):
-        futs = [pool.submit(write_one, os.path.join(args.h5_path, "tr", "tr_" + idx + ".ex"), b, j, errs[j], echos[j])
+    def emit(k, chunk, b, errs, echos, shifts):
+        futs = [pool.submit(write_one, os.path.join(args.h5_path, "tr", "tr_" + idx + ".ex"), b, j, errs[j], echos[j],
+                            shifts[j] if shifts is not None else None)
                 for j, idx in enumerate(chunk)]
         for f in futs:
             f.result()
 
-    def emit_native(k, chunk, b, errs, echos):
+    def emit_native(k, chunk, b, errs, echos, shifts):
         # the whole batch in ONE C call (aec_ex_write_batch: C++ threads, int16 -> float32 on the way out, no
         # interpreter between the files); same bytes as write_one through h5lite
-        names = KEYS + ("stage1_error", "stage1_echo")
-        rows = [[_signal(b, key, j) for key in KEYS] + [errs[j], echos[j]] for j in range(len(chunk))]
+        names = KEYS + ("stage1_error", "stage1_echo") + (("stage1_far_shift",) if shifts is not None else ())
+        rows = [[_signal(b, key, j) for key in KEYS] + [errs[j], echos[j]] + ([shifts[j]] if shifts is not None else [])
+                for j in range(len(chunk))]
         write_ex_batch([os.path.join(args.h5_path, "tr", "tr_" + idx + ".ex") for idx in chunk], names, rows,
                        threads=max(1, write_threads))
 
@@ -487,7 +502,7 @@ def _single_file(args, ids, paths_of, keymap, h5, runner, batch, filename, list_
     count = [0]
     eng = _Engine(args.sr, runner, batch, decode_threads, pinned=(runner is None) if pinned is None else pinned)
 
-    def emit(k, chunk, b, errs, echos):
+    def emit(k, chunk, b, errs, echos, shifts):
         for j in range(len(chunk)):
             g = w.create_group(str(count[0]))                                # test_wav2h5.py:44, val_wav2h5.py:42
             for out_key, src_key in keymap.items():
@@ -501,6 +516,8 @@ def _single_file(args, ids, paths_of, keymap, h5, runner, batch, filename, list_
                 _create_dataset(g, out_key, a, shape)
             _create_dataset(g, "stage1_error", errs[j])
             _create_dataset(g, "stage1_echo", echos[j])
+            if shifts is not None:
+                _create_dataset(g, "stage1_far_shift", shifts[j])
             count[0] += 1
 
     st = eng.run(ids, paths_of, emit)
@@ -578,6 +595,10 @@ def build_parser(kind: str) -> argparse.ArgumentParser:
     p.add_argument("--stage1_algo", choices=sorted(STAGE1_ALGOS), default="nlms",
                    help="nlms / kalman: STFT-domain recurrence; ols-nlms / ols-kalman: overlap-save PBFDAF (frame 512, 1-16 partitions)")
     p.add_argument("--stage1_partitions", type=int, default=4)
+    p.add_argument("--stage1_align_max_delay", type=int, default=0,
+                   help="0: off; else the largest far-end delay (samples, a power of two in 256..8192) searched per "
+                        "utterance -- stage 1 then runs on the far end delayed by the estimate, and each utterance "
+                        "gets a stage1_far_shift dataset (samples)")
     # not in the reference (which always writes through h5py): who writes the .ex (HDF5) files
     p.add_argument("--ex_writer", choices=["auto", "h5py", "native"], default="auto",
                    help="auto: h5py when installed (chunked storage, as the reference writes), else the package's own HDF5 "
@@ -605,9 +626,11 @@ def runner_from_args(args) -> Optional[Callable]:
     """the stage-1 runner the command-line flags ask for; None (-> library default) when they are absent"""
     if not hasattr(args, "stage1_algo"):
         return None
-    from .stage1 import Stage1Config
+    from .stage1 import DelayConfig, Stage1Config
 
-    return default_runner(Stage1Config(algo=STAGE1_ALGOS[args.stage1_algo], partitions=int(args.stage1_partitions)))
+    n = int(getattr(args, "stage1_align_max_delay", 0) or 0)
+    return default_runner(Stage1Config(algo=STAGE1_ALGOS[args.stage1_algo], partitions=int(args.stage1_partitions)),
+                          align=DelayConfig(max_delay=n) if n > 0 else None)
 
 
 def main(kind: str = "train", argv=None):

@@ -161,6 +161,43 @@ int aec_stage1_run_host(aec_host_ctx* ctx, const float* far, const float* mic, f
 int aec_stage1_run_host_pcm16(aec_host_ctx* ctx, const int16_t* far, const int16_t* mic, float* err,
                               float* echo_est, float* erle_db, const int64_t* n_samples, int64_t B, int64_t L,
                               int64_t in_stride, int64_t out_stride, const aec_cfg* cfg);
+/* Far-end bulk delay (GCC-PHAT over the whole utterance) and far-end alignment before stage 1.  The stage-1 filters
+ * model echo paths that start at lag 0 and end before their tail (P * hop samples); a device's playback / capture
+ * latency delays the echo by tens to hundreds of milliseconds, past that tail.  Per utterance, with D = max_delay:
+ *   r[l] = PHAT-weighted cross-correlation of mic and far end at lag l = 0..D (|r| <= 1; DC and Nyquist dropped),
+ *   delay = smallest l maximising |r[l]|, peak = |r[delay]|,
+ *   shift = peak >= min_peak ? max(0, delay - margin) : 0,   far_aligned[n] = far[n - shift] (0 for n < shift).
+ * Exact definition: DESIGN.md "Far-end delay estimation" and oracle/delay_oracle.py.  Whole samples; lags are
+ * non-negative (the microphone never leads the far end); an empty utterance or a silent far end gives 0, 0, 0. */
+typedef struct aec_delay_cfg {
+    int32_t max_delay;    /* D: largest lag searched, a power of two in [256, 8192]   (default 8192: 512 ms at 16 kHz) */
+    int32_t margin;       /* samples of echo path kept in front of the estimated delay, >= 0  (default 128) */
+    float min_peak;       /* peak below which no shift is applied                       (default 0.1) */
+    int32_t reserved[5];
+} aec_delay_cfg;
+int aec_delay_cfg_default(aec_delay_cfg* dcfg);
+/* DEVICE buffers, caller's stream.  far, mic [B][in_stride] (first n_samples[b] or L samples; n_samples nullable
+ * DEVICE int64 [B], clamped to [0, L]); outputs [B]: delay (nullable), shift, peak (nullable); corr nullable
+ * [B][max_delay + 1] = r.  One CTA per utterance: a row's outputs are bit-identical alone or in any batch. */
+int aec_delay_estimate(const float* far, const float* mic, const int64_t* n_samples, int64_t B, int64_t L,
+                       int64_t in_stride, const aec_delay_cfg* dcfg, int32_t* delay, int32_t* shift, float* peak,
+                       float* corr, void* cuda_stream);
+/* far_out[b][n] = far[b][n - shift[b]] for shift[b] <= n < L, 0 below (a negative shift counts as 0).  DEVICE
+ * buffers; far_out [B][out_stride] must not overlap far. */
+int aec_delay_align(const float* far, float* far_out, const int32_t* shift, int64_t B, int64_t L, int64_t in_stride,
+                    int64_t out_stride, void* cuda_stream);
+/* aec_stage1_run_host[_pcm16] with the far end aligned first: each slice runs H2D, (PCM16 conversion), estimate,
+ * align, stage 1 on the aligned far end, D2H.  align = NULL is exactly aec_stage1_run_host[_pcm16].  shift_out /
+ * peak_out: nullable HOST [B], delivered like erle_db (after aec_host_ctx_wait in deferred mode); non-NULL only with
+ * align.  The outputs are those of aec_delay_estimate + aec_delay_align + aec_stage1_run on the device buffers. */
+int aec_stage1_run_host_ex(aec_host_ctx* ctx, const float* far, const float* mic, float* err, float* echo_est,
+                           float* erle_db, const int64_t* n_samples, int64_t B, int64_t L, int64_t in_stride,
+                           int64_t out_stride, const aec_cfg* cfg, const aec_delay_cfg* align, int32_t* shift_out,
+                           float* peak_out);
+int aec_stage1_run_host_pcm16_ex(aec_host_ctx* ctx, const int16_t* far, const int16_t* mic, float* err,
+                                 float* echo_est, float* erle_db, const int64_t* n_samples, int64_t B, int64_t L,
+                                 int64_t in_stride, int64_t out_stride, const aec_cfg* cfg, const aec_delay_cfg* align,
+                                 int32_t* shift_out, float* peak_out);
 /* page-locked host memory helpers (cudaHostAlloc / cudaFreeHost).  Pageable buffers work with the host entries
  * but every copy is then staged by the driver and serialises the slices -- allocate the arrays that
  * `librosa.load` results are gathered into with these.  AEC_HOST_WRITE_COMBINED: for buffers the CPU only
