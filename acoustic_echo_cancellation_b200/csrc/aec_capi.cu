@@ -12,8 +12,6 @@
 
 #include "aec_common.cuh"
 #include "stage1_launch.cuh"
-#include "stage1_kernel_1024.cuh"
-#include "stage1_ols1024_kernel.cuh"   // (includes stage1_ols_kernel.cuh) launchers of the overlap-save kernels
 
 namespace aec {
 
@@ -352,48 +350,46 @@ static int stage1_run_impl(const float* far, const float* mic, float* err, float
     p.win_a = wide ? tab.win_a1k : tab.win_a;
     p.win_s = wide ? tab.win_s1k : tab.win_s;
 
+    // The build to run.  A variant (1000 * warps_per_utterance + register cap, e.g. 2168) names one; 0 asks for the
+    // default, the first build the unit lists for (P, algo, echo) at the warp count chosen here.  A build that was not
+    // compiled is refused before anything is launched, never replaced by another.
     const int P = cfg->partitions;
-    const bool echo = echo_est != nullptr;
-    // variant = 1000 * warps_per_utterance + register cap (e.g. 2144); 0 = library default
-    int nw = 0, minb = 0;
+    const bool ols = cfg->algo == AEC_ALGO_PBFDAF || cfg->algo == AEC_ALGO_PBFKF;
+    int nw = 0, regs = 0;
     if (cfg->variant > 0) {
+        if (cfg->variant < 1000) return AEC_EUNSUPPORTED;        // a register cap alone names no build
+        if (feat || (wide && ols)) return AEC_EUNSUPPORTED;      // these builds follow from P, algo and the batch size
         nw = cfg->variant / 1000;
-        minb = cfg->variant % 1000;
+        regs = cfg->variant % 1000;
+    }
+    Stage1Launch (*lookup)(int P, int algo, bool echo, int nw, int regs) = nullptr;
+    if (feat) {
+        lookup = stage1_build_feat;
+        // 4-partition NLMS: five utterances per SM (168 registers) win on many-wave batches (4144 x 10 s: 8.79 vs
+        // 9.36 ms); for batches of a wave or two the launch ends with a thin last wave either way and four per SM at 200
+        // registers are faster (1024 x 10 s: 2.61 vs 2.88 ms).
+        if (P == 4 && cfg->algo == AEC_ALGO_NLMS) regs = B >= 20LL * p.num_sms ? 168 : 200;
+    } else if (ols) {
+        lookup = wide ? stage1_build_ols1024 : stage1_build_ols;
+    } else if (wide) {
+        lookup = stage1_build_1024;
     } else {
         // measured defaults (DESIGN.md): short filters 2 warps / 2 pairs per thread; 8 partitions and
         // more: 8 warps, one bin per thread (since bin 128 of the ring kernels runs one chunk ahead on the idle
         // synthesis warps this also holds for the 16-partition NLMS filter: 5.71 ms per 2048 x 10 s against 5.95
         // for the 4-warp / 255-register kernel, which remains available as variant 4255)
-        nw = (P <= 4) ? 2 : 8;
-        // (defaults: the first instantiation listed for (P, algo, echo) in stage1_inst_nw*.cu --
-        //  128 registers for the two-warp kernels so that 7 utterances stay resident per SM)
-    }
-    // A variant names one build: a warp count the selected kernel does not have is refused, never silently replaced.
-    cudaError_t e;
-    if (cfg->algo == AEC_ALGO_PBFDAF || cfg->algo == AEC_ALGO_PBFKF) {
-        if (feat) return AEC_EUNSUPPORTED;               // no fused features for the overlap-save filters
-        if (wide) {
-            if (cfg->variant > 0) return AEC_EUNSUPPORTED;
-            e = launch_stage1_ols1024(P, cfg->algo == AEC_ALGO_PBFKF, echo, p, s);
-        } else {
-            if (cfg->variant > 0 && nw != ols_warps(P)) return AEC_EUNSUPPORTED;   // the warp count follows from P
-            e = launch_stage1_ols(P, cfg->algo == AEC_ALGO_PBFKF, echo, minb, p, s);
+        if (nw == 0) nw = P <= 4 ? 2 : 8;
+        switch (nw) {
+            case 1: lookup = stage1_build_nw1; break;
+            case 2: lookup = stage1_build_nw2; break;
+            case 4: lookup = stage1_build_nw4; break;
+            case 8: lookup = stage1_build_nw8; break;
+            default: return AEC_EUNSUPPORTED;
         }
-    } else if (feat) {
-        if (cfg->variant > 0) return AEC_EUNSUPPORTED;   // the feature build is chosen from the batch size
-        e = launch_stage1_feat(P, cfg->algo, p, s);
-    } else if (wide) {
-        if (cfg->variant > 0 && nw != 8) return AEC_EUNSUPPORTED;                // eight warps per utterance
-        e = launch_stage1_1024(P, cfg->algo, echo, minb, p, s);
-    } else
-    switch (nw) {
-        case 1: e = launch_stage1_nw1(P, cfg->algo, echo, minb, p, s); break;
-        case 2: e = launch_stage1_nw2(P, cfg->algo, echo, minb, p, s); break;
-        case 4: e = launch_stage1_nw4(P, cfg->algo, echo, minb, p, s); break;
-        case 8: e = launch_stage1_nw8(P, cfg->algo, echo, minb, p, s); break;
-        default: return AEC_EUNSUPPORTED;
     }
-    if (e == kNoInstance) return AEC_EUNSUPPORTED;     // (P, algo, echo, register cap) not instantiated -- nothing was launched
+    const Stage1Launch launch = lookup(P, cfg->algo, echo_est != nullptr, nw, regs);
+    if (!launch) return AEC_EUNSUPPORTED;
+    const cudaError_t e = launch(p, s);
     if (e != cudaSuccess) {
         set_cuda_error(e, "stage1 kernel launch");
         return AEC_ECUDA;

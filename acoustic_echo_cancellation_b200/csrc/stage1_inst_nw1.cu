@@ -1,13 +1,17 @@
-// Instantiations: 1 warp per utterance (4 mirrored-bin pairs per thread, no block barriers
-// beyond the warp), chunk = 2 frames.  Tuning variants for short filters.
+// Builds: 1 warp per utterance (4 mirrored-bin pairs per thread, no block barriers beyond the warp), chunk = 2 frames.
+// Tuning variants for short filters.
 #include "stage1_launch.cuh"
 
 namespace aec {
+namespace {
+template <int NW, int P, int ALGO, bool ECHO, int REGS>
+using Build = N512Build<NW, P, ALGO, ECHO, REGS, false>;
+}
 
-cudaError_t launch_stage1_nw1(int P, int algo, bool echo, int regs, const Stage1Params& prm, cudaStream_t s) {
-    AEC_TRY_INSTANCE(1, 4, kAlgoNlms, false, 255)
-    AEC_TRY_INSTANCE(1, 4, kAlgoNlms, false, 200)
-    return kNoInstance;
+Stage1Launch stage1_build_nw1(int P, int algo, bool echo, int nw, int regs) {
+    AEC_STAGE1_BUILD(1, 4, kAlgoNlms, false, 255)
+    AEC_STAGE1_BUILD(1, 4, kAlgoNlms, false, 200)
+    return nullptr;
 }
 
 }  // namespace aec

@@ -1,19 +1,23 @@
-// Instantiations: 8 warps per utterance, ONE bin per thread, chunk = 16 frames -- long filters
-// (the per-bin state W_p, X[t-p], C_p of a 16-partition Kalman filter is 81 registers).
+// Builds: 8 warps per utterance, ONE bin per thread, chunk = 16 frames -- long filters (the per-bin state W_p, X[t-p],
+// C_p of a 16-partition Kalman filter is 81 registers).
 #include "stage1_launch.cuh"
 
 namespace aec {
+namespace {
+template <int NW, int P, int ALGO, bool ECHO, int REGS>
+using Build = N512Build<NW, P, ALGO, ECHO, REGS, false>;
+}
 
-cudaError_t launch_stage1_nw8(int P, int algo, bool echo, int regs, const Stage1Params& prm, cudaStream_t s) {
-    AEC_TRY_INSTANCE(8, 16, kAlgoKalman, false, 128)
-    AEC_TRY_INSTANCE(8, 16, kAlgoKalman, true, 128)
-    AEC_TRY_INSTANCE(8, 16, kAlgoNlms, false, 128)
-    AEC_TRY_INSTANCE(8, 16, kAlgoNlms, true, 128)
-    AEC_TRY_INSTANCE(8, 8, kAlgoKalman, false, 128)
-    AEC_TRY_INSTANCE(8, 8, kAlgoKalman, true, 128)
-    AEC_TRY_INSTANCE(8, 8, kAlgoNlms, false, 128)
-    AEC_TRY_INSTANCE(8, 8, kAlgoNlms, true, 128)
-    return kNoInstance;
+Stage1Launch stage1_build_nw8(int P, int algo, bool echo, int nw, int regs) {
+    AEC_STAGE1_BUILD(8, 16, kAlgoKalman, false, 128)
+    AEC_STAGE1_BUILD(8, 16, kAlgoKalman, true, 128)
+    AEC_STAGE1_BUILD(8, 16, kAlgoNlms, false, 128)
+    AEC_STAGE1_BUILD(8, 16, kAlgoNlms, true, 128)
+    AEC_STAGE1_BUILD(8, 8, kAlgoKalman, false, 128)
+    AEC_STAGE1_BUILD(8, 8, kAlgoKalman, true, 128)
+    AEC_STAGE1_BUILD(8, 8, kAlgoNlms, false, 128)
+    AEC_STAGE1_BUILD(8, 8, kAlgoNlms, true, 128)
+    return nullptr;
 }
 
 }  // namespace aec

@@ -1,62 +1,51 @@
-// Instantiations of the overlap-save PBFDAF kernel (algo = 2: NLMS step, algo = 3: Kalman step): two warps per
-// utterance for 1-4 partitions, four for 8, eight for 16 (OlsShape).
+// Builds of the overlap-save PBFDAF kernel (kAlgoPbfdaf: NLMS step, kAlgoPbfkf: Kalman step): two warps per utterance
+// for 1-4 partitions, four for 8, eight for 16 (OlsShape).
 #include "stage1_ols_kernel.cuh"
+#include "stage1_launch.cuh"
 
 namespace aec {
-
-template <int P, bool KAL, bool ECHO, int REGS>
-static cudaError_t launch_ols(const Stage1Params& prm, cudaStream_t s) {
-    auto kern = stage1_ols_kernel<P, KAL, ECHO, REGS>;
-    const size_t smem = OlsSmem::total(P, KAL);
-    static thread_local int configured_dev = -1;
-    int dev = 0;
-    cudaError_t e = cudaGetDevice(&dev);
-    if (e != cudaSuccess) return e;
-    if (configured_dev != dev) {
-        e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        // carve-out: what the resident utterances need, the rest stays L1 (spill reloads of the 128-register builds)
-        int resident = 0;
-        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&resident, kern, OlsShape<P>::NT, smem);
-        if (e != cudaSuccess) return e;
-        if (resident > 0) {
-            const size_t need = size_t(resident) * (smem + 1024);
-            int pct = static_cast<int>((need * 100 + 228 * 1024 - 1) / (228 * 1024));
-            e = cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, pct > 100 ? 100 : pct);
-            if (e != cudaSuccess) return e;
-        }
-        configured_dev = dev;
-    }
-    kern<<<dim3((unsigned)prm.B), dim3(OlsShape<P>::NT), smem, s>>>(prm);
-    return cudaGetLastError();
+namespace {
+template <int NW, int P, int ALGO, bool ECHO, int REGS>
+struct Build {
+    static_assert(NW == OlsShape<P>::NW, "the overlap-save warp count follows from P");
+    static constexpr bool KAL = ALGO == kAlgoPbfkf;
+    static constexpr void (*kernel)(Stage1Params) = stage1_ols_kernel<P, KAL, ECHO, REGS>;
+    static constexpr size_t smem = OlsSmem::total(P, KAL);
+};
 }
 
-template <int P, int REGS_NLMS, int REGS_KAL>
-static cudaError_t launch_ols_p(bool kalman, bool echo, const Stage1Params& prm, cudaStream_t s) {
-    if (kalman) return echo ? launch_ols<P, true, true, REGS_KAL>(prm, s) : launch_ols<P, true, false, REGS_KAL>(prm, s);
-    return echo ? launch_ols<P, false, true, REGS_NLMS>(prm, s) : launch_ols<P, false, false, REGS_NLMS>(prm, s);
-}
-
-// regs: register cap asked for through aec_cfg.variant (0 = the default below)
-cudaError_t launch_stage1_ols(int P, bool kalman, bool echo, int regs, const Stage1Params& prm, cudaStream_t s) {
-    if (P == 4) {
-        // 128 registers (8 utterances per SM) by default.  The Kalman step keeps the far-end history in shared memory
-        // (OlsSmem::ring), which is what lets its 20 extra state registers fit: 2.85 ms per 1024 x 10 s, 11.5 ms per 4096
-        // (history in registers: 3.4 / 12.4 ms at 128 registers with spills, 4.7 / 11.9 ms at 168 without).  The
-        // 168-register builds stay available as variant 2168.
-        if (kalman && regs == 168) return launch_ols_p<4, 128, 168>(kalman, echo, prm, s);
-        if (regs == 0 || regs == 128) return launch_ols_p<4, 128, 128>(kalman, echo, prm, s);
-        // (NLMS step at 168 registers, spill-free: 6 % shorter block latency -- 3660 against 3900 cycles alone on an SM --
-        //  which does not pay for 6 instead of 8 resident utterances; variant 2168)
-        if (!kalman && regs == 168) return launch_ols_p<4, 168, 168>(kalman, echo, prm, s);
-        return kNoInstance;
-    }
-    if (regs != 0 && regs != 128) return kNoInstance;
-    if (P == 16) return launch_ols_p<16, 128, 128>(kalman, echo, prm, s);
-    if (P == 8) return launch_ols_p<8, 128, 128>(kalman, echo, prm, s);
-    if (P == 2) return launch_ols_p<2, 128, 128>(kalman, echo, prm, s);
-    if (P == 1) return launch_ols_p<1, 128, 128>(kalman, echo, prm, s);
-    return kNoInstance;
+Stage1Launch stage1_build_ols(int P, int algo, bool echo, int nw, int regs) {
+    // 128 registers (8 utterances per SM) by default.  The Kalman step keeps the far-end history in shared memory
+    // (OlsSmem::ring), which is what lets its 20 extra state registers fit: 2.85 ms per 1024 x 10 s, 11.5 ms per 4096
+    // (history in registers: 3.4 / 12.4 ms at 128 registers with spills, 4.7 / 11.9 ms at 168 without).
+    AEC_STAGE1_BUILD(2, 4, kAlgoPbfdaf, false, 128)
+    AEC_STAGE1_BUILD(2, 4, kAlgoPbfdaf, true, 128)
+    AEC_STAGE1_BUILD(2, 4, kAlgoPbfkf, false, 128)
+    AEC_STAGE1_BUILD(2, 4, kAlgoPbfkf, true, 128)
+    // The 168-register Kalman builds stay available as variant 2168.
+    AEC_STAGE1_BUILD(2, 4, kAlgoPbfkf, false, 168)
+    AEC_STAGE1_BUILD(2, 4, kAlgoPbfkf, true, 168)
+    // NLMS step at 168 registers, spill-free: 6 % shorter block latency -- 3660 against 3900 cycles alone on an SM --
+    // which does not pay for 6 instead of 8 resident utterances; variant 2168.
+    AEC_STAGE1_BUILD(2, 4, kAlgoPbfdaf, false, 168)
+    AEC_STAGE1_BUILD(2, 4, kAlgoPbfdaf, true, 168)
+    AEC_STAGE1_BUILD(8, 16, kAlgoPbfdaf, false, 128)
+    AEC_STAGE1_BUILD(8, 16, kAlgoPbfdaf, true, 128)
+    AEC_STAGE1_BUILD(8, 16, kAlgoPbfkf, false, 128)
+    AEC_STAGE1_BUILD(8, 16, kAlgoPbfkf, true, 128)
+    AEC_STAGE1_BUILD(4, 8, kAlgoPbfdaf, false, 128)
+    AEC_STAGE1_BUILD(4, 8, kAlgoPbfdaf, true, 128)
+    AEC_STAGE1_BUILD(4, 8, kAlgoPbfkf, false, 128)
+    AEC_STAGE1_BUILD(4, 8, kAlgoPbfkf, true, 128)
+    AEC_STAGE1_BUILD(2, 2, kAlgoPbfdaf, false, 128)
+    AEC_STAGE1_BUILD(2, 2, kAlgoPbfdaf, true, 128)
+    AEC_STAGE1_BUILD(2, 2, kAlgoPbfkf, false, 128)
+    AEC_STAGE1_BUILD(2, 2, kAlgoPbfkf, true, 128)
+    AEC_STAGE1_BUILD(2, 1, kAlgoPbfdaf, false, 128)
+    AEC_STAGE1_BUILD(2, 1, kAlgoPbfdaf, true, 128)
+    AEC_STAGE1_BUILD(2, 1, kAlgoPbfkf, false, 128)
+    AEC_STAGE1_BUILD(2, 1, kAlgoPbfkf, true, 128)
+    return nullptr;
 }
 
 }  // namespace aec

@@ -1,44 +1,28 @@
-// Instantiations of the frame-1024 overlap-save PBFDAF kernel (algo 2 / 3; 4 partitions: four warps per utterance, 8: eight).
+// Builds of the frame-1024 overlap-save PBFDAF kernel (kAlgoPbfdaf / kAlgoPbfkf; 4 partitions: four warps per
+// utterance, 8: eight).
+#include "stage1_launch.cuh"
 #include "stage1_ols1024_kernel.cuh"
 
 namespace aec {
-
-template <int P, bool KAL, bool ECHO>
-static cudaError_t launch_ols1024(const Stage1Params& prm, cudaStream_t s) {
-    auto kern = stage1_ols1024_kernel<P, KAL, ECHO, 128>;
-    constexpr size_t smem = Ols1024Shape<P>::total;
-    static thread_local int configured_dev = -1;
-    int dev = 0;
-    cudaError_t e = cudaGetDevice(&dev);
-    if (e != cudaSuccess) return e;
-    if (configured_dev != dev) {
-        e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        int resident = 0;
-        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&resident, kern, Ols1024Shape<P>::NT, smem);
-        if (e != cudaSuccess) return e;
-        if (resident > 0) {
-            const size_t need = size_t(resident) * (smem + 1024);
-            int pct = static_cast<int>((need * 100 + 228 * 1024 - 1) / (228 * 1024));
-            e = cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, pct > 100 ? 100 : pct);
-            if (e != cudaSuccess) return e;
-        }
-        configured_dev = dev;
-    }
-    kern<<<dim3((unsigned)prm.B), dim3(Ols1024Shape<P>::NT), smem, s>>>(prm);
-    return cudaGetLastError();
+namespace {
+template <int NW, int P, int ALGO, bool ECHO, int REGS>
+struct Build {
+    static_assert(NW == Ols1024Shape<P>::NW, "the frame-1024 overlap-save warp count follows from P");
+    static constexpr void (*kernel)(Stage1Params) = stage1_ols1024_kernel<P, ALGO == kAlgoPbfkf, ECHO, REGS>;
+    static constexpr size_t smem = Ols1024Shape<P>::total;
+};
 }
 
-template <int P>
-static cudaError_t launch_ols1024_p(bool kalman, bool echo, const Stage1Params& prm, cudaStream_t s) {
-    if (kalman) return echo ? launch_ols1024<P, true, true>(prm, s) : launch_ols1024<P, true, false>(prm, s);
-    return echo ? launch_ols1024<P, false, true>(prm, s) : launch_ols1024<P, false, false>(prm, s);
-}
-
-cudaError_t launch_stage1_ols1024(int P, bool kalman, bool echo, const Stage1Params& prm, cudaStream_t s) {
-    if (P == 8) return launch_ols1024_p<8>(kalman, echo, prm, s);
-    if (P == 4) return launch_ols1024_p<4>(kalman, echo, prm, s);
-    return kNoInstance;
+Stage1Launch stage1_build_ols1024(int P, int algo, bool echo, int nw, int regs) {
+    AEC_STAGE1_BUILD(8, 8, kAlgoPbfdaf, false, 128)
+    AEC_STAGE1_BUILD(8, 8, kAlgoPbfdaf, true, 128)
+    AEC_STAGE1_BUILD(8, 8, kAlgoPbfkf, false, 128)
+    AEC_STAGE1_BUILD(8, 8, kAlgoPbfkf, true, 128)
+    AEC_STAGE1_BUILD(4, 4, kAlgoPbfdaf, false, 128)
+    AEC_STAGE1_BUILD(4, 4, kAlgoPbfdaf, true, 128)
+    AEC_STAGE1_BUILD(4, 4, kAlgoPbfkf, false, 128)
+    AEC_STAGE1_BUILD(4, 4, kAlgoPbfkf, true, 128)
+    return nullptr;
 }
 
 }  // namespace aec

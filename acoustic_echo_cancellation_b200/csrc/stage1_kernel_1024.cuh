@@ -287,25 +287,4 @@ __global__ void __launch_bounds__(256) __maxnreg__(REGS) stage1_n1024_kernel(con
     }
 }
 
-template <int P, int ALGO, bool ECHO, int REGS>
-inline cudaError_t launch_stage1_1024_instance(const Stage1Params& prm, cudaStream_t s) {
-    auto kern = stage1_n1024_kernel<P, ALGO, ECHO, REGS>;
-    const size_t smem = Stage1Smem1024::total(ECHO, P);
-    static thread_local int configured_dev = -1;
-    int dev = 0;
-    cudaError_t e = cudaGetDevice(&dev);
-    if (e != cudaSuccess) return e;
-    if (configured_dev != dev) {
-        e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        e = cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
-        if (e != cudaSuccess) return e;
-        configured_dev = dev;
-    }
-    kern<<<dim3((unsigned)prm.B), dim3(256), smem, s>>>(prm);
-    return cudaGetLastError();
-}
-
-cudaError_t launch_stage1_1024(int P, int algo, bool echo, int regs, const Stage1Params& prm, cudaStream_t s);
-
 }  // namespace aec

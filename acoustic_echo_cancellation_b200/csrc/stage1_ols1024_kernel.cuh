@@ -296,7 +296,4 @@ __global__ void __launch_bounds__(Ols1024Shape<P>::NT) __maxnreg__(REGS) stage1_
     }
 }
 
-// stage1_inst_ols1024.cu
-cudaError_t launch_stage1_ols1024(int P, bool kalman, bool echo, const Stage1Params& prm, cudaStream_t s);
-
 }  // namespace aec

@@ -516,7 +516,4 @@ __global__ void __launch_bounds__(OlsShape<P>::NT) __maxnreg__(REGS) stage1_ols_
 #endif
 }
 
-// stage1_inst_ols.cu
-cudaError_t launch_stage1_ols(int P, bool kalman, bool echo, int regs, const Stage1Params& prm, cudaStream_t s);
-
 }  // namespace aec

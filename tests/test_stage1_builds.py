@@ -100,47 +100,21 @@ DEFAULTS = sorted({(b.frame, b.P, b.algo, b.echo) for b in BUILDS if b.entry not
 # ---------------------------------------------------------------------------------------------------------------------
 # a. the table and what the units instantiate (CPU)
 # ---------------------------------------------------------------------------------------------------------------------
-_ALGO_TOKENS = {"kAlgoNlms": NLMS, "kAlgoKalman": KALMAN}
+_ALGO_TOKENS = {"kAlgoNlms": NLMS, "kAlgoKalman": KALMAN, "kAlgoPbfdaf": OLS_NLMS, "kAlgoPbfkf": OLS_KALMAN}
 
 
 def _instantiations():
-    """Every (entry, frame, P, algo, echo, warps, regs) the stage1_inst_*.cu units compile, read from their text."""
+    """Every (entry, frame, P, algo, echo, warps, regs) the stage1_inst_*.cu units compile, read from their
+    AEC_STAGE1_BUILD(NW, P, ALGO, ECHO, REGS) lines."""
     found = set()
-
-    def src(unit):
+    for unit in ("nw1", "nw2", "nw4", "nw8", "1024", "feat", "ols", "ols1024"):
         with open(os.path.join(CSRC, f"stage1_inst_{unit}.cu")) as f:
-            text = f.read()
-        return re.sub(r"//[^\n]*", "", text)           # (instantiations named in comments do not count)
-
-    def flag(tok):
-        return {"true": True, "false": False}[tok.strip()]
-
-    for unit in ("nw1", "nw2", "nw4", "nw8"):
-        for nw, P, algo, echo, regs in re.findall(r"AEC_TRY_INSTANCE\(\s*(\d+)\s*,\s*(\d+)\s*,\s*(\w+)\s*,\s*(\w+)\s*,"
-                                                  r"\s*(\d+)\s*\)", src(unit)):
-            found.add((unit, 512, int(P), _ALGO_TOKENS[algo], flag(echo), int(nw), int(regs)))
-    for P, algo, echo, regs in re.findall(r"AEC_TRY_1024\(\s*(\d+)\s*,\s*(\w+)\s*,\s*(\w+)\s*,\s*(\d+)\s*\)", src("1024")):
-        found.add(("1024", 1024, int(P), _ALGO_TOKENS[algo], flag(echo), 8, int(regs)))   # 8 warps: __launch_bounds__(256)
-    text = src("ols")
-    calls = re.findall(r"launch_ols_p<\s*(\d+)\s*,\s*(\d+)\s*,\s*(\d+)\s*>\s*\(", text)
-    assert calls, "no launch_ols_p<P, REGS_NLMS, REGS_KAL> call found in stage1_inst_ols.cu"
-    for P, rn, rk in calls:
-        P = int(P)
-        for algo, regs in ((OLS_NLMS, int(rn)), (OLS_KALMAN, int(rk))):
-            for echo in (False, True):
-                found.add(("ols", 512, P, algo, echo, 2 if P <= 4 else P // 2, regs))
-    text = src("ols1024")
-    (regs,) = re.findall(r"stage1_ols1024_kernel<\s*P\s*,\s*KAL\s*,\s*ECHO\s*,\s*(\d+)\s*>", text)
-    calls = re.findall(r"launch_ols1024_p<\s*(\d+)\s*>\s*\(", text)
-    assert calls, "no launch_ols1024_p<P> call found in stage1_inst_ols1024.cu"
-    for P in calls:
-        for algo in (OLS_NLMS, OLS_KALMAN):
-            for echo in (False, True):
-                found.add(("ols1024", 1024, int(P), algo, echo, int(P), int(regs)))
-    feats = re.findall(r"launch_stage1_instance<\s*(\d+)\s*,\s*(\d+)\s*,\s*(\w+)\s*,\s*(\w+)\s*,\s*(\d+)\s*,\s*true\s*>",
-                       src("feat"))
-    for nw, P, algo, echo, regs in feats:
-        found.add(("feat", 512, int(P), _ALGO_TOKENS[algo], flag(echo), int(nw), int(regs)))
+            text = re.sub(r"//[^\n]*", "", f.read())      # (builds named in comments do not count)
+        builds = re.findall(r"AEC_STAGE1_BUILD\(\s*(\d+)\s*,\s*(\d+)\s*,\s*(\w+)\s*,\s*(true|false)\s*,\s*(\d+)\s*\)", text)
+        assert builds, f"no AEC_STAGE1_BUILD line in stage1_inst_{unit}.cu"
+        for nw, P, algo, echo, regs in builds:
+            frame = 1024 if unit in ("1024", "ols1024") else 512
+            found.add((unit, frame, int(P), _ALGO_TOKENS[algo], echo == "true", int(nw), int(regs)))
     return found
 
 
