@@ -315,17 +315,6 @@ __global__ void __launch_bounds__(kThreads, 4) features512_kernel(const float* _
 constexpr int kK1k = 513;
 constexpr int kFP1k = 2 * kTilePitch;   // float2 per warp tile
 
-__device__ __forceinline__ TwiddleRegs512 load_twiddles_1k(const Tables& tab, int lane) {
-    TwiddleRegs512 t;
-    t.w1 = __ldg(&tab.tw512w[1 * 32 + lane]);
-    t.w2 = __ldg(&tab.tw512w[2 * 32 + lane]);
-    t.w4 = __ldg(&tab.tw512w[4 * 32 + lane]);
-    t.w8 = __ldg(&tab.tw512w[8 * 32 + lane]);
-    t.wr = (lane >> 4) ? __ldg(&tab.tw512w[16 * 32 + (lane & 15)]) : make_float2(1.f, 0.f);
-    t.sgn = (lane >> 4) ? -1.f : 1.f;
-    return t;
-}
-
 __global__ void __launch_bounds__(kThreads) stft1024_kernel(const float* __restrict__ x, float* __restrict__ spec,
                                                             long long L, long long in_stride, long long T, Tables tab) {
     extern __shared__ __align__(16) unsigned char smem[];
@@ -335,7 +324,7 @@ __global__ void __launch_bounds__(kThreads) stft1024_kernel(const float* __restr
     const long long b = blockIdx.y, t0 = (long long)blockIdx.x * kTT;
     const float* xb = x + b * in_stride;
     float2* tile = tiles + warp * kFP1k;
-    const TwiddleRegs512 twr = load_twiddles_1k(tab, lane);
+    const TwiddleRegs512 twr = TwiddleRegs512::load(tab.tw512w, lane);
     for (int i = 0; i < 4; ++i) {
         const int tt = warp + 4 * i;
         const long long t = t0 + tt;
@@ -396,7 +385,7 @@ __global__ void __launch_bounds__(kThreads) istft1024_kernel(const float* __rest
     }
     __syncthreads();
     float2* tile = tiles + warp * kFP1k;
-    const TwiddleRegs512 twr = load_twiddles_1k(tab, lane);
+    const TwiddleRegs512 twr = TwiddleRegs512::load(tab.tw512w, lane);
     for (int i = 0; i < 4; ++i) {
         const int tt = warp + 4 * i;
 #pragma unroll

@@ -138,6 +138,10 @@ __device__ __forceinline__ void fft256_halfwarp(float2 (&v)[16], float2* tile, c
 // multiplies per call, no memory traffic and no dependence on L1 residency.
 struct TwiddleRegs {
     float2 w1, w2, w4, w8;
+    // from the table tw[q*16 + h] = exp(-2 pi i h q / 256)
+    static __device__ __forceinline__ TwiddleRegs load(const float2* tw, int h) {
+        return {__ldg(&tw[1 * 16 + h]), __ldg(&tw[2 * 16 + h]), __ldg(&tw[4 * 16 + h]), __ldg(&tw[8 * 16 + h])};
+    }
 };
 
 template <bool INV>
@@ -180,6 +184,11 @@ struct TwiddleRegs512 {
     float2 w1, w2, w4, w8;   // exp(-2 pi i l {1,2,4,8} / 512)
     float2 wr;               // lanes 16..31: exp(-2 pi i (l & 15) / 32); lanes 0..15: 1
     float sgn;               // lanes 16..31: -1 (difference); lanes 0..15: +1 (sum)
+    // from the table tw[q*32 + l] = exp(-2 pi i l q / 512), q < 16, whose row 16 is exp(-2 pi i a / 32), a < 16
+    static __device__ __forceinline__ TwiddleRegs512 load(const float2* tw, int lane) {
+        return {__ldg(&tw[1 * 32 + lane]), __ldg(&tw[2 * 32 + lane]), __ldg(&tw[4 * 32 + lane]), __ldg(&tw[8 * 32 + lane]),
+                (lane >> 4) ? __ldg(&tw[16 * 32 + (lane & 15)]) : make_float2(1.f, 0.f), (lane >> 4) ? -1.f : 1.f};
+    }
 };
 
 template <bool INV>

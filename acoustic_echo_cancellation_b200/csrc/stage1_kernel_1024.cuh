@@ -9,8 +9,10 @@
 //     the self-mirrored bin 256 is the last thread's extra, its state in shared memory.
 // STFT conventions: Stage2_lhm/scripts/network/attention_ccrn.py:8-25, 45-52, 82-101 with
 // win_len = fft_len = 1024, win_inc = 512 (golden vectors: tests/golden, arrays *1024).
+// The parameters, the PTX wrappers, the per-bin recurrence (BinState / bin_step) and the real-FFT split it shares with the
+// frame-512 kernel live in stage1_common.cuh.
 #pragma once
-#include "stage1_kernel.cuh"
+#include "stage1_common.cuh"
 
 namespace aec {
 

@@ -50,9 +50,7 @@ __global__ void __launch_bounds__(Ols1024Shape<P>::NT) __maxnreg__(REGS) stage1_
 
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, h = lane & 15, hb = lane >> 4;
 
-    long long n_ll = prm.n_samples ? prm.n_samples[blockIdx.x] : prm.L;
-    n_ll = n_ll < 0 ? 0 : (n_ll > prm.L ? prm.L : n_ll);
-    const int nblk = static_cast<int>(n_ll / HOP);
+    const int nblk = static_cast<int>(utterance_samples(prm, blockIdx.x) / HOP);
     const float* far_b = prm.far + static_cast<long long>(blockIdx.x) * prm.in_stride;
     const float* mic_b = prm.mic + static_cast<long long>(blockIdx.x) * prm.in_stride;
     float* err_b = prm.err + static_cast<long long>(blockIdx.x) * prm.out_stride;
@@ -160,7 +158,7 @@ __global__ void __launch_bounds__(Ols1024Shape<P>::NT) __maxnreg__(REGS) stage1_
                     ols_mid_parallel<P, KAL>(lane, t, midW, midX, midC, midS, tileY + 256, tileW + 256, tileX + 256, prm);
             } else
             if (tid == ((a + 3) & (NW - 1)) * 32 + 31) {              // bin 256, on a warp without a transform
-                auto conj2 = [](float2 z) { return make_float2(2.f * z.x, -2.f * z.y); };   // split / packing twiddle -i
+   // split / packing twiddle -i
                 float2 mw[P], mx[P];                                  // by partition / by delay (as of block t - 1)
                 float mc[PC], ms = *midS;
 #pragma unroll
@@ -171,7 +169,7 @@ __global__ void __launch_bounds__(Ols1024Shape<P>::NT) __maxnreg__(REGS) stage1_
 #pragma unroll
                 for (int p = 0; p < PC; ++p) mc[p] = midC[p];
                 if (t >= 1) {
-                    const float2 ek = conj2(tileY[256]), ca = conj2(tileW[256]);
+                    const float2 ek = mid_conj2(tileY[256]), ca = mid_conj2(tileW[256]);
                     const int cprev = (t - 1) & (P - 1);
 #pragma unroll
                     for (int p = 0; p < P; ++p)
@@ -183,7 +181,7 @@ __global__ void __launch_bounds__(Ols1024Shape<P>::NT) __maxnreg__(REGS) stage1_
 #pragma unroll
                     for (int p = 0; p < P; ++p) midW[p] = mw[p];
                 }
-                const float2 xk = conj2(tileX[256]);
+                const float2 xk = mid_conj2(tileX[256]);
 #pragma unroll
                 for (int p = P - 1; p > 0; --p) mx[p] = mx[p - 1];
                 mx[0] = xk;
@@ -191,12 +189,12 @@ __global__ void __launch_bounds__(Ols1024Shape<P>::NT) __maxnreg__(REGS) stage1_
                 float2 y = make_float2(0.f, 0.f);
 #pragma unroll
                 for (int p = 0; p < P; ++p) y = cfma(mw[p], mx[p], y);
-                tileY[256] = conj2(y);
+                tileY[256] = mid_conj2(y);
                 float2 wc = mw[0];
 #pragma unroll
                 for (int p = 1; p < P; ++p)
                     if (c == p) wc = mw[p];
-                tileW[256] = conj2(wc);
+                tileW[256] = mid_conj2(wc);
             }
         }
         cp_async_wait<1>();                                           // blocks staged one iteration ago have landed
@@ -275,24 +273,13 @@ __global__ void __launch_bounds__(Ols1024Shape<P>::NT) __maxnreg__(REGS) stage1_
         if constexpr (ECHO) echo_b[i] = 0.f;
     }
     if (prm.erle_db != nullptr) {
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) {
-            acc_m += __shfl_xor_sync(0xffffffffu, acc_m, o);
-            acc_e += __shfl_xor_sync(0xffffffffu, acc_e, o);
-        }
+        warp_sum2<16>(acc_m, acc_e);
         if (lane == 0) {
             red[2 * warp] = acc_m;
             red[2 * warp + 1] = acc_e;
         }
         __syncthreads();
-        if (tid == 0) {
-            float m = 0.f, e = 0.f;
-            for (int w = 0; w < NW; ++w) {
-                m += red[2 * w];
-                e += red[2 * w + 1];
-            }
-            prm.erle_db[blockIdx.x] = 10.f * log10f(fmaxf(m, 1e-20f) / fmaxf(e, 1e-20f));
-        }
+        if (tid == 0) store_erle(red, NW, prm, blockIdx.x);
     }
 }
 

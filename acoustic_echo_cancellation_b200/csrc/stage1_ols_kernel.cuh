@@ -2,7 +2,8 @@
 // constraint (time-domain blocks of H = 256 new samples, FFT length 512, P partitions), NLMS step (algo 2) or the
 // diagonal Kalman step of algo 1 (algo 3).  One persistent CTA of two warps per utterance; filter taps, far-end
 // history and the power / covariance state stay in registers for the whole utterance, like the STFT-domain kernels
-// (stage1_kernel.cuh), whose half-warp FFT-256, real-FFT split and bin ownership it shares.
+// (stage1_kernel.cuh), whose bin ownership it shares, and with their half-warp FFT-256 (fft_warp.cuh) and real-FFT split
+// (stage1_common.cuh).
 //
 // Unlike them the recurrence crosses the transform every block -- e(t) needs W(t), W(t) needs E(t-1) = FFT(e(t-1)) --
 // so there is no chunk of frames to batch and the length of the per-block dependency chain is what counts.  Five
@@ -29,7 +30,7 @@
 // holds 14 dB through double talk (DESIGN.md section 2).
 // BUILDER-AUTHORED (the reference has no stage-1 filter): restated by oracle/aec_oracle.py:pbfdaf_ols, parity unpinned.
 #pragma once
-#include "stage1_kernel.cuh"
+#include "stage1_common.cuh"
 
 namespace aec {
 
@@ -49,15 +50,6 @@ struct OlsSmem {
         return base(P) + (ring(P, kalman) ? size_t(P) * 256 * sizeof(float2) : 0);
     }
 };
-
-__device__ __forceinline__ void cp_async16(void* dst_smem, const void* src_gmem) {
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(smem_u32(dst_smem)), "l"(src_gmem) : "memory");
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void cp_async_wait() {
-    asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory");
-}
 
 // Weight update of one bin with the error spectrum E of the block (operation order of oracle/aec_oracle.py).
 // ROT: W / C are in rotating positions (position j = partition (j + t) mod P), X is the ring (slot = block mod P):
@@ -198,9 +190,7 @@ __global__ void __launch_bounds__(OlsShape<P>::NT) __maxnreg__(REGS) stage1_ols_
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, half = lane >> 4, h = lane & 15;
     const int side = tid & 1;                                        // kSplit: 0 = bin k, 1 = bin 256 - k of pair k = tid >> 1
 
-    long long n_ll = prm.n_samples ? prm.n_samples[blockIdx.x] : prm.L;
-    n_ll = n_ll < 0 ? 0 : (n_ll > prm.L ? prm.L : n_ll);
-    const int nblk = static_cast<int>(n_ll / 256);
+    const int nblk = static_cast<int>(utterance_samples(prm, blockIdx.x) / 256);
     const float* far_b = prm.far + static_cast<long long>(blockIdx.x) * prm.in_stride;
     const float* mic_b = prm.mic + static_cast<long long>(blockIdx.x) * prm.in_stride;
     float* err_b = prm.err + static_cast<long long>(blockIdx.x) * prm.out_stride;
@@ -233,18 +223,11 @@ __global__ void __launch_bounds__(OlsShape<P>::NT) __maxnreg__(REGS) stage1_ols_
 #endif
     // tuning (aec_cfg.stagger_ns > 0): start-up skew between the utterances that share an SM, so that the issue-bound
     // update phase of one meets the latency-bound transform phase of another instead of all of them running in step
-    if (prm.stagger_ns > 0) {
-        const unsigned slot = (unsigned)(blockIdx.x / (unsigned)prm.num_sms) & 7u;
-        if (slot) __nanosleep(slot * (unsigned)prm.stagger_ns);
-    }
+    startup_skew(prm);
     __syncthreads();
     const int fw = *fft_warp_s;
 
-    TwiddleRegs twr;
-    twr.w1 = __ldg(&prm.tw256[1 * 16 + h]);
-    twr.w2 = __ldg(&prm.tw256[2 * 16 + h]);
-    twr.w4 = __ldg(&prm.tw256[4 * 16 + h]);
-    twr.w8 = __ldg(&prm.tw256[8 * 16 + h]);
+    const TwiddleRegs twr = TwiddleRegs::load(prm.tw256, h);
 
     // ---- persistent per-bin state ----
     float2 W[NB][P], Xp[kXs ? 1 : NB][kXs ? 1 : P];
@@ -366,8 +349,7 @@ __global__ void __launch_bounds__(OlsShape<P>::NT) __maxnreg__(REGS) stage1_ols_
                     ols_mid_parallel<P, KAL>(lane, t, midW, midX, midC, midS, tileY + 128, tileW + 128, tX + 128, prm);
             } else
             if (tid == ((a + 1) & (NW - 1)) * 32 + 31) {              // bin 128, on a warp with a light transform phase
-                // its split / packing twiddle is -i: the real-signal bin is 2 conj(Z[128]), and back (exact, no multiplies)
-                auto conj2 = [](float2 z) { return make_float2(2.f * z.x, -2.f * z.y); };
+                // its split / packing twiddle is -i: the real-signal bin is 2 conj(Z[128]), and back (mid_conj2)
                 float2 mw[P], mx[P];                                  // by partition / by delay (as of block t - 1)
                 float mc[PC], ms = *midS;
 #pragma unroll
@@ -378,7 +360,7 @@ __global__ void __launch_bounds__(OlsShape<P>::NT) __maxnreg__(REGS) stage1_ols_
 #pragma unroll
                 for (int p = 0; p < PC; ++p) mc[p] = midC[p];
                 if (t >= 1) {
-                    const float2 ek = conj2(tileY[128]), ca = conj2(tileW[128]);
+                    const float2 ek = mid_conj2(tileY[128]), ca = mid_conj2(tileW[128]);
                     const int cprev = (t - 1) & (P - 1);
 #pragma unroll
                     for (int p = 0; p < P; ++p)
@@ -390,7 +372,7 @@ __global__ void __launch_bounds__(OlsShape<P>::NT) __maxnreg__(REGS) stage1_ols_
 #pragma unroll
                     for (int p = 0; p < P; ++p) midW[p] = mw[p];
                 }
-                const float2 xk = conj2(tX[128]);
+                const float2 xk = mid_conj2(tX[128]);
 #pragma unroll
                 for (int p = P - 1; p > 0; --p) mx[p] = mx[p - 1];
                 mx[0] = xk;
@@ -398,12 +380,12 @@ __global__ void __launch_bounds__(OlsShape<P>::NT) __maxnreg__(REGS) stage1_ols_
                 float2 y = make_float2(0.f, 0.f);
 #pragma unroll
                 for (int p = 0; p < P; ++p) y = cfma(mw[p], mx[p], y);
-                tileY[128] = conj2(y);
+                tileY[128] = mid_conj2(y);
                 float2 wc = mw[0];
 #pragma unroll
                 for (int p = 1; p < P; ++p)
                     if (c == p) wc = mw[p];
-                tileW[128] = conj2(wc);
+                tileW[128] = mid_conj2(wc);
             }
         }
         AEC_TICK(0);                                                  // R
@@ -486,10 +468,7 @@ __global__ void __launch_bounds__(OlsShape<P>::NT) __maxnreg__(REGS) stage1_ols_
     cp_async_wait<0>();
 
     // ---- epilogue: zero the output beyond the last whole block, ERLE ----
-    for (long long i = static_cast<long long>(nblk) * 256 + tid; i < prm.out_stride && i < prm.L; i += NT) {
-        err_b[i] = 0.f;
-        if constexpr (ECHO) echo_b[i] = 0.f;
-    }
+    zero_output_tail<ECHO>(err_b, echo_b, static_cast<long long>(nblk) * 256, prm, tid, NT);
     if (prm.erle_db != nullptr) {
 #pragma unroll
         for (int o = 8; o > 0; o >>= 1) {
@@ -501,14 +480,7 @@ __global__ void __launch_bounds__(OlsShape<P>::NT) __maxnreg__(REGS) stage1_ols_
             red[2 * warp + 1] = acc_e;
         }
         __syncthreads();
-        if (tid == 0) {
-            float m = 0.f, e = 0.f;
-            for (int w = 0; w < NW; ++w) {
-                m += red[2 * w];
-                e += red[2 * w + 1];
-            }
-            prm.erle_db[blockIdx.x] = 10.f * log10f(fmaxf(m, 1e-20f) / fmaxf(e, 1e-20f));
-        }
+        if (tid == 0) store_erle(red, NW, prm, blockIdx.x);
     }
 #ifdef AEC_PHASE_TIMING
     if (lane == 0 && prm.dbg)
