@@ -8,7 +8,7 @@ CPU fallback.  See DESIGN.md / INTEGRATION.md.
 """
 from ._lib import ALGO_KALMAN, ALGO_NLMS, ALGO_PBFDAF, ALGO_PBFKF, AecError, LIB_PATH  # noqa: F401
 from .stage1 import (HOST_PORTABLE, HOST_WRITE_COMBINED, DelayConfig, HostPipeline, Stage1Config,  # noqa: F401
-                     align_far, estimate_delay, fp32_peak_tflops, is_pinned, launch_count, num_frames, out_samples,
+                     Stage1Stream, align_far, estimate_delay, fp32_peak_tflops, is_pinned, launch_count, num_frames, out_samples,
                      pinned_empty, stage1_aec, stage1_aec_features)
 from .spectral import ConvSTFT, ConviSTFT, batch_shift, erb_filterbank, stage2_features  # noqa: F401
 from .stage2 import LittleNetInference  # noqa: F401
@@ -18,5 +18,5 @@ __all__ = [
     "launch_count", "num_frames", "out_samples", "pinned_empty", "is_pinned", "HOST_WRITE_COMBINED",
     "HOST_PORTABLE", "stage1_aec", "stage1_aec_features", "ConvSTFT", "ConviSTFT",
     "erb_filterbank", "stage2_features", "batch_shift", "LittleNetInference", "DelayConfig", "estimate_delay",
-    "align_far",
+    "align_far", "Stage1Stream",
 ]

@@ -80,6 +80,10 @@ SIGNATURES = {
     "aec_out_samples": (_I64, [_I64, _I32]),
     "aec_stage1_run": (C.c_int, [_P, _P, _P, _P, _P, _P, _I64, _I64, _I64, _I64, C.POINTER(AecCfg), _P]),
     "aec_stage1_run_features": (C.c_int, [_P, _P, _P, _P, _P, _P, _P, _I64, _I64, _I64, _I64, C.POINTER(AecCfg), _P]),
+    "aec_stage1_state_bytes": (_I64, [C.POINTER(AecCfg)]),
+    "aec_stage1_state_init": (C.c_int, [_P, _I64, _I64, _P, C.POINTER(AecCfg), _P]),
+    "aec_stage1_run_stream": (C.c_int, [_P, _P, _P, _P, _P, _P, _I64, _I64, _I64, _I64, C.POINTER(AecCfg), _P, _I64,
+                                        _P]),
     "aec_host_ctx_create": (C.c_int, [C.POINTER(_P), _I64, _I64]),
     "aec_host_ctx_create_ex": (C.c_int, [C.POINTER(_P), _I64, _I64, _I32, _I32]),
     "aec_host_ctx_destroy": (C.c_int, [_P]),

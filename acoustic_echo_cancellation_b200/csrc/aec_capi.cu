@@ -289,7 +289,8 @@ extern "C" void aec_debug_set_phase_buffer(void* p) { g_phase_buffer = static_ca
 
 static int stage1_run_impl(const float* far, const float* mic, float* err, float* echo_est, float* erle_db,
                            const int64_t* n_samples, int64_t B, int64_t L, int64_t in_stride, int64_t out_stride,
-                           const aec_cfg* cfg, void* cuda_stream, float* feat, const float* erb) {
+                           const aec_cfg* cfg, void* cuda_stream, float* feat, const float* erb,
+                           void* state = nullptr, int64_t state_stride = 0) {
     int rc = validate_cfg(cfg);
     if (rc != AEC_OK) return rc;
     if (B < 0 || L < 0 || in_stride < L || out_stride < L) return AEC_EINVAL;
@@ -331,6 +332,8 @@ static int stage1_run_impl(const float* far, const float* mic, float* err, float
     p.feat = feat;
     p.erb = erb;
     p.feat_frames = aec_num_frames(L, cfg->frame);
+    p.state = static_cast<unsigned char*>(state);
+    p.state_stride = state_stride;
 #ifdef AEC_PHASE_TIMING
     p.dbg = g_phase_buffer;
 #endif
@@ -363,7 +366,9 @@ static int stage1_run_impl(const float* far, const float* mic, float* err, float
         regs = cfg->variant % 1000;
     }
     Stage1Launch (*lookup)(int P, int algo, bool echo, int nw, int regs) = nullptr;
-    if (feat) {
+    if (state) {
+        lookup = stage1_build_ols_stream;          // (aec_stage1_run_stream has refused every other configuration)
+    } else if (feat) {
         lookup = stage1_build_feat;
         // 4-partition NLMS: five utterances per SM (168 registers) win on many-wave batches (4144 x 10 s: 8.79 vs
         // 9.36 ms); for batches of a wave or two the launch ends with a thin last wave either way and four per SM at 200
@@ -411,6 +416,57 @@ extern "C" int aec_stage1_run_features(const float* far, const float* mic, float
     if (!feat || !erb) return AEC_EINVAL;
     return stage1_run_impl(far, mic, err, nullptr, erle_db, n_samples, B, L, in_stride, out_stride, cfg, cuda_stream, feat,
                            erb);
+}
+
+// ------------------------------------------------------------------------------------------
+// stage 1, streaming: the frame-512 overlap-save filters with their state in caller-owned device memory
+// ------------------------------------------------------------------------------------------
+// State bytes of one stream, or the code the streaming entries refuse cfg with (no launch).
+static int64_t stream_state_bytes(const aec_cfg* cfg) {
+    const int rc = validate_cfg(cfg);
+    if (rc != AEC_OK) return rc;
+    if (cfg->algo != AEC_ALGO_PBFDAF && cfg->algo != AEC_ALGO_PBFKF) return AEC_EUNSUPPORTED;
+    if (cfg->frame != 512 || cfg->variant != 0) return AEC_EUNSUPPORTED;
+    const int P = cfg->partitions;
+    if (P != 1 && P != 2 && P != 4 && P != 8 && P != 16) return AEC_EUNSUPPORTED;
+    return OlsStreamState::bytes(P, cfg->algo == AEC_ALGO_PBFKF);
+}
+
+static int check_state(const void* state, int64_t state_stride, const aec_cfg* cfg) {
+    const int64_t bytes = stream_state_bytes(cfg);
+    if (bytes < 0) return (int)bytes;
+    if (!state || (reinterpret_cast<uintptr_t>(state) & 15) != 0) return AEC_EINVAL;
+    if (state_stride < bytes || (state_stride % 16) != 0) return AEC_EINVAL;
+    return AEC_OK;
+}
+
+extern "C" int64_t aec_stage1_state_bytes(const aec_cfg* cfg) { return stream_state_bytes(cfg); }
+
+extern "C" int aec_stage1_state_init(void* state, int64_t B, int64_t state_stride, const uint8_t* reset_mask,
+                                     const aec_cfg* cfg, void* cuda_stream) {
+    int rc = check_state(state, state_stride, cfg);
+    if (rc != AEC_OK) return rc;
+    if (B < 0 || B > 0x7fffffffLL) return AEC_EINVAL;
+    if (B == 0) return AEC_OK;
+    const cudaError_t e = ols_stream_state_init(state, B, state_stride, reset_mask, cfg->partitions,
+                                                cfg->algo == AEC_ALGO_PBFKF, cfg->kalman_c0,
+                                                static_cast<cudaStream_t>(cuda_stream));
+    if (e != cudaSuccess) {
+        set_cuda_error(e, "aec_stage1_state_init");
+        return AEC_ECUDA;
+    }
+    count_launch();
+    return AEC_OK;
+}
+
+extern "C" int aec_stage1_run_stream(const float* far, const float* mic, float* err, float* echo_est, float* erle_db,
+                                     const int64_t* n_samples, int64_t B, int64_t L, int64_t in_stride,
+                                     int64_t out_stride, const aec_cfg* cfg, void* state, int64_t state_stride,
+                                     void* cuda_stream) {
+    const int rc = check_state(state, state_stride, cfg);
+    if (rc != AEC_OK) return rc;
+    return stage1_run_impl(far, mic, err, echo_est, erle_db, n_samples, B, L, in_stride, out_stride, cfg, cuda_stream,
+                           nullptr, nullptr, state, state_stride);
 }
 
 // ------------------------------------------------------------------------------------------

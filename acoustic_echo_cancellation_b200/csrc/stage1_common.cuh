@@ -36,9 +36,30 @@ struct Stage1Params {
     float* feat;           // [B][feat_frames][64]  cat[err_erb, |err_erb - far_erb|]
     const float* erb;      // [257][32] dense cosine bank (ERB.py:10-71), device memory
     long long feat_frames; // rows per utterance (frames of an L-sample signal)
+    // streaming overlap-save builds only (stage1_ols_stream_kernel): row b's filter state at state + b * state_stride,
+    // laid out as OlsStreamState says
+    unsigned char* state;
+    long long state_stride;
 #ifdef AEC_PHASE_TIMING
     long long* dbg;        // developer build only: [B][NW][12] cycles per phase (tools/phase_timing.py)
 #endif
+};
+
+// State of one stream of the frame-512 overlap-save filter after T blocks (include/aec_b200.h, DESIGN.md section 5d): the
+// quantities of oracle/aec_oracle.py:pbfdaf_ols in its rfft units, K = 257 bins, every array on a 16-byte boundary.
+//   blocks int64 (+ 8 reserved bytes) | prev float[256] = x_{T-1} | W complex[P][K] by partition | X complex[P][K],
+//   X[p] = rfft([x_{T-2-p}, x_{T-1-p}]) | algo 2: Pw float[K] | algo 3: Psi float[K], C float[P][K] by partition
+struct OlsStreamState {
+    static constexpr int K = 257;
+    __host__ __device__ static constexpr long long a16(long long n) { return (n + 15) / 16 * 16; }
+    __host__ __device__ static constexpr long long prev() { return 16; }
+    __host__ __device__ static constexpr long long W() { return prev() + 256 * 4; }
+    __host__ __device__ static constexpr long long X(int P) { return W() + a16(8LL * P * K); }
+    __host__ __device__ static constexpr long long S(int P) { return X(P) + a16(8LL * P * K); }     // Pw / Psi
+    __host__ __device__ static constexpr long long C(int P) { return S(P) + a16(4LL * K); }         // algo 3
+    __host__ __device__ static constexpr long long bytes(int P, bool kalman) {
+        return kalman ? C(P) + a16(4LL * P * K) : C(P);
+    }
 };
 
 // Developer instrumentation (compiled out of the product library): lane 0 of every warp accumulates

@@ -1,4 +1,4 @@
-// Launcher glue between the C ABI and the templated stage-1 kernels.  The kernels are built in the eight
+// Launcher glue between the C ABI and the templated stage-1 kernels.  The kernels are built in the nine
 // stage1_inst_*.cu units (split so that the build parallelises); each unit is one look-up function that lists its
 // builds, one AEC_STAGE1_BUILD line per build, and returns the launch function of the build a call asks for.
 #pragma once
@@ -55,6 +55,11 @@ Stage1Launch stage1_build_1024(int P, int algo, bool echo, int nw, int regs);
 Stage1Launch stage1_build_feat(int P, int algo, bool echo, int nw, int regs);     // with the fused Stage-2 features
 Stage1Launch stage1_build_ols(int P, int algo, bool echo, int nw, int regs);
 Stage1Launch stage1_build_ols1024(int P, int algo, bool echo, int nw, int regs);
+// streaming overlap-save builds (frame 512; the filter state crosses the call, OlsStreamState) and their state set-up:
+// rows b with mask null or mask[b] != 0 of the B states at state + b * stride are reset (one launch)
+Stage1Launch stage1_build_ols_stream(int P, int algo, bool echo, int nw, int regs);
+cudaError_t ols_stream_state_init(void* state, long long B, long long stride, const uint8_t* mask, int P, bool kalman,
+                                  float c0, cudaStream_t s);
 
 // One build of a unit: NW warps per utterance, P partitions, algorithm, echo-estimate output, register cap.  Build<...>
 // is the unit's kernel family: its kernel and dynamic shared memory, and, where the kernel fixes its warp count, a

@@ -310,6 +310,123 @@ def stage1_aec_features(far: torch.Tensor, mic: torch.Tensor, erb: torch.Tensor,
 _checked_banks = set()
 
 
+class Stage1Stream:
+    """Online stage 1 for ``streams`` live calls (``aec_stage1_run_stream``): the frame-512 overlap-save filters
+    (algo 2 / 3) with each stream's filter state kept on the device between calls, so that a chunk continues where the
+    previous one stopped.  Chunked processing gives bit for bit the output of ``stage1_aec`` over the whole signal.
+
+    ``process`` takes chunks of any length.  The kernel consumes whole blocks of 256 samples; up to 255 samples per
+    stream wait here for the next chunk, so the output lags the input by at most one block (16 ms at 16 kHz).
+    ``state`` is the ``uint8 [streams, state_stride]`` device tensor of the states (layout: include/aec_b200.h)."""
+
+    HOP = 256
+
+    def __init__(self, streams: int, cfg: Optional[Stage1Config] = None, device=None):
+        self.cfg = cfg or Stage1Config(algo=ALGO_PBFDAF)
+        self._c = self.cfg.to_c()
+        self._lib = _lib.load()
+        nbytes = int(self._lib.aec_stage1_state_bytes(C.byref(self._c)))
+        _lib.check(min(nbytes, 0), "aec_stage1_state_bytes")
+        self.streams = int(streams)
+        self.state_bytes = nbytes
+        self.state_stride = (nbytes + 15) // 16 * 16
+        self.device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
+        with torch.cuda.device(self.device):
+            self.state = torch.empty((self.streams, self.state_stride), dtype=torch.uint8, device=self.device)
+            # pending samples, right-aligned: row b's last _npend[b] columns
+            self._pend = torch.zeros((2, self.streams, self.HOP - 1), dtype=torch.float32, device=self.device)
+            self._npend = torch.zeros((self.streams,), dtype=torch.int64, device=self.device)
+        self.reset()
+
+    def reset(self, rows=None):
+        """Re-initialise the filter state and drop the pending samples of ``rows`` (a bool mask or indices; None: all)."""
+        mask = None
+        with torch.cuda.device(self.device):
+            if rows is not None:
+                rows = torch.as_tensor(rows, device=self.device)
+                if rows.dtype == torch.bool:
+                    mask = rows.to(torch.uint8).contiguous()
+                else:
+                    mask = torch.zeros((self.streams,), dtype=torch.uint8, device=self.device)
+                    mask[rows.to(torch.int64)] = 1
+                if mask.numel() != self.streams:
+                    raise ValueError("rows: a mask of one entry per stream, or stream indices")
+            rc = self._lib.aec_stage1_state_init(self.state.data_ptr(), self.streams, self.state_stride,
+                                                 mask.data_ptr() if mask is not None else None, C.byref(self._c),
+                                                 _stream_ptr(self.state))
+            _lib.check(rc, "aec_stage1_state_init")
+            if mask is None:
+                self._npend.zero_()
+            else:
+                self._npend.masked_fill_(mask.bool(), 0)
+
+    def state_views(self) -> dict:
+        """Named views into ``state`` (writable, aliasing it): ``blocks`` int64 [S], ``prev`` float32 [S, 256], ``W`` and
+        ``X`` complex64 [S, P, 257], then ``Pw`` float32 [S, 257] (algo 2) or ``Psi`` [S, 257] and ``C`` [S, P, 257]
+        (algo 3).  The one place on the Python side that knows the layout."""
+        P, K = self.cfg.partitions, 257
+        a16 = lambda n: (n + 15) // 16 * 16       # noqa: E731
+        w0 = 16 + 4 * self.HOP
+        x0 = w0 + a16(8 * P * K)
+        s0 = x0 + a16(8 * P * K)
+        c0 = s0 + a16(4 * K)
+        st = self.state
+
+        def f32(off, n):
+            return st[:, off:off + 4 * n].view(torch.float32)
+
+        v = {"blocks": st[:, 0:8].view(torch.int64)[:, 0],
+             "prev": f32(16, self.HOP),
+             "W": st[:, w0:w0 + 8 * P * K].view(torch.complex64).unflatten(1, (P, K)),
+             "X": st[:, x0:x0 + 8 * P * K].view(torch.complex64).unflatten(1, (P, K))}
+        if self.cfg.algo == ALGO_PBFKF:
+            v["Psi"] = f32(s0, K)
+            v["C"] = f32(c0, P * K).unflatten(1, (P, K))
+        else:
+            v["Pw"] = f32(s0, K)
+        return v
+
+    def process(self, far: torch.Tensor, mic: torch.Tensor, return_echo: bool = False, return_erle: bool = False):
+        """One chunk of every stream: far, mic [streams, L] float32 CUDA, any L >= 0.  Returns ``err`` [streams, M] and
+        ``n_out`` int64 [streams] (M = the most whole-block samples any row can have; row b's output is its first
+        ``n_out[b]`` samples, zero beyond), then ``echo`` [streams, M] and ``erle_db`` [streams] (over this call's blocks
+        from ``erle_skip_hops`` blocks into the stream) when asked for.  Asynchronous on the current stream."""
+        far, mic = _pair(far, mic)
+        if far.shape[0] != self.streams or far.device != self.device:
+            raise ValueError(f"far and mic must be [{self.streams}, L] tensors on {self.device}")
+        B, L = far.shape
+        H, R = self.HOP, self.HOP - 1
+        width = (R + L + 3) // 4 * 4                                  # 16-byte rows: the bulk-copy staging path
+        M = (R + L) // H * H
+        with torch.cuda.device(self.device):
+            # row b: its pending samples, then the chunk; gathered from [pending (right-aligned) | chunk]
+            both = torch.cat([self._pend, torch.stack([far, mic])], dim=2)                # [2, B, R + L]
+            n = self._npend + L
+            idx = (R - self._npend)[:, None] + torch.arange(width, device=self.device)[None, :]
+            inp = torch.gather(both, 2, idx.clamp(max=R + L - 1).expand(2, B, width))
+            inp.masked_fill_((idx >= R + L).expand(2, B, width), 0.0)
+            n_out = n // H * H
+            err = torch.empty((B, width), dtype=torch.float32, device=self.device)
+            echo = torch.empty_like(err) if return_echo else None
+            erle = torch.empty((B,), dtype=torch.float32, device=self.device) if return_erle else None
+            rc = self._lib.aec_stage1_run_stream(inp[0].data_ptr(), inp[1].data_ptr(), err.data_ptr(),
+                                                 echo.data_ptr() if echo is not None else None,
+                                                 erle.data_ptr() if erle is not None else None,
+                                                 n.data_ptr(), B, width, width, width, C.byref(self._c),
+                                                 self.state.data_ptr(), self.state_stride, _stream_ptr(far))
+            _lib.check(rc, "aec_stage1_run_stream")
+            # the samples past the last whole block wait for the next chunk
+            tail = (n - R)[:, None] + torch.arange(R, device=self.device)[None, :]
+            self._pend = torch.gather(inp, 2, tail.clamp(min=0).expand(2, B, R))
+            self._npend = n - n_out
+        res = [err[:, :M], n_out]
+        if return_echo:
+            res.append(echo[:, :M])
+        if return_erle:
+            res.append(erle)
+        return tuple(res)
+
+
 class HostPipeline:
     """Host-buffer entry (``aec_stage1_run_host``; ``aec_stage1_run_host_pcm16`` for int16 PCM inputs,
     scaled by 1/32768 on the GPU): numpy arrays in, numpy arrays out, copies pipelined against the kernel

@@ -125,6 +125,34 @@ int aec_stage1_run_features(const float* far, const float* mic, float* err, floa
                             const int64_t* n_samples, int64_t B, int64_t L, int64_t in_stride, int64_t out_stride,
                             const aec_cfg* cfg, void* cuda_stream);
 
+/* Streaming stage 1 (online use: a chunk of every live stream per call) for the frame-512 overlap-save filters
+ * (algos 2 / 3, partitions 1 / 2 / 4 / 8 / 16, variant 0).  Each stream's filter state lives in caller-owned DEVICE
+ * memory, row b at state + b * state_stride (16-byte aligned; state_stride >= aec_stage1_state_bytes, a multiple of 16).
+ * Chunked calls give bit for bit the outputs of one aec_stage1_run over the whole signal.
+ * State of one stream after T blocks (the quantities of oracle/aec_oracle.py:pbfdaf_ols in its rfft units, K = 257 bins,
+ * little-endian, every array starting on a 16-byte boundary, the gaps zero):
+ *   offset 0                  int64 blocks = T (+ 8 reserved bytes, zero)
+ *   16                        float prev[256]: the far-end samples of block T - 1 (zeros at T = 0)
+ *   1040                      complex64 W[P][K]: taps by partition p, after the update with E_{T-1}
+ *   1040 + a16(8 P K)         complex64 X[P][K]: X[p] = rfft([x_{T-2-p}, x_{T-1-p}])
+ *   1040 + 2 a16(8 P K)       algo 2: float Pw[K] (smoothed input power); algo 3: float Psi[K] (observation-noise power),
+ *   ... + a16(4 K)            then (algo 3) float C[P][K] (covariances)                    a16(n) = n rounded up to 16
+ * After aec_stage1_state_init: T = 0 and every other byte zero, except C = kalman_c0.
+ * aec_stage1_state_bytes: bytes of one stream's state for cfg, or AEC_EUNSUPPORTED for algos 0 / 1, frame 1024, a
+ *   variant or an unbuilt P (a negative AEC_E* code).
+ * aec_stage1_state_init: (re)initialises rows b with reset_mask == NULL or reset_mask[b] != 0 (nullable DEVICE uint8 [B]);
+ *   the other rows are left untouched.  One launch on the caller's stream.
+ * aec_stage1_run_stream: aec_stage1_run's arguments for one chunk per stream.  Row b consumes n_b / 256 whole blocks
+ *   (n_b = n_samples[b] or L): it writes that many blocks of err / echo_est, zeros beyond them up to L, and the caller
+ *   keeps its remaining n_b mod 256 samples for the next call.  erle_db covers this call's blocks whose index in the
+ *   stream is >= erle_skip_hops (0 dB without any).  A row without a whole block leaves its state untouched. */
+int64_t aec_stage1_state_bytes(const aec_cfg* cfg);
+int aec_stage1_state_init(void* state, int64_t B, int64_t state_stride, const uint8_t* reset_mask, const aec_cfg* cfg,
+                          void* cuda_stream);
+int aec_stage1_run_stream(const float* far, const float* mic, float* err, float* echo_est, float* erle_db,
+                          const int64_t* n_samples, int64_t B, int64_t L, int64_t in_stride, int64_t out_stride,
+                          const aec_cfg* cfg, void* state, int64_t state_stride, void* cuda_stream);
+
 /* Host-buffer variant: the call a data-prep script makes with arrays that came out of
  * `librosa.load` (Stage2_lhm/generate_h5files/train_wav2h5.py:20-23) and whose results go to
  * `create_dataset` (train_wav2h5.py:39-42).  Copies are pipelined against the kernel in
