@@ -11,12 +11,12 @@ from .stage1 import (HOST_PORTABLE, HOST_WRITE_COMBINED, DelayConfig, HostPipeli
                      Stage1Stream, align_far, estimate_delay, fp32_peak_tflops, is_pinned, launch_count, num_frames, out_samples,
                      pinned_empty, stage1_aec, stage1_aec_features)
 from .spectral import ConvSTFT, ConviSTFT, batch_shift, erb_filterbank, stage2_features  # noqa: F401
-from .stage2 import LittleNetInference  # noqa: F401
+from .stage2 import AecStream, LittleNetInference, Stage2Stream  # noqa: F401
 
 __all__ = [
     "ALGO_KALMAN", "ALGO_NLMS", "ALGO_PBFDAF", "ALGO_PBFKF", "AecError", "LIB_PATH", "HostPipeline", "Stage1Config", "fp32_peak_tflops",
     "launch_count", "num_frames", "out_samples", "pinned_empty", "is_pinned", "HOST_WRITE_COMBINED",
     "HOST_PORTABLE", "stage1_aec", "stage1_aec_features", "ConvSTFT", "ConviSTFT",
     "erb_filterbank", "stage2_features", "batch_shift", "LittleNetInference", "DelayConfig", "estimate_delay",
-    "align_far", "Stage1Stream",
+    "align_far", "Stage1Stream", "Stage2Stream", "AecStream",
 ]

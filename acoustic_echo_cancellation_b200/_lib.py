@@ -115,6 +115,10 @@ SIGNATURES = {
     "aec_stage2_synth_dev": (C.c_int, [_P, _P, _P, _P, _I64, _I64, _I64, _I64, _I32, _I32, _P, _P]),
     "aec_stage2_mask": (C.c_int, [_P, C.POINTER(Stage2Weights), _P, _I64, _I64, _I32, _P]),
     "aec_stage2_synth": (C.c_int, [_P, _P, _P, _P, _I64, _I64, _I64, _I64, _I32, _I32, C.c_float, _P]),
+    "aec_stage2_state_bytes": (_I64, []),
+    "aec_stage2_state_init": (C.c_int, [_P, _I64, _I64, _P, _P]),
+    "aec_stage2_run_stream": (C.c_int, [_P, _P, _P, C.POINTER(Stage2Weights), _P, _P, _I64, _I64, _I64, _I64, _P, _I64,
+                                        _I32, _P]),
     "aec_bench_fp32_peak": (C.c_int, [C.c_int, C.POINTER(C.c_double), _P]),
     "aec_launch_count": (_I64, [C.c_int]),
 }

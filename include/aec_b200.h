@@ -332,6 +332,34 @@ int aec_stage2_synth_dev(const float* mic, const float* est_erb, const float* er
                          int64_t in_stride, int64_t out_stride, int32_t frame, int32_t bands, const float* shift_mic_dev,
                          void* cuda_stream);
 
+/* Streaming Stage 2 (online use: the new hops of every live stream per call): features, GRU, mask, gain, inverse STFT
+ * and overlap-add of Little_net in one launch, without the batch-global input shift (in_norm off, ERB.py:254-256 needs
+ * the whole signal).  Frame 512, hop 256, 32 bands.  Each stream's state lives in caller-owned DEVICE memory, row b at
+ * state + b * state_stride (16-byte aligned; state_stride >= aec_stage2_state_bytes(), a multiple of 16).
+ * State of one stream after T frames (little-endian, 3216 bytes):
+ *   offset 0      int64 frames = T (+ 8 reserved bytes, zero)
+ *   16            float h[32]: the GRU state after frame T - 1
+ *   144           float mic_prev[256]: hop T - 1 of the mic input (zeros at T = 0)
+ *   1168          float ref_prev[256]: hop T - 1 of the ref input
+ *   2192          float ola[256]: the windowed second half of frame T - 1 (without the + 1e-9)
+ * After aec_stage2_state_init every byte is zero.
+ * aec_stage2_state_init: (re)initialises rows b with reset_mask == NULL or reset_mask[b] != 0 (nullable DEVICE uint8
+ *   [B]); the other rows and the bytes past aec_stage2_state_bytes() are left untouched.  One launch.
+ * aec_stage2_run_stream: mic (the stage-1 error or the microphone), ref (the far end) [B][in_stride]; row b consumes
+ *   n_b / 256 whole hops (n_b = n_samples[b] or L; n_samples a nullable DEVICE int64 [B]) and computes frames
+ *   T0 .. T0+n-1; it writes output blocks T0-1 .. T0+n-2 to out [B][out_stride] from column 0 (block -1 is not part of
+ *   the signal: a stream's first call with hops writes one block fewer) and zeros after them up to L.  The caller keeps
+ *   the remaining n_b mod 256 samples for the next call.  A row without a whole hop leaves its state untouched.  Chunked
+ *   calls give bit for bit the output of one call over the whole stream; fed one more hop (the last samples zero-padded),
+ *   the concatenated output is the (T-1) * 256 samples of the whole-utterance path with in_norm off (to rounding).
+ *   bands != 32: AEC_EUNSUPPORTED; a null or misaligned state or weight pointer, a bad stride or B < 0: AEC_EINVAL.
+ *   Every refusal launches nothing. */
+int64_t aec_stage2_state_bytes(void);
+int aec_stage2_state_init(void* state, int64_t B, int64_t state_stride, const uint8_t* reset_mask, void* cuda_stream);
+int aec_stage2_run_stream(const float* mic, const float* ref, const float* erb, const aec_stage2_weights* w, float* out,
+                          const int64_t* n_samples, int64_t B, int64_t L, int64_t in_stride, int64_t out_stride,
+                          void* state, int64_t state_stride, int32_t bands, void* cuda_stream);
+
 /* Measurement helpers used by bench.py (not part of the reference-facing surface).
  * aec_bench_fp32_peak: dependent-free FFMA loop on every SM; returns achieved FP32 TFLOP/s. */
 int aec_bench_fp32_peak(int iters, double* tflops, void* cuda_stream);
