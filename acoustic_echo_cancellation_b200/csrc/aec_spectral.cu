@@ -9,6 +9,7 @@
 
 #include "aec_common.cuh"
 #include "fft_warp.cuh"
+#include "stage2_net.cuh"
 
 namespace aec {
 
@@ -18,21 +19,6 @@ constexpr int kTT = 16;        // frames per CTA tile
 constexpr int kThreads = 128;  // 8 half-warps, 2 frames each
 constexpr int kK = 257;
 constexpr int kPitch = kTT + 1;
-
-__device__ __forceinline__ void unpack_pair_s(float2 fa, float2 fb, float2 w, float2& xk, float2& xm) {
-    const float2 a = make_float2(fa.x + fb.x, fa.y - fb.y);
-    const float2 d = make_float2(fa.y + fb.y, fb.x - fa.x);
-    const float2 t = cmul(w, d);
-    xk = make_float2(a.x + t.x, a.y + t.y);
-    xm = make_float2(a.x - t.x, t.y - a.y);
-}
-__device__ __forceinline__ void pack_pair_s(float2 ek, float2 em, float2 w, float2& gk, float2& gm) {
-    const float2 a = make_float2(ek.x + em.x, ek.y - em.y);
-    const float2 d = make_float2(ek.x - em.x, ek.y + em.y);
-    const float2 t = cmulc(d, w);
-    gk = make_float2(a.x - t.y, a.y + t.x);
-    gm = make_float2(a.x + t.y, t.x - a.y);
-}
 
 // Windowed analysis of frame t of one row into the half-warp's tile: tile[k] = Zc[k].
 // `shift` is subtracted from in-range samples only (the zero pad stays zero, as in the
@@ -89,7 +75,7 @@ __global__ void __launch_bounds__(kThreads) stft512_kernel(const float* __restri
             for (int q = 0; q < 8; ++q) {
                 const int k = h + 16 * q;
                 float2 xk, xm;
-                unpack_pair_s(tile[k], tile[(256 - k) & 255], __ldg(&tab.tw512[k]), xk, xm);
+                unpack_pair(tile[k], tile[(256 - k) & 255], __ldg(&tab.tw512[k]), xk, xm);
                 outt[k * kPitch + tt] = xk.x;
                 outt[(kK + k) * kPitch + tt] = (k == 0) ? 0.f : xk.y;
                 outt[(256 - k) * kPitch + tt] = xm.x;
@@ -97,7 +83,7 @@ __global__ void __launch_bounds__(kThreads) stft512_kernel(const float* __restri
             }
             if (h == 0) {
                 float2 xk, xm;
-                unpack_pair_s(tile[128], tile[128], make_float2(0.f, -1.f), xk, xm);
+                unpack_pair(tile[128], tile[128], make_float2(0.f, -1.f), xk, xm);
                 outt[128 * kPitch + tt] = xk.x;
                 outt[(kK + 128) * kPitch + tt] = xk.y;
             }
@@ -142,14 +128,14 @@ __global__ void __launch_bounds__(kThreads) istft512_kernel(const float* __restr
                 em.y = 0.f;
             }
             float2 gk, gm;
-            pack_pair_s(ek, em, __ldg(&tab.tw512[k]), gk, gm);
+            pack_pair(ek, em, __ldg(&tab.tw512[k]), gk, gm);
             tile[k] = gk;
             tile[(256 - k) & 255] = gm;
         }
         if (h == 0) {
             const float2 e = make_float2(inn[128 * kPitch + tt], inn[(kK + 128) * kPitch + tt]);
             float2 gk, gm;
-            pack_pair_s(e, e, make_float2(0.f, -1.f), gk, gm);
+            pack_pair(e, e, make_float2(0.f, -1.f), gk, gm);
             tile[128] = gk;
         }
         __syncwarp();
@@ -204,12 +190,6 @@ constexpr int kFeatMP = 259;   // magnitude row pitch (odd: lanes = frames read 
 // (round 2: the bank is no longer staged densely in shared memory -- 33 KB for 483 non-zeros --; the projection reads
 //  its coefficients through L1 (one broadcast load per bin, ~15 KB of sectors) and the output tile lives in the FFT
 //  tiles, which are dead by then: 51 KB per CTA instead of 88, four CTAs per SM instead of two.)
-__device__ __forceinline__ float sqrt_fast(float x) {
-    float r;
-    asm("sqrt.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x));     // 1 ulp; the arguments are >= 1e-9
-    return r;
-}
-
 __global__ void __launch_bounds__(kThreads, 4) features512_kernel(const float* __restrict__ mic,
                                                                const float* __restrict__ ref,
                                                                const float* __restrict__ erb, float* __restrict__ feat,
@@ -227,17 +207,7 @@ __global__ void __launch_bounds__(kThreads, 4) features512_kernel(const float* _
     const long long b = blockIdx.y;
     const long long n_tiles = (T + kTT - 1) / kTT;
 
-    // non-zero bin range of every band (the cosine bank is ~2 non-zeros per bin)
-    for (int j = tid; j < bands; j += kThreads) {
-        int l = kK, u = 0;
-        for (int k = 0; k < kK; ++k)
-            if (__ldg(erb + k * bands + j) != 0.f) {
-                l = l < k ? l : k;
-                u = k + 1;
-            }
-        lo[j] = l;
-        hi[j] = u;
-    }
+    s2::band_bin_ranges(erb, bands, lo, hi, tid, kThreads);
     const float* xb = (half == 0 ? mic : ref) + b * in_stride;
     // the batch-global scalar of ERB.py:254-255, by value or -- no host round trip -- from aec_batch_shift's output
     const float shift = half == 0 ? (shift_mic_dev ? __ldg(shift_mic_dev) : shift_mic)
@@ -258,18 +228,18 @@ __global__ void __launch_bounds__(kThreads, 4) features512_kernel(const float* _
             for (int q = 0; q < 8; ++q) {
                 const int k = h + 16 * q;
                 float2 xk, xm;
-                unpack_pair_s(tile[k], tile[(256 - k) & 255], __ldg(&tab.tw512[k]), xk, xm);
+                unpack_pair(tile[k], tile[(256 - k) & 255], __ldg(&tab.tw512[k]), xk, xm);
                 if (k == 0) {
                     xk.y = 0.f;
                     xm.y = 0.f;
                 }
-                mrow[k] = sqrt_fast(fmaf(xk.x, xk.x, fmaf(xk.y, xk.y, 1e-9f)));        // ERB.py:277-278
-                mrow[256 - k] = sqrt_fast(fmaf(xm.x, xm.x, fmaf(xm.y, xm.y, 1e-9f)));
+                mrow[k] = sqrt_approx(fmaf(xk.x, xk.x, fmaf(xk.y, xk.y, 1e-9f)));        // ERB.py:277-278
+                mrow[256 - k] = sqrt_approx(fmaf(xm.x, xm.x, fmaf(xm.y, xm.y, 1e-9f)));
             }
             if (h == 0) {
                 float2 xk, xm;
-                unpack_pair_s(tile[128], tile[128], make_float2(0.f, -1.f), xk, xm);
-                mrow[128] = sqrt_fast(fmaf(xk.x, xk.x, fmaf(xk.y, xk.y, 1e-9f)));
+                unpack_pair(tile[128], tile[128], make_float2(0.f, -1.f), xk, xm);
+                mrow[128] = sqrt_approx(fmaf(xk.x, xk.x, fmaf(xk.y, xk.y, 1e-9f)));
             }
             __syncwarp();
         }
@@ -348,7 +318,7 @@ __global__ void __launch_bounds__(kThreads) stft1024_kernel(const float* __restr
         for (int q = 0; q < 8; ++q) {
             const int k = lane + 32 * q;
             float2 xk, xm;
-            unpack_pair_s(tile[k], tile[(512 - k) & 511], __ldg(&tab.tw1024[k]), xk, xm);
+            unpack_pair(tile[k], tile[(512 - k) & 511], __ldg(&tab.tw1024[k]), xk, xm);
             outt[k * kPitch + tt] = xk.x;
             outt[(kK1k + k) * kPitch + tt] = (k == 0) ? 0.f : xk.y;
             outt[(512 - k) * kPitch + tt] = xm.x;
@@ -356,7 +326,7 @@ __global__ void __launch_bounds__(kThreads) stft1024_kernel(const float* __restr
         }
         if (lane == 0) {
             float2 xk, xm;
-            unpack_pair_s(tile[256], tile[256], make_float2(0.f, -1.f), xk, xm);
+            unpack_pair(tile[256], tile[256], make_float2(0.f, -1.f), xk, xm);
             outt[256 * kPitch + tt] = xk.x;
             outt[(kK1k + 256) * kPitch + tt] = xk.y;
         }
@@ -398,14 +368,14 @@ __global__ void __launch_bounds__(kThreads) istft1024_kernel(const float* __rest
                 em.y = 0.f;
             }
             float2 gk, gm;
-            pack_pair_s(ek, em, __ldg(&tab.tw1024[k]), gk, gm);
+            pack_pair(ek, em, __ldg(&tab.tw1024[k]), gk, gm);
             tile[k] = gk;
             tile[(512 - k) & 511] = gm;
         }
         if (lane == 0) {
             const float2 e = make_float2(inn[256 * kPitch + tt], inn[(kK1k + 256) * kPitch + tt]);
             float2 gk, gm;
-            pack_pair_s(e, e, make_float2(0.f, -1.f), gk, gm);
+            pack_pair(e, e, make_float2(0.f, -1.f), gk, gm);
             tile[256] = gk;
         }
         __syncwarp();

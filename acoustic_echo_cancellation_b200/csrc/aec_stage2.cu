@@ -9,32 +9,18 @@
 
 #include "aec_common.cuh"
 #include "fft_warp.cuh"
+#include "stage2_net.cuh"
 
 namespace aec {
 namespace {
 
-constexpr int kH = 32;          // hidden units == ERB bands (Little_net: GRU(2*bands -> bands))
-constexpr int kIn = 64;         // 2 * bands
+using namespace s2;
+
 // utterances (= warps) per CTA: 4 for large batches (the 45 KB of weights are staged once per CTA), 1 for batches that would
 // otherwise leave SMs empty -- the recurrence streams ~400 shared-memory wavefronts per utterance per frame, and four
 // utterances on one SM pay them one after the other while other SMs sit idle
 
-// gate non-linearities on the frame-to-frame chain of the recurrence: MUFU.EX2 + MUFU.RCP forms (a few ulp; the pinned
-// tolerance of the inference is 2e-4 relative) instead of the IEEE division and the branchy tanhf -- each of the three
-// sits on the critical path of every time step
-__device__ __forceinline__ float sigmoidf_(float v) { return __fdividef(1.f, 1.f + __expf(-v)); }
-__device__ __forceinline__ float tanhf_(float v) { return 1.f - __fdividef(2.f, __expf(2.f * v) + 1.f); }
-
-// One warp per utterance, lane j = hidden unit / band j, CH = 8 frames per chunk (round 2: only what depends on h stays
-// on the frame-to-frame chain):
-//   phase 1  W_ih x_t + b for the chunk's 8 frames at once -- no dependence on h, 24 independent accumulators per lane,
-//            every weight load (float4 groups of four inputs per unit, staged transposed in shared memory) used 8 times;
-//   phase 2  the recurrence proper: W_hh h_{t-1} with lane j's three rows of W_hh held in REGISTERS (96 floats), the hidden
-//            state broadcast through 32 floats of shared memory (8 x LDS.128), gates, h_t -> per-chunk buffer;
-//   phase 3  Linear(64->32)+ReLU on cat[h_t, mic_erb_t] and Linear(32->32)+sigmoid for the 8 frames at once, mask * mic_erb.
-// Before, every step ran all 18.4 k multiply-adds of the three layers (and ~400 shared-memory wavefronts of weights) as one
-// dependent chain on a single warp: ~3 400 cycles per frame; the chain is now ~1/6 of that.
-constexpr int kCh = 8;
+// One warp per utterance, lane j = hidden unit / band j, the frames in chunks of kCh (stage2_net.cuh).
 constexpr int kScratch = kCh * kIn + 2 * kCh * kH + kH;   // floats per warp: xs[8][64] + hb[8][32] + os[8][32] + hs[32]
 
 template <int kMaskWarps>
@@ -42,34 +28,9 @@ __global__ void __launch_bounds__(kMaskWarps * 32) stage2_mask_kernel(const floa
                                                                       aec_stage2_weights w, float* __restrict__ est,
                                                                       long long B, long long T) {
     extern __shared__ __align__(16) float sm[];
-    float* wih = sm;                       // [3][16][32][4]
-    float* w1 = wih + kIn * 96;            // [16][32][4]
-    float* w2 = w1 + kIn * kH;             // [8][32][4]
-    float* bias = w2 + kH * kH;            // b_ih[96] b_hh[96] b1[32] b2[32]
-    float* scratch = bias + 256;           // per warp: kScratch floats
+    float* scratch = sm + kWFloats;        // per warp: kScratch floats
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    // weights as float4 groups of four consecutive inputs per (gate, unit): one 16-byte load feeds four FFMAs
-    //   wih : [gate 3][input/4 16][unit 32][4]     w1 : [input/4 16][unit 32][4]     w2 : [input/4 8][unit 32][4]
-    for (int i = tid; i < 96 * kIn; i += blockDim.x) {
-        const int row = i / kIn, col = i % kIn, g = row >> 5, j = row & 31;
-        wih[(((g * (kIn / 4) + (col >> 2)) * 32 + j) << 2) + (col & 3)] = __ldg(w.gru_w_ih + i);
-    }
-    for (int i = tid; i < kH * kIn; i += blockDim.x) {
-        const int j = i / kIn, col = i % kIn;
-        w1[((((col >> 2)) * 32 + j) << 2) + (col & 3)] = __ldg(w.lin1_w + i);
-    }
-    for (int i = tid; i < kH * kH; i += blockDim.x) {
-        const int j = i / kH, col = i % kH;
-        w2[((((col >> 2)) * 32 + j) << 2) + (col & 3)] = __ldg(w.lin2_w + i);
-    }
-    for (int i = tid; i < 96; i += blockDim.x) {
-        bias[i] = __ldg(w.gru_b_ih + i);
-        bias[96 + i] = __ldg(w.gru_b_hh + i);
-    }
-    for (int i = tid; i < kH; i += blockDim.x) {
-        bias[192 + i] = __ldg(w.lin1_b + i);
-        bias[224 + i] = __ldg(w.lin2_b + i);
-    }
+    stage_weights(sm, w, tid, blockDim.x);
     __syncthreads();
     const long long b = (long long)blockIdx.x * kMaskWarps + warp;
     if (b >= B) return;
@@ -79,21 +40,7 @@ __global__ void __launch_bounds__(kMaskWarps * 32) stage2_mask_kernel(const floa
     float* hs = os + kCh * kH;                       // [32]      h_{t-1}, broadcast buffer of the recurrence
     const float* fb = feat + b * T * kIn;
     float* eb = est + b * T * kH;
-    const float b_r = bias[lane] + bias[96 + lane], b_z = bias[32 + lane] + bias[128 + lane];
-    const float b_in = bias[64 + lane], b_hn = bias[160 + lane];
-    const float b_1 = bias[192 + lane], b_2 = bias[224 + lane];
-    // lane j's rows of W_hh (gate order r, z, n), resident in registers for the whole utterance
-    float whr[kH], whz[kH], whn[kH];
-#pragma unroll
-    for (int i = 0; i < kH; ++i) {
-        whr[i] = __ldg(w.gru_w_hh + (0 * kH + lane) * kH + i);
-        whz[i] = __ldg(w.gru_w_hh + (1 * kH + lane) * kH + i);
-        whn[i] = __ldg(w.gru_w_hh + (2 * kH + lane) * kH + i);
-    }
-    const float4* wih4 = reinterpret_cast<const float4*>(wih) + lane;
-    const float4* w14 = reinterpret_cast<const float4*>(w1) + lane;
-    const float4* w24 = reinterpret_cast<const float4*>(w2) + lane;
-    const float4* hs4 = reinterpret_cast<const float4*>(hs);
+    const NetLane net = NetLane::load(sm, w, lane);
     float h = 0.f;
     for (long long t0 = 0; t0 < T; t0 += kCh) {
         const int nf = (int)((T - t0) < kCh ? (T - t0) : kCh);
@@ -105,84 +52,11 @@ __global__ void __launch_bounds__(kMaskWarps * 32) stage2_mask_kernel(const floa
             xs[f * kIn + col] = (f < nf) ? __ldg(fb + (t0 + f) * kIn + col) : 0.f;
         }
         __syncwarp();
-        // ---- phase 1: input projections of the chunk ----
-        float gr[kCh], gz[kCh], gn[kCh];
-#pragma unroll
-        for (int f = 0; f < kCh; ++f) {
-            gr[f] = b_r;
-            gz[f] = b_z;
-            gn[f] = b_in;
-        }
-#pragma unroll 2
-        for (int i4 = 0; i4 < kIn / 4; ++i4) {
-            const float4 wr = wih4[(0 * (kIn / 4) + i4) * 32], wz = wih4[(1 * (kIn / 4) + i4) * 32], wn = wih4[(2 * (kIn / 4) + i4) * 32];
-#pragma unroll
-            for (int f = 0; f < kCh; ++f) {
-                const float4 xv = *reinterpret_cast<const float4*>(xs + f * kIn + 4 * i4);
-                gr[f] = fmaf(wr.w, xv.w, fmaf(wr.z, xv.z, fmaf(wr.y, xv.y, fmaf(wr.x, xv.x, gr[f]))));
-                gz[f] = fmaf(wz.w, xv.w, fmaf(wz.z, xv.z, fmaf(wz.y, xv.y, fmaf(wz.x, xv.x, gz[f]))));
-                gn[f] = fmaf(wn.w, xv.w, fmaf(wn.z, xv.z, fmaf(wn.y, xv.y, fmaf(wn.x, xv.x, gn[f]))));
-            }
-        }
-        // ---- phase 2: the recurrence (the only serial part) ----
-#pragma unroll
-        for (int f = 0; f < kCh; ++f) {
-            if (f < nf) {
-                hs[lane] = h;
-                __syncwarp();
-                // four partial sums per gate: twelve independent chains of eight FFMAs
-                float ar[4] = {0.f, 0.f, 0.f, 0.f}, az[4] = {0.f, 0.f, 0.f, 0.f}, an[4] = {b_hn, 0.f, 0.f, 0.f};
-#pragma unroll
-                for (int i4 = 0; i4 < kH / 4; ++i4) {
-                    const float4 hv = hs4[i4];
-                    ar[0] = fmaf(whr[4 * i4 + 0], hv.x, ar[0]); ar[1] = fmaf(whr[4 * i4 + 1], hv.y, ar[1]);
-                    ar[2] = fmaf(whr[4 * i4 + 2], hv.z, ar[2]); ar[3] = fmaf(whr[4 * i4 + 3], hv.w, ar[3]);
-                    az[0] = fmaf(whz[4 * i4 + 0], hv.x, az[0]); az[1] = fmaf(whz[4 * i4 + 1], hv.y, az[1]);
-                    az[2] = fmaf(whz[4 * i4 + 2], hv.z, az[2]); az[3] = fmaf(whz[4 * i4 + 3], hv.w, az[3]);
-                    an[0] = fmaf(whn[4 * i4 + 0], hv.x, an[0]); an[1] = fmaf(whn[4 * i4 + 1], hv.y, an[1]);
-                    an[2] = fmaf(whn[4 * i4 + 2], hv.z, an[2]); an[3] = fmaf(whn[4 * i4 + 3], hv.w, an[3]);
-                }
-                const float r = sigmoidf_(gr[f] + ((ar[0] + ar[1]) + (ar[2] + ar[3])));
-                const float z = sigmoidf_(gz[f] + ((az[0] + az[1]) + (az[2] + az[3])));
-                const float n = tanhf_(fmaf(r, (an[0] + an[1]) + (an[2] + an[3]), gn[f]));
-                h = fmaf(z, h - n, n);                   // (1 - z) n + z h
-                hb[f * kH + lane] = h;
-                __syncwarp();                            // every lane has read hs before the next step overwrites it
-            } else {
-                hb[f * kH + lane] = 0.f;
-            }
-        }
+        float gr[kCh], gz[kCh], gn[kCh], a1[kCh], a2[kCh];
+        gru_inputs(net, sm, xs, lane, gr, gz, gn);
+        gru_chunk(net, gr, gz, gn, hs, hb, h, nf, lane);
         __syncwarp();
-        // ---- phase 3: linear1 on cat[h, mic_erb] + ReLU, linear2 + sigmoid, mask * mic_erb (ERB.py:295-304) ----
-        float a1[kCh];
-#pragma unroll
-        for (int f = 0; f < kCh; ++f) a1[f] = b_1;
-#pragma unroll 2
-        for (int i4 = 0; i4 < kH / 4; ++i4) {
-            const float4 wa = w14[i4 * 32], wb = w14[(kH / 4 + i4) * 32];      // inputs 0..31 = h, 32..63 = mic_erb
-#pragma unroll
-            for (int f = 0; f < kCh; ++f) {
-                const float4 hv = *reinterpret_cast<const float4*>(hb + f * kH + 4 * i4);
-                const float4 xv = *reinterpret_cast<const float4*>(xs + f * kIn + 4 * i4);
-                a1[f] = fmaf(wa.w, hv.w, fmaf(wa.z, hv.z, fmaf(wa.y, hv.y, fmaf(wa.x, hv.x, a1[f]))));
-                a1[f] = fmaf(wb.w, xv.w, fmaf(wb.z, xv.z, fmaf(wb.y, xv.y, fmaf(wb.x, xv.x, a1[f]))));
-            }
-        }
-#pragma unroll
-        for (int f = 0; f < kCh; ++f) os[f * kH + lane] = fmaxf(a1[f], 0.f);
-        __syncwarp();
-        float a2[kCh];
-#pragma unroll
-        for (int f = 0; f < kCh; ++f) a2[f] = b_2;
-#pragma unroll 2
-        for (int i4 = 0; i4 < kH / 4; ++i4) {
-            const float4 wv = w24[i4 * 32];
-#pragma unroll
-            for (int f = 0; f < kCh; ++f) {
-                const float4 ov = *reinterpret_cast<const float4*>(os + f * kH + 4 * i4);
-                a2[f] = fmaf(wv.w, ov.w, fmaf(wv.z, ov.z, fmaf(wv.y, ov.y, fmaf(wv.x, ov.x, a2[f]))));
-            }
-        }
+        net_outputs(net, sm, xs, hb, os, lane, a1, a2);
 #pragma unroll
         for (int f = 0; f < kCh; ++f)
             if (f < nf) eb[(t0 + f) * kH + lane] = sigmoidf_(a2[f]) * xs[f * kIn + lane];   // est_erb = mask * mic_erb
@@ -190,23 +64,8 @@ __global__ void __launch_bounds__(kMaskWarps * 32) stage2_mask_kernel(const floa
 }
 
 // ---- synthesis: out = iSTFT((est_erb @ erb^T) * STFT(mic - shift)) + 1e-9 -------------------
-constexpr int kTT = 16, kThreads = 128, kK = 257, kPitch = kTT + 1;
+constexpr int kTT = 16, kThreads = 128;
 static_assert(((8 * kTilePitch + kTT * 256) * 8 + kTT * kH * 4 + 2 * kK * 4) % 8 == 0, "coefficient pairs must be 8-byte aligned");
-
-__device__ __forceinline__ void unpack_pair_2(float2 fa, float2 fb, float2 w, float2& xk, float2& xm) {
-    const float2 a = make_float2(fa.x + fb.x, fa.y - fb.y);
-    const float2 d = make_float2(fa.y + fb.y, fb.x - fa.x);
-    const float2 t = cmul(w, d);
-    xk = make_float2(a.x + t.x, a.y + t.y);
-    xm = make_float2(a.x - t.x, t.y - a.y);
-}
-__device__ __forceinline__ void pack_pair_2(float2 ek, float2 em, float2 w, float2& gk, float2& gm) {
-    const float2 a = make_float2(ek.x + em.x, ek.y - em.y);
-    const float2 d = make_float2(ek.x - em.x, ek.y + em.y);
-    const float2 t = cmulc(d, w);
-    gk = make_float2(a.x - t.y, a.y + t.x);
-    gm = make_float2(a.x + t.y, t.x - a.y);
-}
 
 // (round 2: the dense bank is no longer staged in shared memory -- 33 KB per CTA for ~2 non-zeros per bin, re-staged by
 //  every CTA for a single 15-hop tile --; a CTA now walks several tiles, reads the two or three coefficients of a bin
@@ -227,30 +86,11 @@ __global__ void __launch_bounds__(kThreads, 4) stage2_synth_kernel(const float* 
     const int tid = threadIdx.x, lane = tid & 31, hw = tid >> 4, h = lane & 15;
     const long long b = blockIdx.y;
     const float shift = shift_dev ? __ldg(shift_dev) : shift_val;      // ERB.py:254, by value or from aec_batch_shift
-    for (int k = tid; k < kK; k += kThreads) {     // non-zero band range of bin k (the bank is <= 2 bands per bin)
-        int lo = kH, hi = 0;
-        for (int j = 0; j < kH; ++j)
-            if (__ldg(erb + k * kH + j) != 0.f) {
-                lo = min(lo, j);
-                hi = j + 1;
-            }
-        blo[k] = lo < kH ? lo : 0;
-        bhi[k] = hi > lo ? hi : blo[k];
-        // the first two coefficients of the range stay in shared memory (all of them, for the reference's bank)
-        c2[k] = make_float2(lo < hi ? __ldg(erb + k * kH + lo) : 0.f, lo + 1 < hi ? __ldg(erb + k * kH + lo + 1) : 0.f);
-    }
+    const BinBands bank{blo, bhi, c2, erb};
+    bank.stage(tid, kThreads);
     const float* xb = mic + b * in_stride;
     float* yb = y + b * out_stride;
     float2* tile = tiles + hw * kTilePitch;
-    auto gain = [&](int tt, int k) {               // ERB.py:306-307: (mask * mic_erb) @ erb^T
-        const int lo = blo[k], hi = bhi[k];
-        const float2 c = c2[k];
-        const float* e = es + tt * kH + lo;
-        float g = fmaf(e[0], c.x, 0.f);
-        g = fmaf(e[lo + 1 < kH ? 1 : 0], c.y, g);   // (c.y is zero when the range has one band)
-        for (int j = lo + 2; j < hi; ++j) g = fmaf(es[tt * kH + j], __ldg(erb + k * kH + j), g);   // wider banks only
-        return g;
-    };
     const long long n_tiles = (T - 1 + kTT - 2) / (kTT - 1);
     for (long long tile_i = blockIdx.x; tile_i < n_tiles; tile_i += gridDim.x) {
         const long long g0 = tile_i * (kTT - 1);
@@ -294,34 +134,9 @@ __global__ void __launch_bounds__(kThreads, 4) stage2_synth_kernel(const float* 
                 for (int p = 0; p < 16; ++p) tile[h + 16 * fft16_index(p)] = v[p];
                 __syncwarp();
             }
-            // ---- per-bin gain, repack for the inverse transform (in place) ----
-#pragma unroll
-            for (int q = 0; q < 8; ++q) {
-                const int k = h + 16 * q, km = (256 - k) & 255;
-                const float2 wk = __ldg(&tab.tw512[k]);
-                float2 xk, xm, gk, gm;
-                unpack_pair_2(tile[k], tile[km], wk, xk, xm);
-                const float ga = gain(tt, k), gb = gain(tt, 256 - k);
-                xk = make_float2(ga * xk.x, k == 0 ? 0.f : ga * xk.y);       // ERB.py:309-310
-                xm = make_float2(gb * xm.x, k == 0 ? 0.f : gb * xm.y);
-                pack_pair_2(xk, xm, wk, gk, gm);
-                tile[k] = gk;
-                tile[km] = gm;
-            }
-            if (h == 0) {
-                float2 xk, xm, gk, gm;
-                unpack_pair_2(tile[128], tile[128], make_float2(0.f, -1.f), xk, xm);
-                const float ga = gain(tt, 128);
-                xk = make_float2(ga * xk.x, ga * xk.y);
-                pack_pair_2(xk, xk, make_float2(0.f, -1.f), gk, gm);
-                tile[128] = gk;
-            }
-            __syncwarp();
+            // ---- per-bin gain, inverse transform, synthesis window ----
             float2 v[16];
-#pragma unroll
-            for (int j = 0; j < 16; ++j) v[j] = tile[h + 16 * j];
-            __syncwarp();
-            fft256_halfwarp<true>(v, tile, tab.tw256, h);
+            synth_frame(tile, bank, es, tt, tab, h, v);
 #pragma unroll
             for (int p = 0; p < 16; ++p) {
                 const int r = fft16_index(p);

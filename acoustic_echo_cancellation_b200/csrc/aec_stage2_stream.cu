@@ -10,21 +10,20 @@
 // of one call over the whole stream.  (Against LittleNetInference(in_norm=False) the outputs agree to ~1e-7 relative, not
 // always bit for bit: this unit is compiled on its own.)
 //
-// Kept copies: sigmoidf_, tanhf_, unpack_pair_2 and pack_pair_2 (aec_stage2.cu), unpack_pair_s and sqrt_fast
-// (aec_spectral.cu) and the bodies of the three phases are restated here rather than moved into a shared header, so that
-// the existing kernels' units are not touched at all.  A change to any of them must be made in both places.
+// What is per frame -- the Little_net arithmetic shared with the one-shot kernels -- is defined once in stage2_net.cuh;
+// this unit holds what streaming adds: the state layout, the persistent per-stream loop, framing from the carried
+// previous hop, the overlap-add with the carried half-frame and the state epilogue.
 #include <cstdint>
 
 #include "aec_common.cuh"
 #include "fft_warp.cuh"
+#include "stage2_net.cuh"
 
 namespace aec {
 namespace {
 
-constexpr int kH = 32;          // hidden units == ERB bands
-constexpr int kIn = 64;         // 2 * bands
-constexpr int kCh = 8;          // frames per chunk of the recurrence (as stage2_mask_kernel)
-constexpr int kK = 257;
+using namespace s2;
+
 constexpr int kHop = 256;
 constexpr int kSW = 4;          // streams (warps) per CTA
 constexpr int kCtasPerSm = 2;   // persistent grid: at most this many CTAs per SM, each walking streams
@@ -42,7 +41,6 @@ static_assert(S2State::kBytes % 16 == 0 && S2State::kMicPrev % 16 == 0 && S2Stat
               S2State::kOla % 16 == 0, "state fields on 16-byte boundaries");
 
 // shared memory, in floats: CTA-wide weights and bank ranges, then one region per warp
-constexpr int kWFloats = kIn * 96 + kIn * kH + kH * kH + 256;            // wih, w1, w2, biases (as stage2_mask_kernel)
 constexpr int kBankFloats = 2 * kK + 2 * kK + 2 * kH;                     // c2 float2[257], blo/bhi[257], lo/hi[32]
 constexpr int kTileF = 2 * 2 * kTilePitch;                                // two half-warp FFT tiles (float2)
 constexpr int kMagP = 260;                                                // magnitude row pitch
@@ -50,29 +48,6 @@ constexpr int kWarpFloats = kTileF + 2 * kMagP + kCh * kIn + 3 * kCh * kH + kH +
 constexpr size_t kSmemBytes = (size_t)(kWFloats + kBankFloats + kSW * kWarpFloats) * sizeof(float);
 static_assert(kWFloats % 4 == 0 && kBankFloats % 4 == 0 && kWarpFloats % 4 == 0 && (kTileF + 2 * kMagP) % 4 == 0,
               "float4 / float2 regions must stay aligned");
-
-__device__ __forceinline__ float sigmoidf_(float v) { return __fdividef(1.f, 1.f + __expf(-v)); }
-__device__ __forceinline__ float tanhf_(float v) { return 1.f - __fdividef(2.f, __expf(2.f * v) + 1.f); }
-
-__device__ __forceinline__ float sqrt_fast(float x) {
-    float r;
-    asm("sqrt.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x));
-    return r;
-}
-__device__ __forceinline__ void unpack_pair_2(float2 fa, float2 fb, float2 w, float2& xk, float2& xm) {
-    const float2 a = make_float2(fa.x + fb.x, fa.y - fb.y);
-    const float2 d = make_float2(fa.y + fb.y, fb.x - fa.x);
-    const float2 t = cmul(w, d);
-    xk = make_float2(a.x + t.x, a.y + t.y);
-    xm = make_float2(a.x - t.x, t.y - a.y);
-}
-__device__ __forceinline__ void pack_pair_2(float2 ek, float2 em, float2 w, float2& gk, float2& gm) {
-    const float2 a = make_float2(ek.x + em.x, ek.y - em.y);
-    const float2 d = make_float2(ek.x - em.x, ek.y + em.y);
-    const float2 t = cmulc(d, w);
-    gk = make_float2(a.x - t.y, a.y + t.x);
-    gm = make_float2(a.x + t.y, t.x - a.y);
-}
 
 // Windowed analysis of one frame into the half-warp's tile (tile[k] = Zc[k]): samples 0..255 from p0 (the previous hop),
 // 256..511 from p1.  `vec`: both pointers 8-byte aligned.
@@ -98,59 +73,17 @@ __global__ void __launch_bounds__(kSW * 32, kCtasPerSm) stage2_stream_kernel(
     float* __restrict__ out, const int64_t* __restrict__ n_samples, long long B, long long L, long long in_stride,
     long long out_stride, unsigned char* __restrict__ state, long long state_stride, Tables tab) {
     extern __shared__ __align__(16) float sm[];
-    float* wih = sm;                       // [3][16][32][4]
-    float* w1 = wih + kIn * 96;            // [16][32][4]
-    float* w2 = w1 + kIn * kH;             // [8][32][4]
-    float* bias = w2 + kH * kH;            // b_ih[96] b_hh[96] b1[32] b2[32]
     float2* c2 = reinterpret_cast<float2*>(sm + kWFloats);        // [257] first two coefficients of bin k's band range
     int* blo = reinterpret_cast<int*>(c2 + kK);                    // [257] band range of bin k
     int* bhi = blo + kK;
     int* lo = bhi + kK;                                            // [32]  bin range of band j
     int* hi = lo + kH;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, half = lane >> 4, h = lane & 15;
-    // ---- weights, once per CTA (the layouts of stage2_mask_kernel) ----
-    for (int i = tid; i < 96 * kIn; i += blockDim.x) {
-        const int row = i / kIn, col = i % kIn, g = row >> 5, j = row & 31;
-        wih[(((g * (kIn / 4) + (col >> 2)) * 32 + j) << 2) + (col & 3)] = __ldg(w.gru_w_ih + i);
-    }
-    for (int i = tid; i < kH * kIn; i += blockDim.x) {
-        const int j = i / kIn, col = i % kIn;
-        w1[((((col >> 2)) * 32 + j) << 2) + (col & 3)] = __ldg(w.lin1_w + i);
-    }
-    for (int i = tid; i < kH * kH; i += blockDim.x) {
-        const int j = i / kH, col = i % kH;
-        w2[((((col >> 2)) * 32 + j) << 2) + (col & 3)] = __ldg(w.lin2_w + i);
-    }
-    for (int i = tid; i < 96; i += blockDim.x) {
-        bias[i] = __ldg(w.gru_b_ih + i);
-        bias[96 + i] = __ldg(w.gru_b_hh + i);
-    }
-    for (int i = tid; i < kH; i += blockDim.x) {
-        bias[192 + i] = __ldg(w.lin1_b + i);
-        bias[224 + i] = __ldg(w.lin2_b + i);
-    }
-    // ---- bank ranges: per bin (stage2_synth_kernel) and per band (features512_kernel) ----
-    for (int k = tid; k < kK; k += blockDim.x) {
-        int l = kH, u = 0;
-        for (int j = 0; j < kH; ++j)
-            if (__ldg(erb + k * kH + j) != 0.f) {
-                l = min(l, j);
-                u = j + 1;
-            }
-        blo[k] = l < kH ? l : 0;
-        bhi[k] = u > l ? u : blo[k];
-        c2[k] = make_float2(l < u ? __ldg(erb + k * kH + l) : 0.f, l + 1 < u ? __ldg(erb + k * kH + l + 1) : 0.f);
-    }
-    for (int j = tid; j < kH; j += blockDim.x) {
-        int l = kK, u = 0;
-        for (int k = 0; k < kK; ++k)
-            if (__ldg(erb + k * kH + j) != 0.f) {
-                l = l < k ? l : k;
-                u = k + 1;
-            }
-        lo[j] = l;
-        hi[j] = u;
-    }
+    // ---- weights and bank ranges, once per CTA ----
+    stage_weights(sm, w, tid, blockDim.x);
+    const BinBands bank{blo, bhi, c2, erb};
+    bank.stage(tid, blockDim.x);
+    band_bin_ranges(erb, kH, lo, hi, tid, blockDim.x);
     __syncthreads();
 
     float* wreg = sm + kWFloats + kBankFloats + warp * kWarpFloats;
@@ -163,30 +96,7 @@ __global__ void __launch_bounds__(kSW * 32, kCtasPerSm) stage2_stream_kernel(
     float* es = os + kCh * kH;                                     // [kCh][32]   est_erb of the chunk
     float* hs = es + kCh * kH;                                     // [32]        h_{t-1} broadcast buffer
     float* ola = hs + kH;                                          // [256]       pending second half-frame
-    const float b_r = bias[lane] + bias[96 + lane], b_z = bias[32 + lane] + bias[128 + lane];
-    const float b_in = bias[64 + lane], b_hn = bias[160 + lane];
-    const float b_1 = bias[192 + lane], b_2 = bias[224 + lane];
-    float whr[kH], whz[kH], whn[kH];       // lane j's rows of W_hh, in registers for the warp's whole life
-#pragma unroll
-    for (int i = 0; i < kH; ++i) {
-        whr[i] = __ldg(w.gru_w_hh + (0 * kH + lane) * kH + i);
-        whz[i] = __ldg(w.gru_w_hh + (1 * kH + lane) * kH + i);
-        whn[i] = __ldg(w.gru_w_hh + (2 * kH + lane) * kH + i);
-    }
-    const float4* wih4 = reinterpret_cast<const float4*>(wih) + lane;
-    const float4* w14 = reinterpret_cast<const float4*>(w1) + lane;
-    const float4* w24 = reinterpret_cast<const float4*>(w2) + lane;
-    const float4* hs4 = reinterpret_cast<const float4*>(hs);
-    // ERB.py:306-307 for frame ff of the chunk: (mask * mic_erb) @ erb^T at bin k
-    auto gain = [&](int ff, int k) {
-        const int l = blo[k], u = bhi[k];
-        const float2 c = c2[k];
-        const float* e = es + ff * kH + l;
-        float g = fmaf(e[0], c.x, 0.f);
-        g = fmaf(e[l + 1 < kH ? 1 : 0], c.y, g);
-        for (int j = l + 2; j < u; ++j) g = fmaf(es[ff * kH + j], __ldg(erb + k * kH + j), g);
-        return g;
-    };
+    const NetLane net = NetLane::load(sm, w, lane);
 
     for (long long b = (long long)blockIdx.x * kSW + warp; b < B; b += (long long)gridDim.x * kSW) {
         long long n = n_samples ? n_samples[b] : L;
@@ -222,18 +132,18 @@ __global__ void __launch_bounds__(kSW * 32, kCtasPerSm) stage2_stream_kernel(
                         for (int q = 0; q < 8; ++q) {
                             const int k = h + 16 * q;
                             float2 xk, xm2;
-                            unpack_pair_2(tile[k], tile[(256 - k) & 255], __ldg(&tab.tw512[k]), xk, xm2);
+                            unpack_pair(tile[k], tile[(256 - k) & 255], __ldg(&tab.tw512[k]), xk, xm2);
                             if (k == 0) {
                                 xk.y = 0.f;
                                 xm2.y = 0.f;
                             }
-                            mrow[k] = sqrt_fast(fmaf(xk.x, xk.x, fmaf(xk.y, xk.y, 1e-9f)));        // ERB.py:277-278
-                            mrow[256 - k] = sqrt_fast(fmaf(xm2.x, xm2.x, fmaf(xm2.y, xm2.y, 1e-9f)));
+                            mrow[k] = sqrt_approx(fmaf(xk.x, xk.x, fmaf(xk.y, xk.y, 1e-9f)));        // ERB.py:277-278
+                            mrow[256 - k] = sqrt_approx(fmaf(xm2.x, xm2.x, fmaf(xm2.y, xm2.y, 1e-9f)));
                         }
                         if (h == 0) {
                             float2 xk, xm2;
-                            unpack_pair_2(tile[128], tile[128], make_float2(0.f, -1.f), xk, xm2);
-                            mrow[128] = sqrt_fast(fmaf(xk.x, xk.x, fmaf(xk.y, xk.y, 1e-9f)));
+                            unpack_pair(tile[128], tile[128], make_float2(0.f, -1.f), xk, xm2);
+                            mrow[128] = sqrt_approx(fmaf(xk.x, xk.x, fmaf(xk.y, xk.y, 1e-9f)));
                         }
                         __syncwarp();
                         // ERB projection, lane = band (ERB.py:282-283), then cat[mic_erb, |mic_erb - ref_erb|]
@@ -252,84 +162,12 @@ __global__ void __launch_bounds__(kSW * 32, kCtasPerSm) stage2_stream_kernel(
                     }
                 }
                 __syncwarp();
-                // ---- phase 1: input projections of the chunk (stage2_mask_kernel) ----
-                float gr[kCh], gz[kCh], gn[kCh];
-#pragma unroll
-                for (int f = 0; f < kCh; ++f) {
-                    gr[f] = b_r;
-                    gz[f] = b_z;
-                    gn[f] = b_in;
-                }
-#pragma unroll 2
-                for (int i4 = 0; i4 < kIn / 4; ++i4) {
-                    const float4 wr = wih4[(0 * (kIn / 4) + i4) * 32], wz = wih4[(1 * (kIn / 4) + i4) * 32],
-                                 wn = wih4[(2 * (kIn / 4) + i4) * 32];
-#pragma unroll
-                    for (int f = 0; f < kCh; ++f) {
-                        const float4 xv = *reinterpret_cast<const float4*>(xs + f * kIn + 4 * i4);
-                        gr[f] = fmaf(wr.w, xv.w, fmaf(wr.z, xv.z, fmaf(wr.y, xv.y, fmaf(wr.x, xv.x, gr[f]))));
-                        gz[f] = fmaf(wz.w, xv.w, fmaf(wz.z, xv.z, fmaf(wz.y, xv.y, fmaf(wz.x, xv.x, gz[f]))));
-                        gn[f] = fmaf(wn.w, xv.w, fmaf(wn.z, xv.z, fmaf(wn.y, xv.y, fmaf(wn.x, xv.x, gn[f]))));
-                    }
-                }
-                // ---- phase 2: the recurrence ----
-#pragma unroll
-                for (int f = 0; f < kCh; ++f) {
-                    if (f < nf) {
-                        hs[lane] = hcur;
-                        __syncwarp();
-                        float ar[4] = {0.f, 0.f, 0.f, 0.f}, az[4] = {0.f, 0.f, 0.f, 0.f}, an[4] = {b_hn, 0.f, 0.f, 0.f};
-#pragma unroll
-                        for (int i4 = 0; i4 < kH / 4; ++i4) {
-                            const float4 hv = hs4[i4];
-                            ar[0] = fmaf(whr[4 * i4 + 0], hv.x, ar[0]); ar[1] = fmaf(whr[4 * i4 + 1], hv.y, ar[1]);
-                            ar[2] = fmaf(whr[4 * i4 + 2], hv.z, ar[2]); ar[3] = fmaf(whr[4 * i4 + 3], hv.w, ar[3]);
-                            az[0] = fmaf(whz[4 * i4 + 0], hv.x, az[0]); az[1] = fmaf(whz[4 * i4 + 1], hv.y, az[1]);
-                            az[2] = fmaf(whz[4 * i4 + 2], hv.z, az[2]); az[3] = fmaf(whz[4 * i4 + 3], hv.w, az[3]);
-                            an[0] = fmaf(whn[4 * i4 + 0], hv.x, an[0]); an[1] = fmaf(whn[4 * i4 + 1], hv.y, an[1]);
-                            an[2] = fmaf(whn[4 * i4 + 2], hv.z, an[2]); an[3] = fmaf(whn[4 * i4 + 3], hv.w, an[3]);
-                        }
-                        const float r = sigmoidf_(gr[f] + ((ar[0] + ar[1]) + (ar[2] + ar[3])));
-                        const float z = sigmoidf_(gz[f] + ((az[0] + az[1]) + (az[2] + az[3])));
-                        const float nn = tanhf_(fmaf(r, (an[0] + an[1]) + (an[2] + an[3]), gn[f]));
-                        hcur = fmaf(z, hcur - nn, nn);
-                        hb[f * kH + lane] = hcur;
-                        __syncwarp();
-                    } else {
-                        hb[f * kH + lane] = 0.f;
-                    }
-                }
+                // ---- the GRU and linear layers of the chunk ----
+                float gr[kCh], gz[kCh], gn[kCh], a1[kCh], a2[kCh];
+                gru_inputs(net, sm, xs, lane, gr, gz, gn);
+                gru_chunk(net, gr, gz, gn, hs, hb, hcur, nf, lane);
                 __syncwarp();
-                // ---- phase 3: linear1 + ReLU, linear2 + sigmoid, est_erb = mask * mic_erb ----
-                float a1[kCh];
-#pragma unroll
-                for (int f = 0; f < kCh; ++f) a1[f] = b_1;
-#pragma unroll 2
-                for (int i4 = 0; i4 < kH / 4; ++i4) {
-                    const float4 wa = w14[i4 * 32], wb = w14[(kH / 4 + i4) * 32];
-#pragma unroll
-                    for (int f = 0; f < kCh; ++f) {
-                        const float4 hv = *reinterpret_cast<const float4*>(hb + f * kH + 4 * i4);
-                        const float4 xv = *reinterpret_cast<const float4*>(xs + f * kIn + 4 * i4);
-                        a1[f] = fmaf(wa.w, hv.w, fmaf(wa.z, hv.z, fmaf(wa.y, hv.y, fmaf(wa.x, hv.x, a1[f]))));
-                        a1[f] = fmaf(wb.w, xv.w, fmaf(wb.z, xv.z, fmaf(wb.y, xv.y, fmaf(wb.x, xv.x, a1[f]))));
-                    }
-                }
-#pragma unroll
-                for (int f = 0; f < kCh; ++f) os[f * kH + lane] = fmaxf(a1[f], 0.f);
-                __syncwarp();
-                float a2[kCh];
-#pragma unroll
-                for (int f = 0; f < kCh; ++f) a2[f] = b_2;
-#pragma unroll 2
-                for (int i4 = 0; i4 < kH / 4; ++i4) {
-                    const float4 wv = w24[i4 * 32];
-#pragma unroll
-                    for (int f = 0; f < kCh; ++f) {
-                        const float4 ov = *reinterpret_cast<const float4*>(os + f * kH + 4 * i4);
-                        a2[f] = fmaf(wv.w, ov.w, fmaf(wv.z, ov.z, fmaf(wv.y, ov.y, fmaf(wv.x, ov.x, a2[f]))));
-                    }
-                }
+                net_outputs(net, sm, xs, hb, os, lane, a1, a2);
 #pragma unroll
                 for (int f = 0; f < kCh; ++f) es[f * kH + lane] = sigmoidf_(a2[f]) * xs[f * kIn + lane];
                 __syncwarp();
@@ -338,33 +176,8 @@ __global__ void __launch_bounds__(kSW * 32, kCtasPerSm) stage2_stream_kernel(
                     const int ff = (f + half < nf) ? f + half : f;         // an odd last pair: both halves on frame f
                     const long long i = f0 + ff;
                     analyse_hops(i == 0 ? st_mp : xm + (i - 1) * kHop, xm + i * kHop, vec, tile, tab, h);
-#pragma unroll
-                    for (int q = 0; q < 8; ++q) {
-                        const int k = h + 16 * q, km = (256 - k) & 255;
-                        const float2 wk = __ldg(&tab.tw512[k]);
-                        float2 xk, xm2, gk, gm;
-                        unpack_pair_2(tile[k], tile[km], wk, xk, xm2);
-                        const float ga = gain(ff, k), gb = gain(ff, 256 - k);
-                        xk = make_float2(ga * xk.x, k == 0 ? 0.f : ga * xk.y);       // ERB.py:309-310
-                        xm2 = make_float2(gb * xm2.x, k == 0 ? 0.f : gb * xm2.y);
-                        pack_pair_2(xk, xm2, wk, gk, gm);
-                        tile[k] = gk;
-                        tile[km] = gm;
-                    }
-                    if (h == 0) {
-                        float2 xk, xm2, gk, gm;
-                        unpack_pair_2(tile[128], tile[128], make_float2(0.f, -1.f), xk, xm2);
-                        const float ga = gain(ff, 128);
-                        xk = make_float2(ga * xk.x, ga * xk.y);
-                        pack_pair_2(xk, xk, make_float2(0.f, -1.f), gk, gm);
-                        tile[128] = gk;
-                    }
-                    __syncwarp();
                     float2 v[16];
-#pragma unroll
-                    for (int j = 0; j < 16; ++j) v[j] = tile[h + 16 * j];
-                    __syncwarp();
-                    fft256_halfwarp<true>(v, tile, tab.tw256, h);
+                    synth_frame(tile, bank, es, ff, tab, h, v);
                     __syncwarp();
 #pragma unroll
                     for (int p = 0; p < 16; ++p) {

@@ -38,6 +38,33 @@ __device__ __forceinline__ float2 cfmac(float2 a, float2 b, float2 acc) {
     return make_float2(fmaf(a.y, b.y, fmaf(a.x, b.x, acc.x)), fmaf(-a.y, b.x, fmaf(a.x, b.y, acc.y)));
 }
 
+// MUFU.SQRT (1 ulp) for spectral magnitudes sqrt(re^2 + im^2 + 1e-9): the arguments are >= 1e-9
+__device__ __forceinline__ float sqrt_approx(float x) {
+    float r;
+    asm("sqrt.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x));
+    return r;
+}
+
+// Real-FFT split and packing, written for frame 512 (the frame-1024 kernels pass 512 - k and exp(-2 pi i k/1024)).
+// half-size spectra -> the two real-signal bins of the mirrored pair (k, 256-k).
+// fa = Zc[k], fb = Zc[256-k], w = exp(-2 pi i k/512).  The analysis window carries the 1/2.
+__device__ __forceinline__ void unpack_pair(float2 fa, float2 fb, float2 w, float2& xk, float2& xm) {
+    const float2 a = make_float2(fa.x + fb.x, fa.y - fb.y);          // Zc[k] + conj Zc[256-k]
+    const float2 d = make_float2(fa.y + fb.y, fb.x - fa.x);          // (Zc[k] - conj Zc[256-k]) / i
+    const float2 t = cmul(w, d);
+    xk = make_float2(a.x + t.x, a.y + t.y);
+    xm = make_float2(a.x - t.x, t.y - a.y);                          // conj(a - t)
+}
+// two real-signal bins (k, 256-k) -> half-size inverse spectrum entries G[k], G[256-k]
+// (scale 1/512 lives in the synthesis table).
+__device__ __forceinline__ void pack_pair(float2 ek, float2 em, float2 w, float2& gk, float2& gm) {
+    const float2 a = make_float2(ek.x + em.x, ek.y - em.y);          // E[k] + conj E[256-k]
+    const float2 d = make_float2(ek.x - em.x, ek.y + em.y);          // E[k] - conj E[256-k]
+    const float2 t = cmulc(d, w);                                    // d * conj(w)
+    gk = make_float2(a.x - t.y, a.y + t.x);
+    gm = make_float2(a.x + t.y, t.x - a.y);
+}
+
 // 4-point DFT in place.  INV=false: e^{-2 pi i jq/4};  INV=true: e^{+2 pi i jq/4}.
 template <bool INV>
 __device__ __forceinline__ void radix4(float2& a, float2& b, float2& c, float2& d) {

@@ -1,6 +1,6 @@
 // What the stage-1 kernel families share (stage1_kernel.cuh: STFT domain, frame 512; stage1_kernel_1024.cuh: frame 1024;
 // stage1_ols_kernel.cuh / stage1_ols1024_kernel.cuh: overlap-save): the parameter block, the PTX wrappers, the per-bin
-// recurrence of the STFT-domain kernels with its real-FFT split, and the per-utterance contract every kernel keeps: the
+// recurrence of the STFT-domain kernels, and the per-utterance contract every kernel keeps: the
 // sample count (utterance_samples), the zero output tail (zero_output_tail) and the ERLE (store_erle).
 #pragma once
 #include <cstdint>
@@ -160,12 +160,6 @@ __device__ __forceinline__ void cp_async_wait() {
 
 // MUFU.RCP without the range fix-up code of __fdividef / the Newton step of 1.0f / x (the argument
 // is a regularised power, far from the denormal / overflow ranges; 1 ulp is ample for 1e-4 parity)
-// MUFU.SQRT (1 ulp) for the magnitudes of the fused feature epilogue (arguments >= 1e-9; same form as aec_features)
-__device__ __forceinline__ float sqrt_approx(float x) {
-    float r;
-    asm("sqrt.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x));
-    return r;
-}
 __device__ __forceinline__ float rcp_fast(float x) {
     float r;
     asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x));
@@ -264,25 +258,6 @@ __device__ __forceinline__ void bin_step(BinState<P, ALGO>& s, const float2 Xn, 
     }
     E = e;
     Yh = yh;
-}
-
-// half-size spectra -> the two real-signal bins of the mirrored pair (k, 256-k).
-// fa = Zc[k], fb = Zc[256-k], w = exp(-2 pi i k/512).  The analysis window carries the 1/2.
-__device__ __forceinline__ void unpack_pair(float2 fa, float2 fb, float2 w, float2& xk, float2& xm) {
-    const float2 a = make_float2(fa.x + fb.x, fa.y - fb.y);          // Zc[k] + conj Zc[256-k]
-    const float2 d = make_float2(fa.y + fb.y, fb.x - fa.x);          // (Zc[k] - conj Zc[256-k]) / i
-    const float2 t = cmul(w, d);
-    xk = make_float2(a.x + t.x, a.y + t.y);
-    xm = make_float2(a.x - t.x, t.y - a.y);                          // conj(a - t)
-}
-// two real-signal bins (k, 256-k) -> half-size inverse spectrum entries G[k], G[256-k]
-// (scale 1/512 lives in the synthesis table).
-__device__ __forceinline__ void pack_pair(float2 ek, float2 em, float2 w, float2& gk, float2& gm) {
-    const float2 a = make_float2(ek.x + em.x, ek.y - em.y);          // E[k] + conj E[256-k]
-    const float2 d = make_float2(ek.x - em.x, ek.y + em.y);          // E[k] - conj E[256-k]
-    const float2 t = cmulc(d, w);                                    // d * conj(w)
-    gk = make_float2(a.x - t.y, a.y + t.x);
-    gm = make_float2(a.x + t.y, t.x - a.y);
 }
 
 // The self-mirrored bin (k = N/4 on the half-size spectrum) has the split / packing twiddle -i, for which unpack_pair /
