@@ -1,12 +1,14 @@
 """Streaming stage 1 (aec_stage1_run_stream, Stage1Stream): the frame-512 overlap-save filters with their state carried
 from one call to the next.
 
-CPU: the stateful float64 oracle in chunks equals ``pbfdaf_ols`` on the whole signal exactly; the state size follows the
-documented layout; every refusal and argument error returns its code without a GPU and without a launch; the streaming
-unit builds exactly the 20 expected kernels.
+CPU: the stateful float64 oracle in chunks equals ``pbfdaf_ols`` on the whole signal exactly, at default and
+non-default filter parameters; the state size follows the documented layout; every refusal and argument error returns
+its code without a GPU and without a launch; the streaming unit builds exactly the 20 expected kernels.
 GPU (-m gpu): chunked runs equal one ``stage1_aec`` call bit for bit for every build (ragged schedules, 0- and 1-block
-calls, every T0 residue mod P, aligned and unaligned rows); the stored state against the float64 oracle; a warm start from
-the oracle's state; ``Stage1Stream`` chunking and reset; batch and call hygiene; the kernel the profiler names.
+calls, every T0 residue mod P, aligned and unaligned rows), at non-default filter parameters too (with the float64
+oracle and the state after init and reset), and at full occupancy; each call's ERLE against its documented span; the
+stored state against the float64 oracle; a warm start from the oracle's state; ``Stage1Stream`` chunking, reset and
+echo / ERLE outputs; batch and call hygiene; the kernel the profiler names.
 """
 import ctypes as C
 import os
@@ -45,27 +47,38 @@ def _signals(B, n, seed):
 # ---------------------------------------------------------------------------------------------------------------------
 # CPU
 # ---------------------------------------------------------------------------------------------------------------------
+# Non-default filter parameters: the PARAMS sets of test_stage1_builds.py for the overlap-save steps.  Across the sets
+# every field a step rule reads (mu, delta, pb_lambda; kalman_a, kalman_lambda, kalman_c0, kalman_eps) leaves its default.
+PARAMS = {
+    2: [dict(pb_lambda=0.0, mu=1.0, delta=0.05), dict(pb_lambda=0.95, mu=0.2, delta=1.0)],
+    3: [dict(kalman_a=0.99, kalman_lambda=0.5, kalman_c0=0.05, kalman_eps=1e-4),
+        dict(kalman_a=0.995, kalman_lambda=0.8, kalman_c0=3.0, kalman_eps=1e-6)],
+}
+
+
 @pytest.mark.parametrize("P", PS)
 @pytest.mark.parametrize("algo", ALGOS)
 def test_oracle_stream_in_chunks_equals_the_whole_signal(P, algo):
-    cfg = O.AecConfig(partitions=P, algo=algo)
+    """at the default parameters and at each PARAMS set of the step"""
     far, mic = _signals(1, 40 * H + 100, 70 + P + algo)
     far, mic = far[0].astype(np.float64), mic[0].astype(np.float64)
-    e_ref, y_ref = O.pbfdaf_ols(far, mic, cfg)
-    rng = np.random.default_rng(P * 10 + algo)
-    for _ in range(3):
-        pos, state, es, ys = 0, None, [], []
-        while pos < len(far):
-            n = int(rng.choice([0, 1, 2, 3, 5])) * H + int(rng.integers(0, H))
-            e, y, state = pbfdaf_ols_stream(far[pos:pos + n], mic[pos:pos + n], cfg, state)
-            es.append(e)
-            ys.append(y)
-            pos += len(e)
-            if len(e) == 0 and n >= len(far) - pos:
-                break
-        assert state["blocks"] == len(far) // H
-        assert np.array_equal(np.concatenate(es), e_ref)
-        assert np.array_equal(np.concatenate(ys), y_ref)
+    for params in [{}] + PARAMS[algo]:
+        cfg = O.AecConfig(partitions=P, algo=algo, **params)
+        e_ref, y_ref = O.pbfdaf_ols(far, mic, cfg)
+        rng = np.random.default_rng(P * 10 + algo)
+        for _ in range(3):
+            pos, state, es, ys = 0, None, [], []
+            while pos < len(far):
+                n = int(rng.choice([0, 1, 2, 3, 5])) * H + int(rng.integers(0, H))
+                e, y, state = pbfdaf_ols_stream(far[pos:pos + n], mic[pos:pos + n], cfg, state)
+                es.append(e)
+                ys.append(y)
+                pos += len(e)
+                if len(e) == 0 and n >= len(far) - pos:
+                    break
+            assert state["blocks"] == len(far) // H
+            assert np.array_equal(np.concatenate(es), e_ref), params
+            assert np.array_equal(np.concatenate(ys), y_ref), params
 
 
 @pytest.mark.parametrize("P", PS)
@@ -272,6 +285,185 @@ def test_chunked_equals_one_call_with_unaligned_rows():
     want = A.stage1_aec(torch.from_numpy(far).cuda(), torch.from_numpy(mic).cuda(), cfg).cpu().numpy()
     for r in range(B):
         assert np.array_equal(errs[r], want[r, :NBLK * H])
+
+
+def _assert_fresh(s, rows, c0):
+    """rows of Stage1Stream s as state_init leaves them: C = c0 exactly (Kalman step), every other field zero"""
+    for name, t in s.state_views().items():
+        v = t[rows].cpu().numpy()
+        if name == "C":
+            assert (v == np.float32(c0)).all(), f"C after init: {np.unique(v)[:4]} != {c0}"
+        else:
+            assert not v.any(), f"{name} is not zero after init"
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("pset", (0, 1))
+@pytest.mark.parametrize("P", (1, 4, 16))
+@pytest.mark.parametrize("algo", ALGOS)
+def test_chunked_at_non_default_parameters(algo, P, pset):
+    """every other test of the stream kernel runs the default parameters, where a state init that ignored
+    kalman_c0 (the stream kernel reads C from the state) would pass: chunked runs at the PARAMS sets equal one
+    stage1_aec call bit for bit (error and echo), and the float64 oracle at 1e-4; the state right after state_init and
+    after reset by indices and by bool mask is zero except C = kalman_c0"""
+    import acoustic_echo_cancellation_b200 as A
+    torch = _torch()
+    params = PARAMS[algo][pset]
+    B = 4
+    far, mic = _signals(B, NBLK * H, 800 + P + algo)
+    cfg = _cfg(P, algo, **params)
+    c0 = cfg.kalman_c0
+    raw = _Raw(B, cfg)
+    _assert_fresh(raw.s, list(range(B)), c0)
+    scheds = _schedules(P, B, NBLK, np.random.default_rng(P + 3 * algo + 7 * pset))
+    errs, echs, pos = _chunked(raw, far, mic, scheds, echo=True)
+    want_e, want_y = (t.cpu().numpy() for t in A.stage1_aec(torch.from_numpy(far).cuda(), torch.from_numpy(mic).cuda(),
+                                                            cfg, return_echo=True))
+    cfg_o = O.AecConfig(partitions=P, algo=algo, **params)
+    for r in range(B):
+        assert pos[r] == NBLK * H
+        assert np.array_equal(errs[r], want_e[r, :NBLK * H]), f"stream {r}: err differs"
+        assert np.array_equal(echs[r], want_y[r, :NBLK * H]), f"stream {r}: echo differs"
+        e64, y64 = O.pbfdaf_ols(far[r], mic[r], cfg_o)
+        assert np.abs(errs[r] - e64).max() <= 1e-4
+        assert np.abs(echs[r] - y64).max() <= 1e-4
+    before = raw.s.state.clone()
+    raw.s.reset([1, 3])
+    _assert_fresh(raw.s, [1, 3], c0)
+    raw.s.reset(torch.tensor([True, False, False, False]))
+    _assert_fresh(raw.s, [0, 1, 3], c0)
+    assert torch.equal(raw.s.state[2], before[2]), "reset touched a row it was not given"
+
+
+def _call_kind(T0, k, skip):
+    """where a call of k blocks from stream block T0 lies against the ERLE skip"""
+    if k == 0:
+        return "zero"
+    if T0 + k <= skip:
+        return "before"
+    return "after" if T0 >= skip else "across"
+
+
+# per stream, blocks per call: one block at a time (every boundary exactly), calls that straddle 5 and 13 or end / start
+# on them, one call over everything
+ERLE_BLOCKS = [[0] + [1] * 15 + [0, 5, 10], [3, 4, 0, 10, 13], [5, 8, 0, 17], [30]]
+# Stage1Stream: one chunk length per call for all streams; blocks per call 0 3 0 1 4 0 7 5 12 1 0 16
+ERLE_CHUNKS = [100, 700, 1, 255, 1000, 0, 2000, 1300, 3000, 333, 0, 4096]
+
+
+def _check_erle(got, mic, e64, T0, k, skip, what):
+    """got against O.erle_db over the call's blocks (stream blocks T0 .. T0 + k - 1) with index >= skip, within 0.05 dB;
+    exactly 0 dB without any"""
+    a = max(skip - T0, 0)
+    if a >= k:
+        assert got == 0.0, f"{what}, blocks {T0}+{k}, skip {skip}: {got} dB, want exactly 0"
+    else:
+        want = float(O.erle_db(mic[a * H:k * H], e64[a * H:k * H])[0])
+        assert abs(got - want) <= 0.05, f"{what}, blocks {T0}+{k}, skip {skip}: {got} dB vs {want}"
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("skip", (0, 5, 13))
+def test_stream_erle_covers_the_blocks_from_the_skip(skip):
+    """erle_db of every call covers the call's blocks whose index in the stream is >= erle_skip_hops (the only kernel
+    that clamps erle_skip_hops - T0): calls wholly before the skip, across it, wholly after it and without a block,
+    against the float64 oracle (chunked pbfdaf_ols_stream) within 0.05 dB, and exactly 0 dB where no block counts.
+    Once through the C ABI with per-stream schedules, once through Stage1Stream.process(return_echo, return_erle),
+    whose n_out, error, echo and ERLE must equal raw calls over the same blocks."""
+    import acoustic_echo_cancellation_b200 as A
+    torch = _torch()
+    P, algo = 8, 3
+    cfg = _cfg(P, algo, erle_skip_hops=skip)
+    cfg_o = O.AecConfig(partitions=P, algo=algo)
+    B = len(ERLE_BLOCKS)
+    nblk = sum(ERLE_CHUNKS) // H
+    far, mic = _signals(B, (nblk + 1) * H, 900 + skip)
+    rng = np.random.default_rng(skip)
+    kinds = set()
+
+    # the C ABI, a schedule per stream (samples past the last whole block are given and not consumed)
+    raw = _Raw(B, cfg)
+    T0, states = [0] * B, [None] * B
+    for c in range(max(len(s) for s in ERLE_BLOCKS)):
+        ks = [s[c] if c < len(s) else 0 for s in ERLE_BLOCKS]
+        ns = [k * H + int(rng.integers(0, H)) for k in ks]
+        L = max(ns)
+        fk = np.zeros((B, L), np.float32)
+        mk = np.zeros((B, L), np.float32)
+        for b in range(B):
+            fk[b, :ns[b]] = far[b, T0[b] * H:T0[b] * H + ns[b]]
+            mk[b, :ns[b]] = mic[b, T0[b] * H:T0[b] * H + ns[b]]
+        e, _, erle = raw.call(fk, mk, ns, erle=True)
+        for b in range(B):
+            k = ks[b]
+            e64, _, states[b] = pbfdaf_ols_stream(fk[b, :k * H], mk[b, :k * H], cfg_o, states[b])
+            assert np.abs(e[b, :k * H] - e64).max(initial=0.0) <= 1e-4
+            _check_erle(erle[b], mk[b], e64, T0[b], k, skip, f"stream {b}")
+            kinds.add(_call_kind(T0[b], k, skip))
+            T0[b] += k
+    assert kinds == ({"zero", "after"} if skip == 0 else {"zero", "before", "across", "after"})
+
+    # Stage1Stream, the same chunks for every stream, against raw calls over the blocks each call consumes
+    s = A.Stage1Stream(B, cfg)
+    ref = _Raw(B, cfg)
+    ft, mt = torch.from_numpy(far).cuda(), torch.from_numpy(mic).cuda()
+    pos, T, kinds, states = 0, 0, set(), [None] * B
+    for n in ERLE_CHUNKS:
+        err, n_out, echo, erle = s.process(ft[:, pos:pos + n], mt[:, pos:pos + n], return_echo=True, return_erle=True)
+        k = (pos + n) // H - T
+        assert n_out.cpu().tolist() == [k * H] * B
+        assert err.shape[1] >= k * H and echo.shape == err.shape
+        e, y, erle_r = ref.call(far[:, T * H:(T + k) * H], mic[:, T * H:(T + k) * H], [k * H] * B, echo=True,
+                                erle=True)
+        assert np.array_equal(err[:, :k * H].cpu().numpy(), e) and not err[:, k * H:].any()
+        assert np.array_equal(echo[:, :k * H].cpu().numpy(), y), "Stage1Stream's echo differs from the raw call's"
+        assert np.array_equal(erle.cpu().numpy(), erle_r)
+        for b in range(B):
+            e64, _, states[b] = pbfdaf_ols_stream(far[b, T * H:(T + k) * H], mic[b, T * H:(T + k) * H], cfg_o, states[b])
+            _check_erle(erle_r[b], mic[b, T * H:], e64, T, k, skip, f"Stage1Stream, stream {b}")
+        kinds.add(_call_kind(T, k, skip))
+        pos, T = pos + n, T + k
+    assert kinds == ({"zero", "after"} if skip == 0 else {"zero", "before", "across", "after"})
+
+
+def _occupancy_signals(B, n, seed):
+    """B rows: 8 synthetic utterances, each row one of them at its own gain"""
+    rng = np.random.default_rng(seed)
+    far, mic = _signals(8, n, seed)
+    g = (0.25 + 0.75 * rng.random(B)).astype(np.float32)[:, None]
+    idx = np.arange(B) % 8
+    return far[idx] * g, mic[idx] * g
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("P,algo,Bspec", [(4, 3, (16, 5)), (16, 2, (4, 3))], ids=("P4-kalman-16sms+5", "P16-nlms-4sms+3"))
+def test_full_occupancy_chunked_equals_one_call(P, algo, Bspec):
+    """several full waves of co-resident CTAs (the two-warp build picks the warp that starts the transform chain from
+    the hardware warp slot, which only varies when CTAs share an SM), each row its own ragged schedule: every row equals
+    stage1_aec on the same rows bit for bit, two identical runs give identical outputs and stored state, and 16 random
+    rows match the float64 oracle at 1e-4"""
+    import acoustic_echo_cancellation_b200 as A
+    torch = _torch()
+    sms = torch.cuda.get_device_properties(torch.cuda.current_device()).multi_processor_count
+    B, nblk = Bspec[0] * sms + Bspec[1], 24
+    far, mic = _occupancy_signals(B, nblk * H, 1000 + P)
+    cfg = _cfg(P, algo)
+    scheds = _schedules(P, B, nblk, np.random.default_rng(P))
+    runs = []
+    for _ in range(2):
+        raw = _Raw(B, cfg)
+        errs, _, pos = _chunked(raw, far, mic, scheds)
+        assert pos == [nblk * H] * B
+        runs.append((errs, raw.s.state.cpu().numpy()))
+    assert all(np.array_equal(a, b) for a, b in zip(runs[0][0], runs[1][0])), "two identical runs differ"
+    assert np.array_equal(runs[0][1], runs[1][1]), "two identical runs store different states"
+    want = A.stage1_aec(torch.from_numpy(far).cuda(), torch.from_numpy(mic).cuda(), cfg).cpu().numpy()
+    bad = [r for r in range(B) if not np.array_equal(runs[0][0][r], want[r])]
+    assert not bad, f"{len(bad)} rows differ from stage1_aec, first {bad[:8]}"
+    cfg_o = O.AecConfig(partitions=P, algo=algo)
+    for r in np.random.default_rng(B).choice(B, size=16, replace=False):
+        e64, _ = O.pbfdaf_ols(far[r], mic[r], cfg_o)
+        assert np.abs(runs[0][0][r] - e64).max() <= 1e-4, f"row {r}"
 
 
 def _oracle_state(far, mic, cfg_o, k, dtype=np.float64):

@@ -6,9 +6,10 @@ state size follows the documented layout; every refusal and argument error retur
 launch.
 GPU (-m gpu): chunked calls equal one call bit for bit (ragged per-row schedules, 0-, 1-, 16- and 625-hop calls, aligned
 and unaligned rows, batch sizes on both sides of the kernel's persistent-grid threshold); one call and a flush against
-the float64 oracle and, to 1e-6 relative, against ``LittleNetInference(in_norm=False)``; the stored state against the oracle
-state and a warm start from it; ``Stage2Stream`` chunking, flush and reset; hygiene; ``AecStream`` end to end; the kernel
-the profiler names.
+the float64 oracle and, to 1e-6 relative, against ``LittleNetInference(in_norm=False)``; the same over 10 s utterances in
+160-sample chunks, with the state after 625 hops; the stored state against the oracle state and a warm start from it;
+``Stage2Stream`` chunking, flush and reset; hygiene; ``AecStream`` end to end and through flushes and resets of some
+rows; the kernel the profiler names.
 """
 import ctypes as C
 import os
@@ -342,6 +343,46 @@ def test_state_against_the_oracle_and_a_warm_start():
 
 
 @pytest.mark.gpu
+def test_whole_utterances_in_160_sample_chunks():
+    """10 s rows (625 hops) at per-row gains, fed to Stage2Stream in 160-sample chunks and flushed: the carried GRU state
+    and overlap-add must not drift from the one-shot path over a real utterance (the other comparisons with
+    LittleNetInference and the oracle stop at 48 hops; the 640-hop test compares the streaming kernel with itself).
+    Output within 1e-6 x max|LittleNetInference(in_norm=False)| (up to 6.0e-7 measured on these rows on a B200, of the
+    same size at hop 48 as at hop 624: float32 rounding, not a drift) and TOL_NET of the float64 oracle;
+    h and ola after 625 hops against little_net_stream's float64 state, as at 37 hops in
+    test_state_against_the_oracle_and_a_warm_start."""
+    import acoustic_echo_cancellation_b200 as A
+    torch = _torch()
+    w, erb = _weights()
+    B, n, chunk = 4, 625 * H, 160
+    mic, ref = _signals(B, n, 21)
+    s = _stream(B)
+    outs = []
+    for pos in range(0, n, chunk):
+        o, c = s.process(mic[:, pos:pos + chunk], ref[:, pos:pos + chunk])
+        c = c.cpu().tolist()
+        assert c == [c[0]] * B
+        outs.append(o[:, :c[0]])
+    v = {name: t.cpu().numpy() for name, t in s.state_views().items()}
+    o, c = s.flush()
+    assert c.cpu().tolist() == [H] * B
+    got = torch.cat(outs + [o[:, :H]], dim=1).cpu().numpy()
+    assert got.shape == (B, n)
+    want = A.LittleNetInference(w, erb)(mic, ref, in_norm=False).cpu().numpy()
+    m64, r64 = mic.cpu().numpy().astype(np.float64), ref.cpu().numpy().astype(np.float64)
+    want64 = O.stage2_little_net(m64, r64, erb, w, in_norm=False)
+    for b in range(B):
+        err = np.abs(got[b] - want[b]).max() / np.abs(want[b]).max()
+        assert err <= 1e-6, f"row {b}: {err:.3g} x max|LittleNetInference|"
+        err = np.abs(got[b] - want64[b]).max() / np.abs(want64[b]).max()
+        assert err <= TOL_NET, f"row {b}: {err:.3g} x max|oracle|"
+        _, st = little_net_stream(m64[b], r64[b], erb, w)
+        assert v["frames"][b] == 625
+        assert np.abs(v["h"][b] - st["h"]).max() <= TOL_NET         # |h| < 1
+        assert np.abs(v["ola"][b] - st["ola"]).max() <= TOL_NET * np.abs(st["ola"]).max()
+
+
+@pytest.mark.gpu
 @pytest.mark.parametrize("chunk", (1, 160, 333))
 def test_stage2_stream_any_chunk_length(chunk):
     torch = _torch()
@@ -468,6 +509,88 @@ def test_aec_stream_end_to_end():
         assert err_r <= TOL_NET, err_r
         for other in results[:-1]:
             assert np.array_equal(other[r], results[-1][r]), "chunked differs from unchunked"
+
+
+# One call sequence for all six streams: ("p", chunk length) is a process call, ("flush", rows) / ("reset", rows) end the
+# listed rows' segments.  Row 4 is flushed after 161 samples (no whole hop); row 1 mid-stream with 160 far-end samples
+# held back by stage 1, then continues; row 3 is reset by bool mask; row 5 is flushed twice in a row (238 samples held
+# back); rows 0 and 2 run through to the final flush of every row.
+LIFECYCLE = [("p", 0), ("p", 1), ("p", 160), ("flush", [4]), ("p", 255), ("p", 4096), ("flush", [1]), ("p", 257),
+             ("reset", [False, False, False, True, False, False]), ("p", 333), ("p", 256), ("flush", [5]),
+             ("flush", [5]), ("p", 160), ("p", 4096), ("p", 1), ("p", 0), ("flush", None)]
+
+
+def _lifecycle(s, far, mic):
+    """run LIFECYCLE on AecStream s; returns per row the list of its segments (first sample, end, flushed, output), and
+    checks every call's n_out and, after every call, the bookkeeping between the stages: stage 2 holds no pending
+    samples (AecStream.flush relies on it) and AecStream holds back as many far-end samples as stage 1 holds"""
+    torch = _torch()
+    B = far.shape[0]
+    pos, start, outs, segs = 0, [0] * B, [[] for _ in range(B)], [[] for _ in range(B)]
+
+    def emitted(k):             # output samples of a segment of k samples before its flush
+        return max(k // H - 1, 0) * H
+
+    for op, arg in LIFECYCLE:
+        if op == "p":
+            o, c = s.process(far[:, pos:pos + arg], mic[:, pos:pos + arg])
+            want = [emitted(pos + arg - start[r]) - emitted(pos - start[r]) for r in range(B)]
+            pos += arg
+        elif op == "flush":
+            o, c = s.flush(arg)
+            rows = range(B) if arg is None else arg
+            want = [(H if pos - start[r] >= H else 0) if r in rows else 0 for r in range(B)]
+        else:
+            s.reset(arg)
+            rows, c = [r for r in range(B) if arg[r]], None
+        if c is not None:
+            assert c.cpu().tolist() == want, f"{op} {arg}: n_out {c.cpu().tolist()} != {want}"
+            for r in range(B):
+                outs[r].append(o[r, :want[r]].cpu().numpy())
+        assert not bool(s.s2._npend.any()), f"after {op} {arg}: stage 2 holds samples between calls"
+        assert torch.equal(s._nfar, s.s1._npend), f"after {op} {arg}: far-end samples held back != stage 1's pending"
+        if op != "p":
+            for r in rows:
+                segs[r].append((start[r], pos, op == "flush", np.concatenate(outs[r])))
+                start[r], outs[r] = pos, []
+    assert all(not o for o in outs)
+    return segs
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("P,algo", [(16, 3), (4, 2)], ids=("P16-kalman", "P4-nlms"))
+def test_aec_stream_lifecycle(P, algo):
+    """AecStream's own bookkeeping (the far-end samples stage 1 holds back, flush and reset of some rows while the others
+    continue, chunks of 0, 1, 160, 255, 256, 257, 333 and 4096 samples): a mistake there mispairs the error and far-end
+    samples of one stream and leaves the others right.  Every segment of every row between lifecycle events equals a
+    fresh AecStream over that segment in one call (and a flush, where the segment was flushed) bit for bit, and
+    LittleNetInference(in_norm=False)(stage1_aec(far, mic), far) on the segment within TOL_NET (a reset segment: the
+    samples it produced); a flushed segment yields (num_frames(len) - 1) * 256 samples."""
+    import acoustic_echo_cancellation_b200 as A
+    torch = _torch()
+    w, erb = _weights()
+    net = A.LittleNetInference(w, erb)
+    cfg = A.Stage1Config(partitions=P, algo=algo)
+    n = sum(a for op, a in LIFECYCLE if op == "p")
+    far, mic = _echo_signals(6, n, 30 + P)
+    segs = _lifecycle(A.AecStream(6, cfg, w, erb), far, mic)
+    assert [len(x) for x in segs] == [1, 2, 1, 2, 2, 3]
+    for r in range(6):
+        for a, b, flushed, got in segs[r]:
+            f, m = far[r:r + 1, a:b], mic[r:r + 1, a:b]
+            fresh = A.AecStream(1, cfg, w, erb)
+            o, c = fresh.process(f, m)
+            one = [o[0, :int(c[0])]]
+            if flushed:
+                o, c = fresh.flush()
+                one.append(o[0, :int(c[0])])
+                assert got.shape == ((A.num_frames(b - a) - 1) * H,)
+            assert np.array_equal(got, torch.cat(one).cpu().numpy()), f"row {r}, samples {a}:{b}"
+            if got.size:
+                want = net(A.stage1_aec(f.contiguous(), m.contiguous(), cfg), f.contiguous(), in_norm=False)
+                want = want[0].cpu().numpy()
+                err = np.abs(got - want[:got.size]).max() / np.abs(want).max()
+                assert err <= TOL_NET, f"row {r}, samples {a}:{b}: {err:.3g}"
 
 
 @pytest.mark.gpu
